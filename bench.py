@@ -2,7 +2,7 @@
 """Benchmark of the proximal-Langevin hot path (BASELINE.json metric:
 "MYULA iterations/s at L=256 (per chain and x chains)").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one MYULA iteration (mcmc.py:158-164 of the reference: data-fidelity
 gradient through Psi^dagger, fused soft-threshold prox + Langevin update with
@@ -307,12 +307,29 @@ def release_plans():
     torch.cuda.empty_cache()
 
 
-def measure_chains(ctx, args, nch, total_chains, steps, blocks=0, block_iters=100, e2e_steps=0, real=False):
+DUMP_SAMPLES = 1 << 20  # complex values kept per dumped array: 16 MiB of float64, 32 MiB for the two arrays
+
+
+def sample_outputs(t):
+    """float64 [k, 2] (real, imaginary parts) of a complex device tensor: all its elements in row-major order when there
+    are at most DUMP_SAMPLES, else DUMP_SAMPLES of them at sorted flat indices drawn without replacement from a generator
+    seeded with 0, i.e. the same elements for the same shape in every run"""
+    import torch
+
+    flat = t.reshape(-1)
+    if flat.numel() > DUMP_SAMPLES:
+        idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_SAMPLES, replace=False))
+        flat = flat[torch.as_tensor(idx, device=flat.device)]
+    return torch.view_as_real(flat).cpu().numpy()
+
+
+def measure_chains(ctx, args, nch, total_chains, steps, blocks=0, block_iters=100, e2e_steps=0, real=False, dump=False):
     """`steps` MYULA iterations of `nch` chains on this GPU (config 5 / the BASELINE metric): device-resident value, per-stage
     device times, optional sustained blocks and the end-to-end figure through host buffers.  Chain c of the job draws
     Philox stream c whatever the sharding.  `real`: REAL-valued data (the drivers' `_mw_` input route,
     experiments/earthtopography/main.py:83-85) and MYULA(real_pairs=True): the `nch` real chains travel as nch / 2
-    complex device chains."""
+    complex device chains.  `dump`: out["outputs"] holds samples (`sample_outputs`) of the chain states and pixel
+    predictions the last timed step returned."""
     import ctypes as C
 
     torch = ctx.torch
@@ -351,11 +368,16 @@ def measure_chains(ctx, args, nch, total_chains, steps, blocks=0, block_iters=10
     for _ in range(max(args.warmup, 3)):
         X, P = m.iterate(X, P)
     # the GPU leaves its idle clocks only after some tens of ms of load: keep iterating (untimed)
-    # until 0.3 s have passed so that the timed region starts at the sustained clock
+    # until 0.3 s have passed so that the timed region starts at the sustained clock.  The timed region then restarts
+    # from the state and Philox step reached after the warm-up iterations, so that its inputs do not depend on how
+    # many iterations fitted into the 0.3 s
+    X0, P0, step0 = X.clone(), P.clone(), m._step_counter
     t_w = time.perf_counter()
     while time.perf_counter() - t_w < 0.3:
         X, P = m.iterate(X, P)
         torch.cuda.synchronize()
+    X, P, m._step_counter = X0, P0, step0
+    del X0, P0
     ctx.barrier()
     sampler = ClockSampler(ctx.local)
     sampler.start()
@@ -368,6 +390,7 @@ def measure_chains(ctx, args, nch, total_chains, steps, blocks=0, block_iters=10
         X, P = m.iterate(X, P)
     e1.record()
     ctx.barrier()
+    last = (X, P)  # what the last timed step returned (the iterations below allocate new tensors)
     ms = e0.elapsed_time(e1)
     ms_kind = (C.c_double * 3)()
     cnt_kind = (C.c_longlong * 3)()
@@ -428,7 +451,9 @@ def measure_chains(ctx, args, nch, total_chains, steps, blocks=0, block_iters=10
         out["e2e_bytes"] = (ncoef + (npix if with_preds else 0)) * nch_dev * 16
         out["e2e_with_preds"] = with_preds
         del Xh, Ph, Xo, Po
-    del m, outer, op, reg, X, P
+    if dump:
+        out["outputs"] = {"state": sample_outputs(last[0]), "predictions": sample_outputs(m._pix(last[1]))}
+    del m, outer, op, reg, X, P, last
     return out
 
 
@@ -638,8 +663,12 @@ def run_ours(args):
     L, B, J_min, nch = args.L, args.B, args.J_min, args.chains
     world = ctx.world
     main = measure_chains(ctx, args, nch, nch * world, args.steps, blocks=args.blocks, block_iters=args.block_iters,
-                          e2e_steps=max(1, min(args.steps, args.e2e_steps)))
+                          e2e_steps=max(1, min(args.steps, args.e2e_steps)), dump=bool(args.dump_outputs) and ctx.rank == 0)
     release_plans()
+    if "outputs" in main:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in main.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     extras = {}
     if not args.no_extras and not args.no_real_pairs and nch % 2 == 0:
         # the same sweep on REAL-valued data (the drivers' `_mw_` route): two real chains per complex device chain
@@ -702,12 +731,6 @@ def run_ours(args):
             release_plans()
             extras["configs"] = measure_configs(ctx, args)
             release_plans()
-            os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-            try:
-                json.dump({k: extras[k] for k in ("per_chain_latency", "configs", "config4_msharded") if k in extras},
-                          open(os.path.join(ROOT, "gpurun_out", "config_timings.json"), "w"), indent=1)
-            except OSError:
-                pass
         peak = dgemm_peak(torch)
         hbm_peak, hbm_src = hbm_peak_gbs()
         traffic, tsrc = load_traffic()
@@ -1039,7 +1062,14 @@ def main():
     ap.add_argument("--workload", default="chains", choices=["chains", "wl-msharded"],
                     help="chains: the BASELINE metric (independent chains, weak scaling); wl-msharded: config 4, one "
                          "weak-lensing chain m-sharded over the GPUs (strong scaling; defaults L=512 B=2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's chains) to DIR/state.npy and DIR/predictions.npy: "
+                         "float64 [k, 2] real and imaginary parts of the new chain states and of their pixel predictions, "
+                         "each cut to a fixed sample of 2^20 elements when larger (sample_outputs); the inputs are the "
+                         "same in every run with the same arguments")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "chains"):
+        ap.error("--dump-outputs applies to the chains workload of --impl ours")
     # stdout carries exactly ONE JSON line: everything else this process prints (the samplers' "DONE", progress lines,
     # library banners) goes to stderr; emit() writes the line to the real stdout
     global _REAL_STDOUT

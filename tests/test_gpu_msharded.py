@@ -7,7 +7,7 @@
   unsharded plan (itself pinned to the oracle/fixtures in test_gpu_parity.py) at
   bandlimits with several 64-ring blocks.
 * `test_two_processes_*`: real one-process-per-GPU run over CUDA IPC + NVLink,
-  skipped when fewer than two GPUs are visible (run with `gpurun --gpus 2`).
+  skipped when fewer than two GPUs are visible.
 """
 import os
 import subprocess
@@ -151,7 +151,7 @@ def test_two_processes_over_nvlink():
     import torch
 
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
            "--master-port", "29533", os.path.join(ROOT, "scripts", "msharded_check.py"), "--L", "136", "--B", "2"]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
