@@ -268,7 +268,11 @@ __global__ void pxm_legendre_naive_kernel(const double* __restrict__ tab, const 
   const int row = threadIdx.x & 63;
   for (int col = blockIdx.y * blockDim.x / 64 + (threadIdx.x >> 6); col < nld; col += gridDim.y * (blockDim.x / 64)) {
     const int tl = row / TILE_ROWS;
-    if (tl >= item.nmt_out) continue;
+    if (tl >= item.nmt_out) {
+      // padded rows of harmonic buffers: zeros, as the tensor-core kernel writes them (outputs need no initialisation)
+      if (item.pad) cmat[item.c_off + pxm_il_index(row, col, nld)] = 0.0;
+      continue;
+    }
     double acc = 0.0;
     for (int s = 0; s < item.seg_count; ++s) {
       const PxmLegSeg sg = segs[item.seg_begin + s];

@@ -12,6 +12,7 @@ import pytest
 from scipy import sparse
 
 from conftest import golden, rel_l2
+from oracle.philox_ref import philox_uniform as _philox_uniform
 
 pytestmark = pytest.mark.gpu
 
@@ -706,20 +707,6 @@ def test_weaklensing_harmonic_fusion_equals_pixel_space_composition(px):
     a = np.vdot(y1, t._inverse_harmonic(x1))
     b = np.vdot(t._inverse_adjoint_harmonic(y1), x1)
     assert abs(a - b) / abs(a) < TOL
-
-
-def _philox_uniform(seed, stream, step):
-    """host restatement of the uniform `pxm_pxmala_accept` draws: Philox4x32-10, counter
-    (0xFFFFFFFF, 0xFFFFFFFF, step_lo, step_hi ^ stream*0x85EBCA6B), key (seed_lo, seed_hi ^ stream)"""
-    M = 0xFFFFFFFF
-    c = [M, M, step & M, ((step >> 32) & M) ^ ((stream * 0x85EBCA6B) & M)]
-    k0, k1 = seed & M, ((seed >> 32) & M) ^ (stream & M)
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c[0], 0xCD9E8D57 * c[2]
-        c = [((p1 >> 32) ^ c[1] ^ k0) & M, p1 & M, ((p0 >> 32) ^ c[3] ^ k1) & M, p0 & M]
-        k0, k1 = (k0 + 0x9E3779B9) & M, (k1 + 0xBB67AE85) & M
-    bits = (c[0] << 32) | c[1]
-    return ((bits >> 11) + 0.5) / 9007199254740992.0
 
 
 @pytest.mark.parametrize("setting", ["analysis", "synthesis"])
