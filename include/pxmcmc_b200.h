@@ -272,6 +272,31 @@ int pxm_quantile_columns(const double* d_chain, long long nsamples, long long nc
                          double gamma_a, long long lo_b, double gamma_b, double* d_out_a, double* d_out_b, void* stream);
 int pxm_quantile_columns_max_samples(void);
 
+/* ---- streaming posterior summaries --------------------------------------------
+ * (no counterpart in the reference, which stores every tracked sample.)  Per-element running moments of a batch of
+ * chains on the tracking grid, from which the pooled mean and variance, split-R-hat and a batch-means ESS follow
+ * without storing samples (DESIGN.md 7b).  d_x: the chains' state or predictions, complex [nchains][n].
+ * mode 0: the real part of every chain; 1: real and imaginary part as two components; 2: packed real chain pairs
+ * (real part = logical chain 2c, imaginary part = 2c + 1).  A slot is one component of one logical chain:
+ * mode 0 slot = c, modes 1 and 2 slot = 2c + part; nslots = nchains (mode 0) or 2 nchains.
+ * Accumulator: 8 fields, each [nslots][n] doubles, in this order: mean and M2 of half A (samples [0, h)), middle
+ * sample (j = h when nsamples is odd), mean and M2 of half B ([nsamples - h, nsamples)), open batch sum, mean and M2
+ * of the batch means; h = nsamples / 2, batch size b = max(1, floor(sqrt nsamples)), a = nsamples / b batches.
+ * pxm_stats_accumulator_doubles: its size (-1 on a bad argument).  pxm_stats_reset: zero it.
+ * pxm_stats_accumulate: push sample j of every chain (d_j == NULL) or sample d_j[c] of chain c (< 0: chain c takes no
+ * sample now); 0 <= j < nsamples.  Every sample index of a chain is pushed once, in increasing order.
+ * pxm_stats_partials: the partial record, 10 fields each [ncomp][n] doubles (ncomp = 2 in mode 1, else 1), over the
+ * logical chains in order: half-chain count, mean and M2 of the half-chain means, sum of the half-chain variances
+ * (ddof 1); sample count, pooled mean, pooled M2; batch count, mean and M2 of the batch means.  Records of disjoint
+ * chain groups combine with Chan's rule.  d_chain_mean / d_chain_var (may be NULL): [nslots][n] per-chain mean and
+ * variance (ddof 1). */
+long long pxm_stats_accumulator_doubles(long long n, long long nchains, int mode);
+int pxm_stats_reset(double* d_acc, long long n, long long nchains, int mode, void* stream);
+int pxm_stats_accumulate(double* d_acc, const void* d_x, long long n, long long nchains, int mode, long long nsamples,
+                         long long j, const long long* d_j, void* stream);
+int pxm_stats_partials(const double* d_acc, long long n, long long nchains, int mode, long long nsamples,
+                       double* d_partial, double* d_chain_mean, double* d_chain_var, void* stream);
+
 /* ---- measurement aids (bench.py) ---------------------------------------------
  * pxm_profile_begin/end bracket a region in which every library call records a
  * CUDA-event pair on its launching stream; end() returns the summed device time

@@ -97,6 +97,10 @@ SIGNATURES = {
     "pxm_gc_compact": (_i, [_vp, _vp, _vp, _i, _ll, _vp, _vp, _vp]),
     "pxm_quantile_columns": (_i, [_vp, _ll, _ll, _ll, _ll, _d, _ll, _d, _vp, _vp, _vp]),
     "pxm_quantile_columns_max_samples": (_i, []),
+    "pxm_stats_accumulator_doubles": (_ll, [_ll, _ll, _i]),
+    "pxm_stats_reset": (_i, [_vp, _ll, _ll, _i, _vp]),
+    "pxm_stats_accumulate": (_i, [_vp, _vp, _ll, _ll, _i, _ll, _ll, _vp, _vp]),
+    "pxm_stats_partials": (_i, [_vp, _ll, _ll, _i, _ll, _vp, _vp, _vp, _vp]),
     "pxm_profile_begin": (_i, [_i]),
     "pxm_profile_end": (_i, [C.POINTER(_d), C.POINTER(_ll)]),
     "pxm_launch_count": (_ll, []),

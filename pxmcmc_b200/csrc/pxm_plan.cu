@@ -1567,6 +1567,43 @@ int pxm_quantile_columns(const double* d_chain, long long nsamples, long long nc
 }
 int pxm_quantile_columns_max_samples(void) { return pxm_quantile_max_samples(); }
 
+long long pxm_stats_accumulator_doubles(long long n, long long nchains, int mode) {
+  if (n < 1 || nchains < 1 || mode < 0 || mode > 2) {
+    pxm_set_error("bad argument: stats_accumulator_doubles: n >= 1, nchains >= 1, mode 0, 1 or 2");
+    return -1;
+  }
+  return 8 * pxm_stats_slots(mode, nchains) * n;
+}
+
+int pxm_stats_reset(double* d_acc, long long n, long long nchains, int mode, void* stream) {
+  const long long nd = pxm_stats_accumulator_doubles(n, nchains, mode);
+  PXM_REQUIRE(nd > 0 && d_acc != nullptr, "stats_reset: null accumulator, n >= 1, nchains >= 1, mode 0, 1 or 2");
+  PXM_CUDA(cudaMemsetAsync(d_acc, 0, (size_t)nd * sizeof(double), (cudaStream_t)stream));
+  return PXM_OK;
+}
+
+int pxm_stats_accumulate(double* d_acc, const void* d_x, long long n, long long nchains, int mode, long long nsamples,
+                         long long j, const long long* d_j, void* stream) {
+  PXM_REQUIRE(d_acc != nullptr && d_x != nullptr, "stats_accumulate: null pointer");
+  PXM_REQUIRE(n >= 1 && nchains >= 1 && nchains <= 65535, "stats_accumulate: n >= 1, 1 <= nchains <= 65535");
+  PXM_REQUIRE(mode >= 0 && mode <= 2, "stats_accumulate: mode 0 (real part), 1 (re + im) or 2 (packed real pairs)");
+  PXM_REQUIRE(nsamples >= 1, "stats_accumulate: nsamples >= 1");
+  PXM_REQUIRE(d_j != nullptr || (j >= 0 && j < nsamples), "stats_accumulate: sample index j outside [0, nsamples)");
+  ProfScope _ps(2, (cudaStream_t)stream);
+  return pxm_launch_stats_accumulate(d_acc, d_x, (size_t)n, (size_t)nchains, mode, nsamples, j, d_j, (cudaStream_t)stream);
+}
+
+int pxm_stats_partials(const double* d_acc, long long n, long long nchains, int mode, long long nsamples,
+                       double* d_partial, double* d_chain_mean, double* d_chain_var, void* stream) {
+  PXM_REQUIRE(d_acc != nullptr && d_partial != nullptr, "stats_partials: null pointer");
+  PXM_REQUIRE(n >= 1 && nchains >= 1, "stats_partials: n >= 1, nchains >= 1");
+  PXM_REQUIRE(mode >= 0 && mode <= 2, "stats_partials: mode 0 (real part), 1 (re + im) or 2 (packed real pairs)");
+  PXM_REQUIRE(nsamples >= 1, "stats_partials: nsamples >= 1");
+  ProfScope _ps(2, (cudaStream_t)stream);
+  return pxm_launch_stats_partials(d_acc, (size_t)n, (size_t)nchains, mode, nsamples, d_partial, d_chain_mean,
+                                   d_chain_var, (cudaStream_t)stream);
+}
+
 int pxm_csr_spmv(const int* d_indptr, const int* d_indices, const double* d_vals, const void* d_x, void* d_y,
                  int nrows, long long ncols, long long nchains, void* stream) {
   ProfScope _ps(2, (cudaStream_t)stream);

@@ -146,4 +146,10 @@ int pxm_quantile_max_samples();
 int pxm_launch_quantile_columns(const double* chain, long long nsamples, long long ncols, long long ld, long long lo_a,
                                 double g_a, long long lo_b, double g_b, double* out_a, double* out_b, cudaStream_t st);
 
+long long pxm_stats_slots(int mode, long long nchains);
+int pxm_launch_stats_accumulate(double* acc, const void* x, size_t n, size_t nchains, int mode, long long nsamples,
+                                long long j, const long long* d_j, cudaStream_t st);
+int pxm_launch_stats_partials(const double* acc, size_t n, size_t nchains, int mode, long long nsamples, double* rec,
+                              double* cmean, double* cvar, cudaStream_t st);
+
 int pxm_debug_naive();

@@ -466,3 +466,39 @@ def csr_spmv_dev(indptr, indices, vals, x, nrows, ncols):
     out = new_c((x2.shape[0], nrows), x2.device)
     check(lib.pxm_csr_spmv(ptr(indptr), ptr(indices), ptr(vals), ptr(x2), ptr(out), nrows, ncols, x2.shape[0], stream_ptr()))
     return out[0] if was1 else out
+
+
+# ---------------------------------------------------------------------------
+# streaming posterior summaries (pxm_stats_*): accumulators are flat float64 tensors in the library's layout
+# ---------------------------------------------------------------------------
+def stats_accumulator(n, nchains, mode):
+    """zeroed accumulator for `nchains` complex chains of length `n` (mode 0 real part, 1 re + im, 2 packed pairs)"""
+    nd = int(lib.pxm_stats_accumulator_doubles(int(n), int(nchains), int(mode)))
+    if nd < 0:
+        raise _lib.PxmError(lib.pxm_last_error().decode())
+    acc = torch.empty(nd, dtype=FDT, device=dev())
+    check(lib.pxm_stats_reset(ptr(acc), int(n), int(nchains), int(mode), stream_ptr()))
+    return acc
+
+
+def stats_accumulate_dev(acc, x, mode, nsamples, j=0, d_j=None):
+    """push sample j (or, per chain, d_j[c]; < 0 skips the chain) of the complex chains x [nchains, n]"""
+    x2, _ = batch2d(x)
+    if x2.dtype != CDT or not x2.is_contiguous():
+        raise ValueError("stats_accumulate: x must be a contiguous complex128 [nchains, n] tensor")
+    if d_j is not None and (d_j.dtype != torch.int64 or d_j.numel() != x2.shape[0]):
+        raise ValueError("stats_accumulate: d_j must be an int64 tensor with one entry per chain")
+    check(lib.pxm_stats_accumulate(ptr(acc), ptr(x2), x2.shape[1], x2.shape[0], int(mode), int(nsamples), int(j), ptr(d_j),
+                                   stream_ptr()))
+
+
+def stats_partials_dev(acc, n, nchains, mode, nsamples, per_chain=True):
+    """(record [10, ncomp, n], chain mean [nslots, n] or None, chain variance [nslots, n] or None) device tensors"""
+    ncomp = 2 if mode == 1 else 1
+    nslots = nchains if mode == 0 else 2 * nchains
+    rec = torch.empty((10, ncomp, n), dtype=FDT, device=acc.device)
+    cm = torch.empty((nslots, n), dtype=FDT, device=acc.device) if per_chain else None
+    cv = torch.empty((nslots, n), dtype=FDT, device=acc.device) if per_chain else None
+    check(lib.pxm_stats_partials(ptr(acc), int(n), int(nchains), int(mode), int(nsamples), ptr(rec), ptr(cm), ptr(cv),
+                                 stream_ptr()))
+    return rec, cm, cv

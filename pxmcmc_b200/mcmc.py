@@ -11,6 +11,9 @@ sequence of libpxmcmc_b200 kernels.  Two extra keyword-only knobs:
   Philox4x32-10 Gaussians inside the update kernel (throughput mode).
 * ``nchains`` runs that many independent chains as one batch (tracked arrays gain
   a leading chain axis when ``nchains > 1``).
+* ``summarise=("chain",)`` or ``("chain", "predictions")`` keeps streaming posterior summaries on the device (mean,
+  variance, split-R-hat, ESS; see `diagnostics`) instead of, or besides, the tracked arrays: ``sampler.summary`` after
+  ``run()``.
 """
 import numpy as np
 import torch
@@ -62,11 +65,15 @@ class PxMCMC:
     """Common machinery (pxmcmc/mcmc.py:46-140)."""
 
     def __init__(self, forward, prior, mcmcparams=PxMCMCParams(), *, noise="host", nchains=1, seed=0, stream0=0,
-                 spill_dir=None, async_spill=True):
+                 spill_dir=None, async_spill=True, summarise=None):
         """`spill_dir`: directory in which the two large tracked arrays (`chain`, `preds`) live as .npy memory maps
         instead of host RAM (SURVEY.md 8(f)1: 5 000 x 1.22 M samples of config 4 are 49 GB).  `async_spill`: tracked
         samples leave the device through pinned staging buffers on a copy stream while the chain keeps iterating
-        (the run loops never wait for a device -> host copy); False restores the synchronous copy."""
+        (the run loops never wait for a device -> host copy); False restores the synchronous copy.
+        `summarise`: None, ("chain",) or ("chain", "predictions"): running moments of every tracked-grid sample are
+        kept on the device, independently of `track` (one kernel launch per grid sample and target, no host
+        synchronisation, no stored samples); after `run()`, `summary` = {target: diagnostics.Summary} and
+        `summary_partials()` the raw partial records (multi-GPU: sharding.gather_summary)."""
         self.forward = forward
         self.prior = prior
         self.spill_dir = spill_dir
@@ -80,6 +87,8 @@ class PxMCMC:
         self.seed = int(seed)
         self.stream0 = int(stream0)  # global index of this sampler's first chain (Philox stream id)
         self._step_counter = 0
+        self._summarise = self._check_summarise(summarise)
+        self._stats = None
         self._initialise_tracking_arrays()
 
     # ------------------------------------------------------------------ helpers
@@ -312,6 +321,8 @@ class PxMCMC:
         for name in self._TRACKED:
             if hasattr(self, name):
                 d["track_" + name] = getattr(self, name)
+        if self._stats is not None:
+            d.update({"stats_" + k: v for k, v in self._stats.state().items()})
         kind, keys, pos, has_gauss, cached = np.random.get_state()
         d.update(rng_keys=keys, rng_pos=pos, rng_has_gauss=has_gauss, rng_cached=cached)
         tmp = path + ".tmp.npz"
@@ -331,10 +342,16 @@ class PxMCMC:
                     if arr.shape != getattr(self, name).shape:
                         raise ValueError(f"checkpoint array {name} has shape {arr.shape}, expected {getattr(self, name).shape}")
                     getattr(self, name)[...] = arr
+            if self._stats is not None:
+                missing = [k for k in self._stats.acc if "stats_" + k not in f.files]
+                if missing:
+                    raise ValueError(f"checkpoint carries no summary accumulators for {missing}: it was written by a "
+                                     "sampler without summarise=...")
+                self._stats.load({k: f["stats_" + k] for k in self._stats.acc})
             self._step_counter = int(f["step_counter"])
             self.delta = float(f["delta"])
             np.random.set_state(("MT19937", f["rng_keys"], int(f["rng_pos"]), int(f["rng_has_gauss"]), float(f["rng_cached"])))
-            return {k: f[k] for k in f.files if not k.startswith(("track_", "rng_"))}
+            return {k: f[k] for k in f.files if not k.startswith(("track_", "rng_", "stats_"))}
 
     def save_checkpoint(self, path, i, j, X_curr, curr_preds):
         """Everything `run(resume=path)` needs to continue the chain exactly where it stands after iteration
@@ -364,6 +381,61 @@ class PxMCMC:
         w_re = D.to_dev_f(np.random.randn(n * self.nchains))
         w_im = D.to_dev_f(np.random.randn(n * self.nchains)) if self.complex else None
         return w_re, w_im
+
+    # ------------------------------------------------------------------ streaming posterior summaries
+    def _check_summarise(self, summarise):
+        if summarise is None:
+            return ()
+        if isinstance(summarise, str):
+            summarise = (summarise,)
+        t = tuple(summarise)
+        if not t or len(set(t)) != len(t) or any(k not in ("chain", "predictions") for k in t):
+            raise ValueError('summarise must be None, ("chain",) or ("chain", "predictions")')
+        if getattr(self.forward, "_pxm_allreduce", None) is not None:
+            raise NotImplementedError("summarise: streaming summaries of m-sharded single-chain runs are not implemented "
+                                      "(each rank holds only part of every sample)")
+        return t
+
+    def _stats_begin(self, nchains_dev=None, pairs=False):
+        """fresh accumulators at the start of run() (nsamples fixes the half-chain and batch boundaries); modes as in
+        pxm_stats_accumulate: the chain is complex (re + im) only with `complex`, predictions are real parts"""
+        from .diagnostics import StreamingSummary
+
+        self._stats, self.summary = None, None
+        if not self._summarise:
+            return
+        nch = self.nchains if nchains_dev is None else nchains_dev
+        lay = {}
+        if "chain" in self._summarise:
+            lay["chain"] = (self.forward.nparams, nch, 2 if pairs else (1 if self.complex else 0))
+        if "predictions" in self._summarise:
+            lay["predictions"] = (len(self.forward.data), nch, 2 if pairs else 0)
+        self._stats = StreamingSummary(lay, self.nsamples)
+
+    def _stats_push(self, X, P, j=0, d_j=None):
+        """push tracked-grid sample j (per chain: d_j) of the state X and the PIXEL predictions P (may be None when
+        predictions are not summarised)"""
+        if self._stats is None:
+            return
+        if "chain" in self._stats.acc:
+            self._stats.push("chain", X, j, d_j)
+        if "predictions" in self._stats.acc:
+            self._stats.push("predictions", P, j, d_j)
+
+    def _stats_end(self):
+        if self._stats is None:
+            return
+        from .diagnostics import finalize
+
+        self._partials = self._stats.partials()
+        self.summary = {k: finalize([p]) for k, p in self._partials.items()}
+
+    def summary_partials(self):
+        """{target: partial record dict} of the last run (combine several with diagnostics.finalize or
+        sharding.gather_summary)"""
+        if getattr(self, "_partials", None) is None:
+            raise RuntimeError("no summary: construct the sampler with summarise=... and call run()")
+        return self._partials
 
 
 class _Spill:
@@ -535,6 +607,7 @@ class MYULA(PxMCMC):
             return self._run_pairs(start_point, checkpoint, checkpoint_every, resume)
         i = 0
         j = 0
+        self._stats_begin()
         if resume is not None:
             i, j, X_curr, curr_preds = self.load_checkpoint(resume)
         else:
@@ -555,7 +628,9 @@ class MYULA(PxMCMC):
                 X_curr, curr_preds = self.iterate(X_curr, curr_preds)
             if i >= self.nburn:
                 if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
-                    self._track_dev(j, X_curr, curr_preds)
+                    P_pix = self._pix(curr_preds) if "predictions" in self._summarise else curr_preds
+                    self._track_dev(j, X_curr, P_pix)
+                    self._stats_push(X_curr, P_pix, j)
                     j += 1
                 if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
                     self._track_flush()
@@ -570,6 +645,7 @@ class MYULA(PxMCMC):
         if checkpoint is not None:
             self.save_checkpoint(checkpoint, i, j, X_curr, curr_preds)
         self._track_flush()
+        self._stats_end()
         curr_preds = self._pix(curr_preds)
         if graphed is not None:
             X_curr, curr_preds = X_curr.clone(), curr_preds.clone()
@@ -583,6 +659,7 @@ class MYULA(PxMCMC):
         eng = self._pair_engine
         i = 0
         j = 0
+        self._stats_begin(eng.nchains, pairs=True)  # on the packed chains: no unpack copy
         if resume is not None:
             i, j, X_curr, _ = self.load_checkpoint(resume)
         else:
@@ -601,7 +678,9 @@ class MYULA(PxMCMC):
                 Xp, Pp = eng.iterate(Xp, Pp)
             if i >= self.nburn:
                 if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
-                    self._track_dev(j, self.unpack(Xp), self.unpack(eng._pix(Pp)))
+                    Pp_pix = eng._pix(Pp)
+                    self._track_dev(j, self.unpack(Xp), self.unpack(Pp_pix))
+                    self._stats_push(Xp, Pp_pix, j)
                     j += 1
                 if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
                     self._track_flush()
@@ -617,6 +696,7 @@ class MYULA(PxMCMC):
         if checkpoint is not None:
             self.save_checkpoint(checkpoint, i, j, self.unpack(Xp), self.unpack(eng._pix(Pp)))
         self._track_flush()
+        self._stats_end()
         self._final_state = (self.unpack(Xp), self.unpack(eng._pix(Pp)))
         if graphed is not None:
             graphed.release()
@@ -667,6 +747,9 @@ class MYULA(PxMCMC):
         group g, device->host copy of group g-1 -- so that both PCIe directions and the SMs work at
         the same time (the transfers, not the kernels, bound this path).  Results do not depend on
         the grouping: chains are independent and chain c always draws Philox stream stream0 + c."""
+        if self._summarise:
+            raise NotImplementedError("summarise: iterate_host has no tracking grid (run() does); use a sampler "
+                                      "without summarise=...")
         dv = D.dev()
         xh = X_host if D.is_dev(X_host) else torch.from_numpy(np.ascontiguousarray(X_host, dtype=np.complex128))
         if preds_host is None:
@@ -902,6 +985,7 @@ class PxMALA(MYULA):
         acc_chunks, dl_chunks = [], []  # drained parts of the traces: [nch, cap] each
         i = 0
         js = np.zeros(nch, dtype=np.int64)  # tracked samples per chain (accepted proposals on the thinning grid)
+        self._stats_begin()
         if resume is not None:
             ck = self._load_ckpt(resume)
             i, js = int(ck["i"]), ck["js"].astype(np.int64)
@@ -974,6 +1058,10 @@ class PxMALA(MYULA):
             if on_grid or verbose:
                 st = S.cpu().numpy()  # the only host synchronisation
                 take = [c for c in range(nch) if on_grid and st[c, 9] != 0.0 and js[c] < self.nsamples]
+                if take and self._stats is not None:  # every chain's own sample index, -1: no sample now
+                    jd = np.full(nch, -1, dtype=np.int64)
+                    jd[take] = js[take]
+                    self._stats_push(cur[0], cur[1], d_j=torch.from_numpy(jd).to(dv))
                 if take:
                     Xh = D.to_host(cur[0]) if hasattr(self, "chain") else None
                     Ph = D.to_host(cur[1]) if hasattr(self, "preds") else None
@@ -1048,6 +1136,7 @@ class PxMALA(MYULA):
         self.deltas_trace = [float(v) for v in dt[0]] if nch == 1 else dt
         self.delta = float(S[0, 0].item())
         self.deltas = S[:, 0].cpu().numpy()
+        self._stats_end()
         self._final_state = (X_curr.clone(), curr_preds.clone())
         print("\nDONE")
 
@@ -1077,6 +1166,7 @@ class PxMALA(MYULA):
         self.deltas_trace = [self.delta]
         i = 0
         j = 0
+        self._stats_begin()
         if resume is not None:
             ck = self._load_ckpt(resume)
             i, j = int(ck["i"]), int(ck["j"])
@@ -1129,6 +1219,7 @@ class PxMALA(MYULA):
             if i >= self.nburn:
                 if (self.ngap == 0 or (i - self.nburn) % self.ngap == 0) and accept:
                     self._tracking(j, X_curr, curr_preds, [logpiXc], [L2Xc], [priorXc])
+                    self._stats_push(X_curr, curr_preds, j)
                     j += 1
             if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
                 self._print_progress(j - 1, np.real(logpiXc), L2=np.real(L2Xc), prior=priorXc,
@@ -1138,6 +1229,7 @@ class PxMALA(MYULA):
                 save(i)
         if checkpoint is not None:
             save(i)
+        self._stats_end()
         self._final_state = (X_curr, curr_preds)
         print("\nDONE")
 
@@ -1197,6 +1289,7 @@ class SKROCK(PxMCMC):
         """the loop of pxmcmc/mcmc.py:308-336.  `checkpoint` / `checkpoint_every` / `resume` as in `MYULA.run`."""
         i = 0
         j = 0
+        self._stats_begin()
         if resume is not None:
             i, j, X_curr, curr_preds = self.load_checkpoint(resume)
         else:
@@ -1214,6 +1307,7 @@ class SKROCK(PxMCMC):
             if i >= self.nburn:
                 if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
                     self._track_dev(j, X_curr, curr_preds)
+                    self._stats_push(X_curr, curr_preds, j)
                     j += 1
             if self.verbosity > 0 and (i + 1) % self.verbosity == 0 and j > 0:
                 self._track_flush()
@@ -1225,6 +1319,7 @@ class SKROCK(PxMCMC):
         if checkpoint is not None:
             self.save_checkpoint(checkpoint, i, j, X_curr, curr_preds)
         self._track_flush()
+        self._stats_end()
         if graphed is not None:
             X_curr, curr_preds = X_curr.clone(), curr_preds.clone()
         self._final_state = (X_curr, curr_preds)

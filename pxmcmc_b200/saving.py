@@ -5,7 +5,11 @@ parameters and any keyword arguments become attributes.
 The reference writes HDF5 through h5py (pxmcmc/saving.py:18-36).  h5py is used when it can be
 imported (same file, same names: the reference's plot scripts read it unchanged); otherwise the
 same names go into ``<filename>.npz`` (datasets as arrays, attributes under ``attrs/<name>``) and
-``load_mcmc`` reads either."""
+``load_mcmc`` reads either.
+
+Streaming posterior summaries (``PxMCMC(summarise=...)``, an extension) are written, when present, as datasets
+``summary/<target>/<statistic>`` (plus ``nchains`` and ``nsamples``); ``load_mcmc`` returns them under the same flat
+names and ``summaries`` turns them back into ``diagnostics.Summary`` objects."""
 import os
 
 import numpy as np
@@ -20,6 +24,11 @@ def _collect(mcmc, params, kwargs):
         if hasattr(mcmc, attr):
             arr = np.asarray(getattr(mcmc, attr))
             data[name] = arr.astype("i1") if name == "acceptances" else arr
+    for target, sm in (getattr(mcmc, "summary", None) or {}).items():
+        for stat, arr in sm.as_dict().items():
+            data[f"summary/{target}/{stat}"] = np.asarray(arr)
+        data[f"summary/{target}/nchains"] = np.asarray(sm.nchains)
+        data[f"summary/{target}/nsamples"] = np.asarray(sm.nsamples)
     attrs = {k: getattr(params, k) for k in params.__dict__.keys()}
     attrs.update(kwargs)
     return data, attrs
@@ -59,4 +68,18 @@ def load_mcmc(path):
     import h5py
 
     with h5py.File(path, "r") as f:
-        return {k: f[k][()] for k in f.keys()}, dict(f.attrs)
+        data = {}
+        f.visititems(lambda name, obj: data.__setitem__(name, obj[()]) if isinstance(obj, h5py.Dataset) else None)
+        return data, dict(f.attrs)
+
+
+def summaries(data):
+    """{target: diagnostics.Summary} from the datasets `load_mcmc` returned (empty when the file has none)"""
+    from .diagnostics import Summary
+
+    out = {}
+    for target in sorted({k.split("/")[1] for k in data if k.startswith("summary/")}):
+        pre = f"summary/{target}/"
+        stats = {k[len(pre):]: data[k] for k in data if k.startswith(pre)}
+        out[target] = Summary(int(stats.pop("nchains")), int(stats.pop("nsamples")), **stats)
+    return out

@@ -59,3 +59,34 @@ def max_over_ranks(value, group=None):
         t = t.cuda()
     dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
     return float(t.item())
+
+
+def gather_summary(partials, nchains_total, group=None, chain_arrays=True):
+    """Streaming posterior summaries of chains sharded over ranks: `partials` = this rank's
+    `sampler.summary_partials()` ({target: partial record dict}); rank 0 receives every rank's records and returns
+    {target: diagnostics.Summary} over all `nchains_total` logical chains (per-chain arrays in global chain order, as
+    `gather_chains`; `chain_arrays=False` leaves them out and sends only the records), None elsewhere."""
+    from .diagnostics import finalize
+
+    def strip(p):
+        return p if chain_arrays else {k: v for k, v in p.items() if k not in ("chain_mean", "chain_var")}
+
+    mine = {k: strip(p) for k, p in partials.items()}
+    import torch.distributed as dist
+
+    if not dist.is_available() or not dist.is_initialized():
+        got = [mine]
+    else:
+        rank = dist.get_rank(group)
+        got = [None] * dist.get_world_size(group) if rank == 0 else None
+        dist.gather_object(mine, got, dst=0, group=group)
+        if rank != 0:
+            return None
+    out = {}
+    for k in got[0]:
+        parts = [g[k] for g in got]
+        total = sum(int(p["nchains"]) for p in parts)
+        if total != int(nchains_total):
+            raise ValueError(f"gather_summary: the ranks hold {total} chains of {k}, expected {nchains_total}")
+        out[k] = finalize(parts, chain_arrays=chain_arrays)
+    return out
