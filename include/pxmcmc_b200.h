@@ -297,6 +297,22 @@ int pxm_stats_accumulate(double* d_acc, const void* d_x, long long n, long long 
 int pxm_stats_partials(const double* d_acc, long long n, long long nchains, int mode, long long nsamples,
                        double* d_partial, double* d_chain_mean, double* d_chain_var, void* stream);
 
+/* ---- rank-normalised convergence diagnostics of stored chains ---------------------
+ * (no counterpart in the reference.)  Column col < ncols of d_chain holds the S = m n samples of m chains, x[c][i] =
+ * d_chain[(c n + i) ld + col] (the layout of a tracked [nchains][nsamples][nparams] array).  Per column, as defined in
+ * DESIGN.md 7b (Vehtari et al. 2021; ArviZ rhat(method="rank"), ess(method="bulk" | "tail")):
+ *   d_rhat[col]      rank-normalised split-R-hat, the larger of the bulk and the folded (|x - median|) R; NaN when
+ *                    either is NaN;
+ *   d_ess_bulk[col]  ESS of the rank-normalised split chains;
+ *   d_ess_tail[col]  the smaller ESS of the split indicators 1[x <= q05] and 1[x <= q95] (numpy's linear quantiles
+ *                    over all S samples).
+ * All three are NaN for a column with a non-finite sample, and for every column when n < 4.  S <=
+ * pxm_quantile_columns_max_samples().  d_scratch: pxm_rank_diagnostics_scratch_doubles(m, n, ncols) doubles (the
+ * columns, transposed); the query returns -1 on a bad argument. */
+long long pxm_rank_diagnostics_scratch_doubles(long long m, long long n, long long ncols);
+int pxm_rank_diagnostics(const double* d_chain, long long m, long long n, long long ncols, long long ld,
+                         double* d_scratch, double* d_rhat, double* d_ess_bulk, double* d_ess_tail, void* stream);
+
 /* ---- measurement aids (bench.py) ---------------------------------------------
  * pxm_profile_begin/end bracket a region in which every library call records a
  * CUDA-event pair on its launching stream; end() returns the summed device time

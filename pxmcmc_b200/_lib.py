@@ -101,6 +101,8 @@ SIGNATURES = {
     "pxm_stats_reset": (_i, [_vp, _ll, _ll, _i, _vp]),
     "pxm_stats_accumulate": (_i, [_vp, _vp, _ll, _ll, _i, _ll, _ll, _vp, _vp]),
     "pxm_stats_partials": (_i, [_vp, _ll, _ll, _i, _ll, _vp, _vp, _vp, _vp]),
+    "pxm_rank_diagnostics_scratch_doubles": (_ll, [_ll, _ll, _ll]),
+    "pxm_rank_diagnostics": (_i, [_vp, _ll, _ll, _ll, _ll, _vp, _vp, _vp, _vp, _vp]),
     "pxm_profile_begin": (_i, [_i]),
     "pxm_profile_end": (_i, [C.POINTER(_d), C.POINTER(_ll)]),
     "pxm_launch_count": (_ll, []),

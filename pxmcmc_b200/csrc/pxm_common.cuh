@@ -79,6 +79,13 @@ PXM_HD size_t pxm_il_index(int row, int col, int nld) {
   return ((size_t)(row >> 2) * (size_t)nld + (size_t)col) * 4 + (size_t)(row & 3);
 }
 
+// numpy's _lerp (quantile method "linear"): a + (b-a) t, or b - (b-a)(1-t) when t >= 0.5.  Explicitly rounded
+// products, so that no translation unit contracts them into an FMA numpy does not evaluate.
+__device__ __forceinline__ double pxm_lerp_np(double a, double b, double t) {
+  const double d = b - a;
+  return (t >= 0.5) ? __dsub_rn(b, __dmul_rn(d, 1.0 - t)) : __dadd_rn(a, __dmul_rn(d, t));
+}
+
 PXM_HD int pxm_round_up(int x, int m) { return (x + m - 1) / m * m; }
 PXM_HD int pxm_ceil_div(int x, int m) { return (x + m - 1) / m; }
 

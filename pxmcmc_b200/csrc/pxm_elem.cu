@@ -604,12 +604,8 @@ __global__ void k_csr_spmv_multi(const int* __restrict__ indptr, const int* __re
 // Column quantiles of a stored chain [nsamples][ld] (np.quantile(chain, (q_a, q_b), axis=0), method
 // "linear": /root/reference/pxmcmc/uncertainty.py:7-16).  A CTA keeps C adjacent columns in shared
 // memory (rows arrive as C consecutive doubles: coalesced), sorts every column with a bitonic network
-// and interpolates exactly like numpy's _lerp: a + (b-a) t, or b - (b-a)(1-t) when t >= 0.5.
+// and interpolates exactly like numpy's _lerp (pxm_lerp_np).
 // ---------------------------------------------------------------------------
-__device__ __forceinline__ double lerp_np(double a, double b, double t) {
-  const double d = b - a;
-  return (t >= 0.5) ? b - d * (1.0 - t) : a + d * t;
-}
 __global__ void k_quantile_columns(const double* __restrict__ chain, long long nsamples, long long ncols, long long ld,
                                    int npad, int C, long long lo_a, double g_a, long long lo_b, double g_b,
                                    double* __restrict__ out_a, double* __restrict__ out_b) {
@@ -644,8 +640,8 @@ __global__ void k_quantile_columns(const double* __restrict__ chain, long long n
   for (int c = threadIdx.x; c < nc; c += blockDim.x) {
     const double* col = qs + c * cs;
     const long long hi_a = min(lo_a + 1, nsamples - 1), hi_b = min(lo_b + 1, nsamples - 1);
-    out_a[col0 + c] = lerp_np(col[lo_a], col[hi_a], g_a);
-    out_b[col0 + c] = lerp_np(col[lo_b], col[hi_b], g_b);
+    out_a[col0 + c] = pxm_lerp_np(col[lo_a], col[hi_a], g_a);
+    out_b[col0 + c] = pxm_lerp_np(col[lo_b], col[hi_b], g_b);
   }
 }
 

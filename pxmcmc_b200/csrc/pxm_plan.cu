@@ -7,6 +7,7 @@
 //     [ring FFT in] -> [DMMA contraction over rings] -> [DMMA contraction over l] -> [ring FFT out]
 // with stages dropped at the harmonic-space boundary of the pyssht-level calls.
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstring>
 #include <map>
@@ -1602,6 +1603,25 @@ int pxm_stats_partials(const double* d_acc, long long n, long long nchains, int 
   ProfScope _ps(2, (cudaStream_t)stream);
   return pxm_launch_stats_partials(d_acc, (size_t)n, (size_t)nchains, mode, nsamples, d_partial, d_chain_mean,
                                    d_chain_var, (cudaStream_t)stream);
+}
+
+long long pxm_rank_diagnostics_scratch_doubles(long long m, long long n, long long ncols) {
+  if (m < 1 || n < 1 || ncols < 0 || m * n > pxm_quantile_max_samples() || ncols > INT_MAX) {
+    pxm_set_error("bad argument: rank_diagnostics: m >= 1, n >= 1, m n <= 16384 samples per column, 0 <= ncols < 2^31");
+    return -1;
+  }
+  return m * n * ncols;
+}
+
+int pxm_rank_diagnostics(const double* d_chain, long long m, long long n, long long ncols, long long ld,
+                         double* d_scratch, double* d_rhat, double* d_ess_bulk, double* d_ess_tail, void* stream) {
+  PXM_REQUIRE(pxm_rank_diagnostics_scratch_doubles(m, n, ncols) >= 0,
+              "rank_diagnostics: m >= 1, n >= 1, m n <= 16384 samples per column, 0 <= ncols < 2^31");
+  PXM_REQUIRE(ld >= ncols && ld >= 1, "rank_diagnostics: leading dimension ld >= ncols");
+  PXM_REQUIRE(ncols == 0 || (d_chain && d_scratch && d_rhat && d_ess_bulk && d_ess_tail), "rank_diagnostics: null pointer");
+  ProfScope _ps(2, (cudaStream_t)stream);
+  return pxm_launch_rank_diagnostics(d_chain, m, n, ncols, ld, d_scratch, d_rhat, d_ess_bulk, d_ess_tail,
+                                     (cudaStream_t)stream);
 }
 
 int pxm_csr_spmv(const int* d_indptr, const int* d_indices, const double* d_vals, const void* d_x, void* d_y,

@@ -152,4 +152,7 @@ int pxm_launch_stats_accumulate(double* acc, const void* x, size_t n, size_t nch
 int pxm_launch_stats_partials(const double* acc, size_t n, size_t nchains, int mode, long long nsamples, double* rec,
                               double* cmean, double* cvar, cudaStream_t st);
 
+int pxm_launch_rank_diagnostics(const double* chain, long long m, long long n, long long ncols, long long ld,
+                                double* scratch, double* rhat, double* ess_bulk, double* ess_tail, cudaStream_t st);
+
 int pxm_debug_naive();

@@ -502,3 +502,19 @@ def stats_partials_dev(acc, n, nchains, mode, nsamples, per_chain=True):
     check(lib.pxm_stats_partials(ptr(acc), int(n), int(nchains), int(mode), int(nsamples), ptr(rec), ptr(cm), ptr(cv),
                                  stream_ptr()))
     return rec, cm, cv
+
+
+def rank_diagnostics_dev(x, m, n):
+    """(rhat, ess_bulk, ess_tail) [ncols] device tensors of the columns of x, a float64 CUDA tensor [m n, ncols] with
+    unit column stride whose row c n + i is sample i of chain c (pxm_rank_diagnostics)"""
+    if x.dtype != FDT or x.dim() != 2 or x.shape[0] != m * n or (x.shape[1] > 1 and x.stride(1) != 1):
+        raise ValueError("rank_diagnostics: x must be a float64 [m n, ncols] tensor with unit column stride")
+    ncols = x.shape[1]
+    nd = int(lib.pxm_rank_diagnostics_scratch_doubles(int(m), int(n), ncols))
+    if nd < 0:
+        raise _lib.PxmError(lib.pxm_last_error().decode())
+    scratch = torch.empty(nd, dtype=FDT, device=x.device)
+    out = torch.empty((3, ncols), dtype=FDT, device=x.device)
+    check(lib.pxm_rank_diagnostics(ptr(x), int(m), int(n), ncols, max(x.stride(0), 1), ptr(scratch), ptr(out[0]),
+                                   ptr(out[1]), ptr(out[2]), stream_ptr()))
+    return out[0], out[1], out[2]

@@ -18,8 +18,12 @@ h = n // 2, b = max(1, isqrt(n)), a = n // b:
 The device keeps running moments (``pxm_stats_accumulate`` on the tracking grid) and reduces them to partial records
 (``pxm_stats_partials``); ``finalize`` combines the records of any number of chain groups (GPUs, calls) with Chan's
 rule and applies the formulas above.
+
+``rank_diagnostics`` works on STORED samples instead: the rank-normalised split-R-hat and the bulk and tail ESS of
+Vehtari et al. (2021), which need every pooled value (``pxm_rank_diagnostics``, DESIGN.md 7b).
 """
 import math
+from collections import namedtuple
 
 import numpy as np
 
@@ -178,3 +182,55 @@ class StreamingSummary:
             if src.shape != tuple(a.shape):
                 raise ValueError(f"checkpoint summary accumulator {k} has shape {src.shape}, expected {tuple(a.shape)}")
             a.copy_(torch.from_numpy(np.ascontiguousarray(src)))
+
+
+RankDiagnostics = namedtuple("RankDiagnostics", ["rhat", "ess_bulk", "ess_tail"])
+
+
+def rank_diagnostics(chains, max_bytes=2 << 30):
+    """Rank-normalised split-R-hat and bulk / tail ESS of every parameter of stored chains (Vehtari, Gelman, Simpson,
+    Carpenter & Buerkner 2021; what ArviZ's rhat(method="rank") and ess(method="bulk" | "tail") report), on the GPU.
+
+    :param chains: [nchains, nsamples, nparams] real array (a tracked ``chain`` / ``preds`` of a multi-chain sampler),
+        or [nsamples, nparams] for one chain: numpy (``np.memmap`` included) or a float64 CUDA tensor.  Complex
+        chains: pass ``.real`` and ``.imag`` separately.  nchains * nsamples <= 16 384.
+    :param max_bytes: device memory of one block of columns (the block and its transposed copy); host arrays are
+        uploaded block by block.
+    :return: ``RankDiagnostics(rhat, ess_bulk, ess_tail)``, each [nparams], of the same kind as ``chains``.  All three
+        are NaN for a parameter with a non-finite sample, and for every parameter when nsamples < 4."""
+    from . import device as D
+    from ._lib import lib
+
+    on_dev = D.is_dev(chains)
+    if on_dev:
+        if chains.is_complex():
+            raise TypeError("rank_diagnostics: complex chains; pass .real and .imag separately")
+    else:
+        chains = np.asarray(chains)
+        if np.iscomplexobj(chains):
+            raise TypeError("rank_diagnostics: complex chains; pass .real and .imag separately")
+    if chains.ndim not in (2, 3):
+        raise ValueError(f"rank_diagnostics: expected [nchains, nsamples, nparams] or [nsamples, nparams], got "
+                         f"{chains.ndim} dimensions")
+    m, n, npar = (1,) + tuple(chains.shape) if chains.ndim == 2 else tuple(chains.shape)
+    S, limit = m * n, lib.pxm_quantile_columns_max_samples()
+    if S > limit:
+        raise ValueError(f"rank_diagnostics: {m} x {n} = {S} samples per parameter exceed the {limit} of the "
+                         f"shared-memory sort")
+    step = max(32, int(max_bytes // (16 * max(S, 1))) // 32 * 32)  # columns per block
+    if on_dev:
+        x = chains.reshape(S, npar).to(D.FDT)
+        if npar > 1 and x.stride(1) != 1:
+            x = x.contiguous()
+        out = [x.new_empty(npar) for _ in range(3)]
+        for c0 in range(0, npar, step):
+            for o, r in zip(out, D.rank_diagnostics_dev(x[:, c0:c0 + step], m, n)):
+                o[c0:c0 + step] = r
+        return RankDiagnostics(*out)
+    x = chains.reshape(S, npar)
+    out = np.empty((3, npar))
+    for c0 in range(0, npar, step):
+        res = D.rank_diagnostics_dev(D.to_dev_f(x[:, c0:c0 + step]), m, n)
+        for k in range(3):
+            out[k, c0:c0 + step] = D.to_host(res[k])
+    return RankDiagnostics(out[0], out[1], out[2])
