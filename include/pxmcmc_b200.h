@@ -297,6 +297,28 @@ int pxm_stats_accumulate(double* d_acc, const void* d_x, long long n, long long 
 int pxm_stats_partials(const double* d_acc, long long n, long long nchains, int mode, long long nsamples,
                        double* d_partial, double* d_chain_mean, double* d_chain_var, void* stream);
 
+/* ---- streaming credible intervals ----------------------------------------------
+ * (pxmcmc/uncertainty.py:7-16 takes them from the stored chain.)  numpy's linear quantiles at q_a and q_b of the
+ * npooled = N samples that the logical chains push over a run, per element and component, without storing them
+ * (DESIGN.md 7b).  lo_a, gamma_a, lo_b, gamma_b: numpy's virtual indices of q_a and q_b for N values (0 <= lo < N).
+ * d_x, modes 0 / 1 / 2 and d_j as in pxm_stats_accumulate.  The state keeps the K_lo = min(lo_a + 2, N) smallest and
+ * the K_hi = N - lo_b largest values of every column t < T (T = 2 n in mode 1, column t = part t / n of element
+ * t % n; T = n otherwise): the lower heaps [T][K_lo], the upper heaps [T][K_hi], then a NaN flag row [T] (doubles).
+ * pxm_credible_state_doubles: its size (-1 on a bad argument).  pxm_credible_reset: zero it.
+ * pxm_credible_push: offer one sample of every chain (d_j == NULL) or of the chains with d_j[c] >= 0 (the value of
+ * d_j[c] is not read otherwise); `count` = samples pooled per column before this push (the chains' logical parts
+ * included: 2 per active chain in mode 2).  Pushes come in order and no more than N samples are pooled.
+ * pxm_credible_finalize: after exactly N pooled samples, d_lower / d_upper [T] = numpy's quantiles at q_a / q_b,
+ * lerp(x(lo), x(min(lo + 1, N - 1)), gamma) evaluated as numpy's _lerp does; NaN where a NaN was pushed. */
+long long pxm_credible_state_doubles(long long n, int mode, long long npooled, long long lo_a, long long lo_b);
+int pxm_credible_reset(double* d_state, long long n, int mode, long long npooled, long long lo_a, long long lo_b,
+                       void* stream);
+int pxm_credible_push(double* d_state, const void* d_x, long long n, long long nchains, int mode, long long npooled,
+                      long long lo_a, long long lo_b, long long count, const long long* d_j, void* stream);
+int pxm_credible_finalize(const double* d_state, long long n, int mode, long long npooled, long long lo_a,
+                          double gamma_a, long long lo_b, double gamma_b, double* d_lower, double* d_upper,
+                          void* stream);
+
 /* ---- rank-normalised convergence diagnostics of stored chains ---------------------
  * (no counterpart in the reference.)  Column col < ncols of d_chain holds the S = m n samples of m chains, x[c][i] =
  * d_chain[(c n + i) ld + col] (the layout of a tracked [nchains][nsamples][nparams] array).  Per column, as defined in

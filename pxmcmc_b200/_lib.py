@@ -103,6 +103,10 @@ SIGNATURES = {
     "pxm_stats_partials": (_i, [_vp, _ll, _ll, _i, _ll, _vp, _vp, _vp, _vp]),
     "pxm_rank_diagnostics_scratch_doubles": (_ll, [_ll, _ll, _ll]),
     "pxm_rank_diagnostics": (_i, [_vp, _ll, _ll, _ll, _ll, _vp, _vp, _vp, _vp, _vp]),
+    "pxm_credible_state_doubles": (_ll, [_ll, _i, _ll, _ll, _ll]),
+    "pxm_credible_reset": (_i, [_vp, _ll, _i, _ll, _ll, _ll, _vp]),
+    "pxm_credible_push": (_i, [_vp, _vp, _ll, _ll, _i, _ll, _ll, _ll, _ll, _vp, _vp]),
+    "pxm_credible_finalize": (_i, [_vp, _ll, _i, _ll, _ll, _d, _ll, _d, _vp, _vp, _vp]),
     "pxm_profile_begin": (_i, [_i]),
     "pxm_profile_end": (_i, [C.POINTER(_d), C.POINTER(_ll)]),
     "pxm_launch_count": (_ll, []),

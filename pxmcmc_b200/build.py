@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.environ.get("PXM_LIB_OUT", os.path.join(HERE, "libpxmcmc_b200.so"))
 SOURCES = ["pxm_plan.cu", "pxm_tables.cu", "pxm_legendre.cu", "pxm_fft.cu", "pxm_healpix.cu", "pxm_elem.cu", "pxm_paths.cu", "pxm_stats.cu",
-           "pxm_rank.cu"]
+           "pxm_rank.cu", "pxm_credible.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-Xptxas", "-v"] + os.environ.get("PXM_EXTRA_NVCC_FLAGS", "").split()
 # the elementwise file must not contract a*b+c into FMAs: the reference's numpy

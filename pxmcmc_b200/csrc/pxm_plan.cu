@@ -1624,6 +1624,53 @@ int pxm_rank_diagnostics(const double* d_chain, long long m, long long n, long l
                                      (cudaStream_t)stream);
 }
 
+long long pxm_credible_state_doubles(long long n, int mode, long long npooled, long long lo_a, long long lo_b) {
+  long long klo = 0, khi = 0;
+  const long long T = (mode == 1 ? 2 : 1) * n;
+  if (n < 1 || n > INT_MAX || mode < 0 || mode > 2 || pxm_credible_tails(npooled, lo_a, lo_b, &klo, &khi) != PXM_OK ||
+      klo + khi + 1 > LLONG_MAX / T) {
+    pxm_set_error("bad argument: credible_state_doubles: 1 <= n < 2^31, mode 0, 1 or 2, npooled >= 1, "
+                  "0 <= lo_a, lo_b < npooled");
+    return -1;
+  }
+  return (klo + khi + 1) * T;
+}
+
+int pxm_credible_reset(double* d_state, long long n, int mode, long long npooled, long long lo_a, long long lo_b,
+                       void* stream) {
+  const long long nd = pxm_credible_state_doubles(n, mode, npooled, lo_a, lo_b);
+  PXM_REQUIRE(nd > 0 && d_state != nullptr, "credible_reset: null state or bad size arguments");
+  PXM_CUDA(cudaMemsetAsync(d_state, 0, (size_t)nd * sizeof(double), (cudaStream_t)stream));
+  return PXM_OK;
+}
+
+int pxm_credible_push(double* d_state, const void* d_x, long long n, long long nchains, int mode, long long npooled,
+                      long long lo_a, long long lo_b, long long count, const long long* d_j, void* stream) {
+  long long klo = 0, khi = 0;
+  PXM_REQUIRE(d_state != nullptr && d_x != nullptr, "credible_push: null pointer");
+  PXM_REQUIRE(pxm_credible_state_doubles(n, mode, npooled, lo_a, lo_b) > 0,
+              "credible_push: 1 <= n < 2^31, mode 0, 1 or 2, npooled >= 1, 0 <= lo_a, lo_b < npooled");
+  PXM_REQUIRE(nchains >= 1 && nchains <= INT_MAX, "credible_push: 1 <= nchains < 2^31");
+  PXM_REQUIRE(count >= 0 && count <= npooled, "credible_push: 0 <= count <= npooled");
+  pxm_credible_tails(npooled, lo_a, lo_b, &klo, &khi);
+  ProfScope _ps(2, (cudaStream_t)stream);
+  return pxm_launch_credible_push(d_state, d_x, (size_t)n, (size_t)nchains, mode, klo, khi, count, d_j,
+                                  (cudaStream_t)stream);
+}
+
+int pxm_credible_finalize(const double* d_state, long long n, int mode, long long npooled, long long lo_a,
+                          double gamma_a, long long lo_b, double gamma_b, double* d_lower, double* d_upper,
+                          void* stream) {
+  long long klo = 0, khi = 0;
+  PXM_REQUIRE(d_state != nullptr && d_lower != nullptr && d_upper != nullptr, "credible_finalize: null pointer");
+  PXM_REQUIRE(pxm_credible_state_doubles(n, mode, npooled, lo_a, lo_b) > 0,
+              "credible_finalize: 1 <= n < 2^31, mode 0, 1 or 2, npooled >= 1, 0 <= lo_a, lo_b < npooled");
+  pxm_credible_tails(npooled, lo_a, lo_b, &klo, &khi);
+  ProfScope _ps(2, (cudaStream_t)stream);
+  return pxm_launch_credible_finalize(d_state, (size_t)n, mode, npooled, klo, khi, lo_a, gamma_a, lo_b, gamma_b,
+                                      d_lower, d_upper, (cudaStream_t)stream);
+}
+
 int pxm_csr_spmv(const int* d_indptr, const int* d_indices, const double* d_vals, const void* d_x, void* d_y,
                  int nrows, long long ncols, long long nchains, void* stream) {
   ProfScope _ps(2, (cudaStream_t)stream);

@@ -155,4 +155,11 @@ int pxm_launch_stats_partials(const double* acc, size_t n, size_t nchains, int m
 int pxm_launch_rank_diagnostics(const double* chain, long long m, long long n, long long ncols, long long ld,
                                 double* scratch, double* rhat, double* ess_bulk, double* ess_tail, cudaStream_t st);
 
+int pxm_credible_tails(long long npooled, long long lo_a, long long lo_b, long long* klo, long long* khi);
+int pxm_launch_credible_push(double* st, const void* x, size_t n, size_t nchains, int mode, long long klo,
+                             long long khi, long long count, const long long* d_j, cudaStream_t s);
+int pxm_launch_credible_finalize(const double* st, size_t n, int mode, long long npooled, long long klo, long long khi,
+                                 long long lo_a, double g_a, long long lo_b, double g_b, double* out_lo,
+                                 double* out_hi, cudaStream_t s);
+
 int pxm_debug_naive();

@@ -518,3 +518,45 @@ def rank_diagnostics_dev(x, m, n):
     check(lib.pxm_rank_diagnostics(ptr(x), int(m), int(n), ncols, max(x.stride(0), 1), ptr(scratch), ptr(out[0]),
                                    ptr(out[1]), ptr(out[2]), stream_ptr()))
     return out[0], out[1], out[2]
+
+
+# ---------------------------------------------------------------------------
+# streaming credible intervals (pxm_credible_*): tail heaps in a flat float64 tensor in the library's layout; `tails`
+# = (npooled, lo_a, gamma_a, lo_b, gamma_b) as diagnostics.credible_tails gives them
+# ---------------------------------------------------------------------------
+def credible_state_doubles(n, mode, tails):
+    N, lo_a, _, lo_b, _ = tails
+    nd = int(lib.pxm_credible_state_doubles(int(n), int(mode), int(N), int(lo_a), int(lo_b)))
+    if nd < 0:
+        raise _lib.PxmError(lib.pxm_last_error().decode())
+    return nd
+
+
+def credible_state(n, mode, tails):
+    """zeroed tail heaps of `n` elements (mode 0 real part, 1 re + im, 2 packed pairs)"""
+    N, lo_a, _, lo_b, _ = tails
+    st = torch.empty(credible_state_doubles(n, mode, tails), dtype=FDT, device=dev())
+    check(lib.pxm_credible_reset(ptr(st), int(n), int(mode), int(N), int(lo_a), int(lo_b), stream_ptr()))
+    return st
+
+
+def credible_push_dev(st, x, mode, tails, count, d_j=None):
+    """offer one sample of every chain of x [nchains, n] (with d_j: of the chains whose entry is >= 0); `count`
+    samples are pooled per column before this push"""
+    x2, _ = batch2d(x)
+    if x2.dtype != CDT or not x2.is_contiguous():
+        raise ValueError("credible_push: x must be a contiguous complex128 [nchains, n] tensor")
+    if d_j is not None and (d_j.dtype != torch.int64 or d_j.numel() != x2.shape[0]):
+        raise ValueError("credible_push: d_j must be an int64 tensor with one entry per chain")
+    N, lo_a, _, lo_b, _ = tails
+    check(lib.pxm_credible_push(ptr(st), ptr(x2), x2.shape[1], x2.shape[0], int(mode), int(N), int(lo_a), int(lo_b),
+                                int(count), ptr(d_j), stream_ptr()))
+
+
+def credible_finalize_dev(st, n, mode, tails):
+    """(lower, upper) device tensors [ncomp, n] (ncomp = 2 in mode 1, else 1)"""
+    N, lo_a, g_a, lo_b, g_b = tails
+    out = torch.empty((2, 2 if mode == 1 else 1, int(n)), dtype=FDT, device=st.device)
+    check(lib.pxm_credible_finalize(ptr(st), int(n), int(mode), int(N), int(lo_a), float(g_a), int(lo_b), float(g_b),
+                                    ptr(out[0]), ptr(out[1]), stream_ptr()))
+    return out[0], out[1]

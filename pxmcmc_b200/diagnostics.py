@@ -52,17 +52,21 @@ class Summary:
     def wavelet_maps(self, name, L, B, J_min):
         """statistic `name` ([..., n] over the wavelet coefficients) split into one MW (theta, phi) map per scale, as
         `uncertainty.wavelet_credible_interval_range` does"""
-        from .utils import _multires_bandlimits
+        return _wavelet_maps(getattr(self, name), name, L, B, J_min)
 
-        v = np.asarray(getattr(self, name))
-        maps, start = [], 0
-        for bl in _multires_bandlimits(L, B, J_min):
-            length = bl * (2 * bl - 1)
-            maps.append(v[..., start:start + length].reshape(v.shape[:-1] + (bl, 2 * bl - 1)))
-            start += length
-        if start != v.shape[-1]:
-            raise ValueError(f"{name} has {v.shape[-1]} entries, the wavelet tiling {start}")
-        return maps
+
+def _wavelet_maps(v, name, L, B, J_min):
+    from .utils import _multires_bandlimits
+
+    v = np.asarray(v)
+    maps, start = [], 0
+    for bl in _multires_bandlimits(L, B, J_min):
+        length = bl * (2 * bl - 1)
+        maps.append(v[..., start:start + length].reshape(v.shape[:-1] + (bl, 2 * bl - 1)))
+        start += length
+    if start != v.shape[-1]:
+        raise ValueError(f"{name} has {v.shape[-1]} entries, the wavelet tiling {start}")
+    return maps
 
 
 def _chan(a, b):
@@ -182,6 +186,99 @@ class StreamingSummary:
             if src.shape != tuple(a.shape):
                 raise ValueError(f"checkpoint summary accumulator {k} has shape {src.shape}, expected {tuple(a.shape)}")
             a.copy_(torch.from_numpy(np.ascontiguousarray(src)))
+
+
+def credible_tails(npooled, alpha):
+    """(npooled, lo_a, gamma_a, lo_b, gamma_b): numpy's linear-quantile virtual indices of alpha / 2 and 1 - alpha / 2
+    among npooled values, evaluated as `uncertainty.credible_interval_range` evaluates them"""
+    from .uncertainty import _virtual_index
+
+    N = int(npooled)
+    return (N,) + _virtual_index(N, alpha / 2) + _virtual_index(N, 1 - alpha / 2)
+
+
+class CredibleIntervals:
+    """(1 - alpha) credible intervals of one target (`PxMCMC(credible=...)`): ``lower`` and ``upper`` are numpy's
+    linear quantiles at alpha / 2 and 1 - alpha / 2 over the ``npooled`` = nchains * nsamples tracked samples of every
+    element, pooled over the logical chains; ``range = upper - lower`` is what `uncertainty.credible_interval_range`
+    gives for the stored samples.  Real components: [n]; complex chains: a leading axis of 2 (re, im)."""
+
+    def __init__(self, alpha, nchains, nsamples, lower, upper):
+        self.alpha, self.nchains, self.nsamples = float(alpha), int(nchains), int(nsamples)
+        self.npooled = self.nchains * self.nsamples
+        self.lower, self.upper = np.asarray(lower), np.asarray(upper)
+        self.range = self.upper - self.lower
+
+    def wavelet_maps(self, name, L, B, J_min):
+        """`lower`, `upper` or `range` split into one MW (theta, phi) map per wavelet scale (`Summary.wavelet_maps`)"""
+        return _wavelet_maps(getattr(self, name), name, L, B, J_min)
+
+
+class StreamingCredible:
+    """Device tail heaps of the targets one sampler bounds (`PxMCMC(credible=...)`).  `targets`: {name: (n, nchains,
+    mode)} with n the vector length, nchains the device chains and mode as in pxm_credible_push (all targets of a
+    sampler pool the same logical chains).  `count`: samples pooled per element so far."""
+
+    def __init__(self, targets, nsamples, alpha):
+        import torch
+
+        from . import device as D
+
+        self.layout = {k: tuple(int(x) for x in v) for k, v in targets.items()}
+        _, nch, mode = next(iter(self.layout.values()))
+        self.parts = 2 if mode == 2 else 1  # logical chains per device chain
+        self.alpha, self.nsamples = float(alpha), int(nsamples)
+        self.nchains = nch * self.parts
+        self.tails = credible_tails(self.nchains * self.nsamples, self.alpha)
+        need = sum(8 * D.credible_state_doubles(n, m, self.tails) for n, _, m in self.layout.values())
+        free = torch.cuda.mem_get_info(D.dev())[0]
+        if need > free:
+            raise ValueError(f"credible: the tail heaps of {self.nchains} x {self.nsamples} pooled samples at alpha = "
+                             f"{self.alpha} need {need} bytes of device memory, {free} are free (fewer samples or a "
+                             f"larger alpha need less)")
+        self.heaps = {k: D.credible_state(n, m, self.tails) for k, (n, _, m) in self.layout.items()}
+        self.count = 0
+
+    def push(self, samples, d_j=None, nactive=None):
+        """one push per target of `samples` = {target: [nchains, n] device tensor}; `nactive`: chains with d_j >= 0
+        (known on the host, so the pooled count needs no synchronisation); None: every chain"""
+        from . import device as D
+
+        for k, (_, nch, mode) in self.layout.items():
+            D.credible_push_dev(self.heaps[k], samples[k], mode, self.tails, self.count, d_j)
+        self.count += (nch if nactive is None else int(nactive)) * self.parts
+
+    def intervals(self):
+        """{target: CredibleIntervals} (one pxm_credible_finalize launch per target)"""
+        from . import device as D
+
+        if self.count != self.tails[0]:
+            raise RuntimeError(f"credible: {self.count} of {self.tails[0]} samples pooled")
+        out = {}
+        for k, (n, _, mode) in self.layout.items():
+            lo, hi = (D.to_host(a) for a in D.credible_finalize_dev(self.heaps[k], n, mode, self.tails))
+            if mode != 1:
+                lo, hi = lo[0], hi[0]
+            out[k] = CredibleIntervals(self.alpha, self.nchains, self.nsamples, lo, hi)
+        return out
+
+    def state(self):
+        """host copies of the heaps and the pooled count (checkpoints)"""
+        from . import device as D
+
+        d = {k: D.to_host(a) for k, a in self.heaps.items()}
+        d["count"] = np.int64(self.count)
+        return d
+
+    def load(self, arrays):
+        import torch
+
+        for k, a in self.heaps.items():
+            src = np.asarray(arrays[k])
+            if src.shape != tuple(a.shape):
+                raise ValueError(f"checkpoint credible heaps {k} have shape {src.shape}, expected {tuple(a.shape)}")
+            a.copy_(torch.from_numpy(np.ascontiguousarray(src)))
+        self.count = int(arrays["count"])
 
 
 RankDiagnostics = namedtuple("RankDiagnostics", ["rhat", "ess_bulk", "ess_tail"])

@@ -14,6 +14,9 @@ sequence of libpxmcmc_b200 kernels.  Two extra keyword-only knobs:
 * ``summarise=("chain",)`` or ``("chain", "predictions")`` keeps streaming posterior summaries on the device (mean,
   variance, split-R-hat, ESS; see `diagnostics`) instead of, or besides, the tracked arrays: ``sampler.summary`` after
   ``run()``.
+* ``credible=("chain",)`` or ``("chain", "predictions")`` keeps the (1 - ``credible_alpha``) credible intervals of
+  every element on the device, exactly numpy's quantiles of the samples the tracked arrays would hold, without storing
+  them: ``sampler.credible_intervals`` after ``run()``.
 """
 import numpy as np
 import torch
@@ -65,7 +68,7 @@ class PxMCMC:
     """Common machinery (pxmcmc/mcmc.py:46-140)."""
 
     def __init__(self, forward, prior, mcmcparams=PxMCMCParams(), *, noise="host", nchains=1, seed=0, stream0=0,
-                 spill_dir=None, async_spill=True, summarise=None):
+                 spill_dir=None, async_spill=True, summarise=None, credible=None, credible_alpha=0.05):
         """`spill_dir`: directory in which the two large tracked arrays (`chain`, `preds`) live as .npy memory maps
         instead of host RAM (SURVEY.md 8(f)1: 5 000 x 1.22 M samples of config 4 are 49 GB).  `async_spill`: tracked
         samples leave the device through pinned staging buffers on a copy stream while the chain keeps iterating
@@ -73,7 +76,11 @@ class PxMCMC:
         `summarise`: None, ("chain",) or ("chain", "predictions"): running moments of every tracked-grid sample are
         kept on the device, independently of `track` (one kernel launch per grid sample and target, no host
         synchronisation, no stored samples); after `run()`, `summary` = {target: diagnostics.Summary} and
-        `summary_partials()` the raw partial records (multi-GPU: sharding.gather_summary)."""
+        `summary_partials()` the raw partial records (multi-GPU: sharding.gather_summary).
+        `credible`: None, ("chain",) or ("chain", "predictions"): the alpha / 2 and 1 - alpha / 2 tails of every
+        tracked-grid sample are kept on the device (alpha = `credible_alpha`, one kernel launch per grid sample and
+        target, about alpha of the stored chain's memory); after `run()`, `credible_intervals` = {target:
+        diagnostics.CredibleIntervals}, bit for bit numpy's quantiles of the samples the tracked arrays would hold."""
         self.forward = forward
         self.prior = prior
         self.spill_dir = spill_dir
@@ -89,6 +96,12 @@ class PxMCMC:
         self._step_counter = 0
         self._summarise = self._check_summarise(summarise)
         self._stats = None
+        self._credible = self._check_summarise(credible, "credible")
+        alpha = float(credible_alpha)
+        if not 0.0 < alpha < 1.0:
+            raise ValueError(f"credible_alpha must lie in (0, 1), got {credible_alpha}")
+        self._credible_alpha = alpha
+        self._cred, self.credible_intervals = None, None
         self._initialise_tracking_arrays()
 
     # ------------------------------------------------------------------ helpers
@@ -323,6 +336,8 @@ class PxMCMC:
                 d["track_" + name] = getattr(self, name)
         if self._stats is not None:
             d.update({"stats_" + k: v for k, v in self._stats.state().items()})
+        if self._cred is not None:
+            d.update({"cred_" + k: v for k, v in self._cred.state().items()})
         kind, keys, pos, has_gauss, cached = np.random.get_state()
         d.update(rng_keys=keys, rng_pos=pos, rng_has_gauss=has_gauss, rng_cached=cached)
         tmp = path + ".tmp.npz"
@@ -348,10 +363,17 @@ class PxMCMC:
                     raise ValueError(f"checkpoint carries no summary accumulators for {missing}: it was written by a "
                                      "sampler without summarise=...")
                 self._stats.load({k: f["stats_" + k] for k in self._stats.acc})
+            if self._cred is not None:
+                keys = list(self._cred.heaps) + ["count"]
+                missing = [k for k in keys if "cred_" + k not in f.files]
+                if missing:
+                    raise ValueError(f"checkpoint carries no credible-interval heaps for {missing}: it was written by "
+                                     "a sampler without credible=...")
+                self._cred.load({k: f["cred_" + k] for k in keys})
             self._step_counter = int(f["step_counter"])
             self.delta = float(f["delta"])
             np.random.set_state(("MT19937", f["rng_keys"], int(f["rng_pos"]), int(f["rng_has_gauss"]), float(f["rng_cached"])))
-            return {k: f[k] for k in f.files if not k.startswith(("track_", "rng_", "stats_"))}
+            return {k: f[k] for k in f.files if not k.startswith(("track_", "rng_", "stats_", "cred_"))}
 
     def save_checkpoint(self, path, i, j, X_curr, curr_preds):
         """Everything `run(resume=path)` needs to continue the chain exactly where it stands after iteration
@@ -383,46 +405,56 @@ class PxMCMC:
         return w_re, w_im
 
     # ------------------------------------------------------------------ streaming posterior summaries
-    def _check_summarise(self, summarise):
+    def _check_summarise(self, summarise, option="summarise"):
         if summarise is None:
             return ()
         if isinstance(summarise, str):
             summarise = (summarise,)
         t = tuple(summarise)
         if not t or len(set(t)) != len(t) or any(k not in ("chain", "predictions") for k in t):
-            raise ValueError('summarise must be None, ("chain",) or ("chain", "predictions")')
+            raise ValueError(f'{option} must be None, ("chain",) or ("chain", "predictions")')
         if getattr(self.forward, "_pxm_allreduce", None) is not None:
-            raise NotImplementedError("summarise: streaming summaries of m-sharded single-chain runs are not implemented "
-                                      "(each rank holds only part of every sample)")
+            raise NotImplementedError(f"{option}: streaming {'summaries' if option == 'summarise' else 'intervals'} of "
+                                      "m-sharded single-chain runs are not implemented (each rank holds only part of "
+                                      "every sample)")
         return t
 
     def _stats_begin(self, nchains_dev=None, pairs=False):
         """fresh accumulators at the start of run() (nsamples fixes the half-chain and batch boundaries); modes as in
         pxm_stats_accumulate: the chain is complex (re + im) only with `complex`, predictions are real parts"""
-        from .diagnostics import StreamingSummary
+        from .diagnostics import StreamingCredible, StreamingSummary
 
         self._stats, self.summary = None, None
-        if not self._summarise:
-            return
+        self._cred, self.credible_intervals = None, None
         nch = self.nchains if nchains_dev is None else nchains_dev
-        lay = {}
-        if "chain" in self._summarise:
-            lay["chain"] = (self.forward.nparams, nch, 2 if pairs else (1 if self.complex else 0))
-        if "predictions" in self._summarise:
-            lay["predictions"] = (len(self.forward.data), nch, 2 if pairs else 0)
-        self._stats = StreamingSummary(lay, self.nsamples)
 
-    def _stats_push(self, X, P, j=0, d_j=None):
-        """push tracked-grid sample j (per chain: d_j) of the state X and the PIXEL predictions P (may be None when
-        predictions are not summarised)"""
-        if self._stats is None:
-            return
-        if "chain" in self._stats.acc:
-            self._stats.push("chain", X, j, d_j)
-        if "predictions" in self._stats.acc:
-            self._stats.push("predictions", P, j, d_j)
+        def layout(targets):
+            lay = {}
+            if "chain" in targets:
+                lay["chain"] = (self.forward.nparams, nch, 2 if pairs else (1 if self.complex else 0))
+            if "predictions" in targets:
+                lay["predictions"] = (len(self.forward.data), nch, 2 if pairs else 0)
+            return lay
+
+        if self._summarise:
+            self._stats = StreamingSummary(layout(self._summarise), self.nsamples)
+        if self._credible:  # the heaps are sized for the run's pooled sample count
+            self._cred = StreamingCredible(layout(self._credible), self.nsamples, self._credible_alpha)
+
+    def _stats_push(self, X, P, j=0, d_j=None, nactive=None):
+        """push tracked-grid sample j (per chain: d_j; `nactive` chains take one) of the state X and the PIXEL
+        predictions P (may be None when predictions are neither summarised nor bounded)"""
+        if self._stats is not None:
+            if "chain" in self._stats.acc:
+                self._stats.push("chain", X, j, d_j)
+            if "predictions" in self._stats.acc:
+                self._stats.push("predictions", P, j, d_j)
+        if self._cred is not None:
+            self._cred.push({"chain": X, "predictions": P}, d_j, nactive)
 
     def _stats_end(self):
+        if self._cred is not None:
+            self.credible_intervals = self._cred.intervals()
         if self._stats is None:
             return
         from .diagnostics import finalize
@@ -628,7 +660,7 @@ class MYULA(PxMCMC):
                 X_curr, curr_preds = self.iterate(X_curr, curr_preds)
             if i >= self.nburn:
                 if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
-                    P_pix = self._pix(curr_preds) if "predictions" in self._summarise else curr_preds
+                    P_pix = self._pix(curr_preds) if "predictions" in self._summarise + self._credible else curr_preds
                     self._track_dev(j, X_curr, P_pix)
                     self._stats_push(X_curr, P_pix, j)
                     j += 1
@@ -750,6 +782,9 @@ class MYULA(PxMCMC):
         if self._summarise:
             raise NotImplementedError("summarise: iterate_host has no tracking grid (run() does); use a sampler "
                                       "without summarise=...")
+        if self._credible:
+            raise NotImplementedError("credible: iterate_host has no tracking grid (run() does); use a sampler "
+                                      "without credible=...")
         dv = D.dev()
         xh = X_host if D.is_dev(X_host) else torch.from_numpy(np.ascontiguousarray(X_host, dtype=np.complex128))
         if preds_host is None:
@@ -1058,10 +1093,10 @@ class PxMALA(MYULA):
             if on_grid or verbose:
                 st = S.cpu().numpy()  # the only host synchronisation
                 take = [c for c in range(nch) if on_grid and st[c, 9] != 0.0 and js[c] < self.nsamples]
-                if take and self._stats is not None:  # every chain's own sample index, -1: no sample now
+                if take and (self._stats is not None or self._cred is not None):  # own sample index, -1: none now
                     jd = np.full(nch, -1, dtype=np.int64)
                     jd[take] = js[take]
-                    self._stats_push(cur[0], cur[1], d_j=torch.from_numpy(jd).to(dv))
+                    self._stats_push(cur[0], cur[1], d_j=torch.from_numpy(jd).to(dv), nactive=len(take))
                 if take:
                     Xh = D.to_host(cur[0]) if hasattr(self, "chain") else None
                     Ph = D.to_host(cur[1]) if hasattr(self, "preds") else None

@@ -9,7 +9,9 @@ same names go into ``<filename>.npz`` (datasets as arrays, attributes under ``at
 
 Streaming posterior summaries (``PxMCMC(summarise=...)``, an extension) are written, when present, as datasets
 ``summary/<target>/<statistic>`` (plus ``nchains`` and ``nsamples``); ``load_mcmc`` returns them under the same flat
-names and ``summaries`` turns them back into ``diagnostics.Summary`` objects."""
+names and ``summaries`` turns them back into ``diagnostics.Summary`` objects.  Streaming credible intervals
+(``PxMCMC(credible=...)``) likewise go into ``credible/<target>/{lower,upper,range,alpha,nchains,nsamples}``, read back
+by ``credible_intervals``."""
 import os
 
 import numpy as np
@@ -29,6 +31,9 @@ def _collect(mcmc, params, kwargs):
             data[f"summary/{target}/{stat}"] = np.asarray(arr)
         data[f"summary/{target}/nchains"] = np.asarray(sm.nchains)
         data[f"summary/{target}/nsamples"] = np.asarray(sm.nsamples)
+    for target, ci in (getattr(mcmc, "credible_intervals", None) or {}).items():
+        for name in ("lower", "upper", "range", "alpha", "nchains", "nsamples"):
+            data[f"credible/{target}/{name}"] = np.asarray(getattr(ci, name))
     attrs = {k: getattr(params, k) for k in params.__dict__.keys()}
     attrs.update(kwargs)
     return data, attrs
@@ -82,4 +87,15 @@ def summaries(data):
         pre = f"summary/{target}/"
         stats = {k[len(pre):]: data[k] for k in data if k.startswith(pre)}
         out[target] = Summary(int(stats.pop("nchains")), int(stats.pop("nsamples")), **stats)
+    return out
+
+
+def credible_intervals(data):
+    """{target: diagnostics.CredibleIntervals} from the datasets `load_mcmc` returned (empty when the file has none)"""
+    from .diagnostics import CredibleIntervals
+
+    out = {}
+    for target in sorted({k.split("/")[1] for k in data if k.startswith("credible/")}):
+        f = {k: data[f"credible/{target}/{k}"] for k in ("alpha", "nchains", "nsamples", "lower", "upper")}
+        out[target] = CredibleIntervals(float(f["alpha"]), int(f["nchains"]), int(f["nsamples"]), f["lower"], f["upper"])
     return out
