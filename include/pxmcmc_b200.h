@@ -225,14 +225,34 @@ int pxm_resid_invcov(const void* d_preds, const void* d_data, const void* d_invc
 int pxm_reduce_scratch_elems(void);
 int pxm_reduce(int kind, const void* a, const void* b, const void* c, const void* d, const double* w, double delta,
                double lmda, long long n, long long nchains, void* d_partial, void* d_out, void* stream);
-/* pxm_lincomb: out = c0 + sum_k coef_k x_k (+ cz*z, z real): SKROCK stages
- * (pxmcmc/mcmc.py:349-368) and the analysis prox assembly (pxmcmc/prior.py:52-53). */
+/* pxm_lincomb: out = c0 + sum_k coef_k x_k (+ cz*z, z real): the analysis prox assembly (pxmcmc/prior.py:52-53);
+ * SKROCK's stages run pxm_skrock_stage. */
 int pxm_lincomb(int nx, const void* const* d_xs, const double* coefs, const double* d_z, double cz, double c0,
                 void* d_out, long long total, void* stream);
 /* pxm_gradlogpi: PxMCMC._gradlogpi (pxmcmc/mcmc.py:84-89): -((X - P)/lmda) - gradg with
  * P = soft(X, T) when d_prox == NULL. */
 int pxm_gradlogpi(const void* d_X, const void* d_prox, const double* d_T, double T_scalar, const void* d_gradg,
                   double lmda, void* d_out, long long n, long long nchains, void* stream);
+/* SKROCK stages (pxmcmc/mcmc.py:338-368; Abdulle, Almuslimani & Vilmart 2018), one kernel each.
+ * pxm_skrock_shift: Y = X + c Z.
+ * pxm_skrock_stage: out = a g + b U + c V + c0 (+ e Z), g = -((P - prox(P))/lmda) - gradg, prox = soft(P, T) when
+ *   d_prox == NULL (T: d_T of length n, or T_scalar).  With noise (noise_mode != 0) P = U + c_shift Z is recomputed in
+ *   registers (stage 1: U = X, d_V = NULL, gradg of Y; Y and Z are not read back), else P = U (stage j >= 2: U = K_{j-1},
+ *   V = K_{j-2}).  The sum runs in the order of the reference's stage expressions, every product rounded: U, g, Z when
+ *   d_V == NULL, else g, U, V; then c0 (added to the real part).  The reference scheme (b = nu_j, c = -1, c0 = k_j)
+ *   equals pxm_gradlogpi + pxm_lincomb bit for bit.  d_out may be d_U or d_V.
+ * Z: noise_mode 1 injected real d_z_re; 2 injected d_z_re + i d_z_im; 3 the Philox normals pxm_philox_normal draws at
+ *   (seed, stream0 + chain, step); 4 complex Philox: one draw of 2n normals per chain, the first n the real and the
+ *   last n the imaginary parts.  d_step != NULL: the step is read from the device (CUDA-graph replays).
+ * All arrays [nchains][n]; the chain comes from the launch grid. */
+int pxm_skrock_shift(const void* d_X, double c, const double* d_z_re, const double* d_z_im, int noise_mode,
+                     unsigned long long seed, unsigned long long step, const unsigned long long* d_step,
+                     unsigned int stream0, void* d_Y, long long n, long long nchains, void* stream);
+int pxm_skrock_stage(const void* d_U, const void* d_V, const void* d_gradg, const void* d_prox, const double* d_T,
+                     double T_scalar, double lmda, double a, double b, double c, double c0, double c_shift, double e,
+                     const double* d_z_re, const double* d_z_im, int noise_mode, unsigned long long seed,
+                     unsigned long long step, const unsigned long long* d_step, unsigned int stream0, void* d_out,
+                     long long n, long long nchains, void* stream);
 /* masked gather / zero-filled scatter with optional per-datum weight:
  * WeakLensing.mask_forward/mask_adjoint/cov_weight (pxmcmc/measurements.py:242-304). */
 int pxm_masked_gather(const void* d_full, const int* d_idx, const double* d_w, void* d_sel, long long nsel,

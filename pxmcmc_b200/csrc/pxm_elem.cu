@@ -426,8 +426,8 @@ __global__ void k_gradlogpi(const cplx* __restrict__ X, const cplx* __restrict__
 }
 
 // ---------------------------------------------------------------------------
-// generic complex linear combination with real coefficients (SKROCK stages,
-// analysis-setting prox assembly):  out = c0 + sum_k a_k x_k  (+ cz * z, z real)
+// generic complex linear combination with real coefficients (analysis-setting prox
+// assembly; SKROCK's stages run k_skrock_stage):  out = c0 + sum_k a_k x_k  (+ cz * z, z real)
 // (/root/reference/pxmcmc/mcmc.py:349-368, prior.py:52-53)
 // ---------------------------------------------------------------------------
 struct LinArgs {
@@ -454,6 +454,163 @@ __global__ void k_lincomb(LinArgs p) {
     if (p.z) re += p.cz * p.z[i];
     re += p.c0;
     p.out[i] = make_double2(re, im);
+  }
+}
+
+// ---------------------------------------------------------------------------
+// SKROCK stages (/root/reference/pxmcmc/mcmc.py:338-368 and the published scheme of Abdulle, Almuslimani & Vilmart
+// 2018), one pass per stage instead of gradlogpi + lincomb (+ philox_normal + lincomb at stage 1):
+//   shift:  Y = U + cs Z
+//   stage:  out = a g + b U + c V + c0 (+ e Z),  g = -((P - prox(P))/lmda) - gradg,
+//           P = U + cs Z when Z is present (stage 1: neither Y nor Z is read back), else P = U.
+// Each sum is accumulated in the order of the lincomb terms it replaces (stage 1: U, g, Z; later stages: g, U, V),
+// products rounded on their own (this file is compiled without FMA contraction, as k_lincomb and k_gradlogpi are), so
+// the reference scheme reproduces the composed kernels bit for bit.
+// Z: injected real (mode 1) or real and imaginary (mode 2) normals, or the Philox normals pxm_philox_normal draws at
+// (seed, stream0 + chain, step), regenerated here: mode 3 real, mode 4 complex = one draw of 2n normals per chain, the
+// first n the real and the last n the imaginary parts.
+// grid = (blocks per chain, chains in this launch); a thread owns elements (2 pr, 2 pr + 1) of one chain, so one
+// Box-Muller pair serves both real parts and no 64-bit division runs per element.
+// ---------------------------------------------------------------------------
+struct SkrockArgs {
+  const cplx* U;
+  const cplx* V;      // null at stage 1
+  const cplx* gradg;  // stage only
+  const cplx* prox;   // may be null -> soft(P, T)
+  const double* Tv;   // may be null -> Ts
+  double Ts, lmda;
+  double a, b, c, c0, cs, e;
+  const double* z_re;  // modes 1, 2
+  const double* z_im;  // mode 2
+  int noise_mode;      // 0 none, 1 injected real, 2 injected complex, 3 Philox real, 4 Philox complex
+  unsigned long long seed, step;
+  const unsigned long long* step_ptr;  // may be null; otherwise the step is read from the device (CUDA-graph replays)
+  unsigned int stream0;
+  cplx* out;
+  size_t n;
+};
+
+// the normals of elements e0 and e0 + 1 (when `two`) of `chain`; i0 = chain * n + e0
+__device__ __forceinline__ void skrock_noise(const SkrockArgs& p, size_t chain, size_t e0, size_t i0, bool two,
+                                             double zr[2], double zi[2]) {
+  zr[0] = zr[1] = zi[0] = zi[1] = 0.0;
+  if (p.noise_mode == 1 || p.noise_mode == 2) {
+    zr[0] = p.z_re[i0];
+    if (two) zr[1] = p.z_re[i0 + 1];
+    if (p.noise_mode == 2) {
+      zi[0] = p.z_im[i0];
+      if (two) zi[1] = p.z_im[i0 + 1];
+    }
+  } else if (p.noise_mode >= 3) {
+    const unsigned int stream = p.stream0 + (unsigned int)chain;
+    philox_normal2(p.seed, stream, p.step, e0 >> 1, &zr[0], &zr[1]);
+    if (p.noise_mode == 4) {
+      const size_t k = p.n + e0;  // index of the imaginary part of element e0 in the chain's 2n draw
+      double z0, z1;
+      philox_normal2(p.seed, stream, p.step, k >> 1, &z0, &z1);
+      if (!(k & 1)) {
+        zi[0] = z0;
+        zi[1] = z1;
+      } else {
+        zi[0] = z1;
+        if (two) philox_normal2(p.seed, stream, p.step, (k >> 1) + 1, &zi[1], &z1);
+      }
+    }
+  }
+}
+
+__global__ void k_skrock_shift(SkrockArgs p, size_t chain0) {
+  if (p.step_ptr) p.step = *p.step_ptr;
+  const size_t npairs = (p.n + 1) >> 1, chain = chain0 + blockIdx.y;
+  const bool cz = p.noise_mode == 2 || p.noise_mode == 4;
+  for (size_t pr = blockIdx.x * (size_t)blockDim.x + threadIdx.x; pr < npairs; pr += (size_t)gridDim.x * blockDim.x) {
+    const size_t e0 = 2 * pr, i0 = chain * p.n + e0;
+    const bool two = e0 + 1 < p.n;
+    cplx u[2];
+    u[0] = p.U[i0];
+    u[1] = two ? p.U[i0 + 1] : make_double2(0.0, 0.0);
+    double zr[2], zi[2];
+    skrock_noise(p, chain, e0, i0, two, zr, zi);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      if (h == 1 && !two) break;
+      // lincomb([(1, U)], z=Z, cz=cs) / lincomb([(1, U), (cs, Z_re + i Z_im)]): 0 + 1 U, + cs Z, + 0 (real part)
+      double re = 0.0, im = 0.0;
+      re += u[h].x;
+      im += u[h].y;
+      re += p.cs * zr[h];
+      if (cz) im += p.cs * zi[h];
+      re += 0.0;
+      p.out[i0 + h] = make_double2(re, im);
+    }
+  }
+}
+
+__global__ void k_skrock_stage(SkrockArgs p, size_t chain0) {
+  if (p.step_ptr) p.step = *p.step_ptr;
+  const size_t npairs = (p.n + 1) >> 1, chain = chain0 + blockIdx.y;
+  const bool noise = p.noise_mode != 0, cz = p.noise_mode == 2 || p.noise_mode == 4;
+  for (size_t pr = blockIdx.x * (size_t)blockDim.x + threadIdx.x; pr < npairs; pr += (size_t)gridDim.x * blockDim.x) {
+    const size_t e0 = 2 * pr, i0 = chain * p.n + e0;
+    const bool two = e0 + 1 < p.n;
+    // every input of the pair is requested before any arithmetic
+    cplx u[2], g[2], v[2], px[2];
+    double T[2];
+    u[0] = p.U[i0];
+    g[0] = p.gradg[i0];
+    u[1] = two ? p.U[i0 + 1] : make_double2(0.0, 0.0);
+    g[1] = two ? p.gradg[i0 + 1] : make_double2(0.0, 0.0);
+    if (p.V) {
+      v[0] = p.V[i0];
+      v[1] = two ? p.V[i0 + 1] : make_double2(0.0, 0.0);
+    }
+    if (p.prox) {
+      px[0] = p.prox[i0];
+      px[1] = two ? p.prox[i0 + 1] : make_double2(0.0, 0.0);
+    } else {
+      T[0] = p.Tv ? p.Tv[e0] : p.Ts;
+      T[1] = (p.Tv && two) ? p.Tv[e0 + 1] : p.Ts;
+    }
+    double zr[2], zi[2];
+    skrock_noise(p, chain, e0, i0, two, zr, zi);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      if (h == 1 && !two) break;
+      cplx P = u[h];
+      if (noise) {  // the shift's Y, recomputed in registers (same operations as k_skrock_shift)
+        double re = 0.0, im = 0.0;
+        re += u[h].x;
+        im += u[h].y;
+        re += p.cs * zr[h];
+        if (cz) im += p.cs * zi[h];
+        re += 0.0;
+        P = make_double2(re, im);
+      }
+      if (!p.prox) px[h] = soft_c(P, T[h]);
+      // k_gradlogpi
+      const double gx = -((P.x - px[h].x) / p.lmda) - g[h].x, gy = -((P.y - px[h].y) / p.lmda) - g[h].y;
+      // k_lincomb, terms in the order the stages list them
+      double re = 0.0, im = 0.0;
+      if (p.V) {
+        re += p.a * gx;
+        im += p.a * gy;
+        re += p.b * u[h].x;
+        im += p.b * u[h].y;
+        re += p.c * v[h].x;
+        im += p.c * v[h].y;
+      } else {
+        re += p.b * u[h].x;
+        im += p.b * u[h].y;
+        re += p.a * gx;
+        im += p.a * gy;
+      }
+      if (noise) {
+        re += p.e * zr[h];
+        if (cz) im += p.e * zi[h];
+      }
+      re += p.c0;
+      p.out[i0 + h] = make_double2(re, im);
+    }
   }
 }
 
@@ -900,6 +1057,48 @@ int pxm_launch_lincomb(int nx, const void* const* xs, const double* as, const do
   return PXM_OK;
 }
 
+int pxm_launch_skrock(int stage, const void* U, const void* V, const void* gradg, const void* prox, const double* Tv,
+                      double Ts, double lmda, double a, double b, double c, double c0, double cs, double e,
+                      const double* z_re, const double* z_im, int noise_mode, unsigned long long seed,
+                      unsigned long long step, const unsigned long long* d_step, unsigned int stream0, void* out, size_t n,
+                      size_t nchains, cudaStream_t st) {
+  SkrockArgs p;
+  p.U = (const cplx*)U;
+  p.V = (const cplx*)V;
+  p.gradg = (const cplx*)gradg;
+  p.prox = (const cplx*)prox;
+  p.Tv = Tv;
+  p.Ts = Ts;
+  p.lmda = lmda;
+  p.a = a;
+  p.b = b;
+  p.c = c;
+  p.c0 = c0;
+  p.cs = cs;
+  p.e = e;
+  p.z_re = z_re;
+  p.z_im = z_im;
+  p.noise_mode = noise_mode;
+  p.seed = seed;
+  p.step = step;
+  p.step_ptr = d_step;
+  p.stream0 = stream0;
+  p.out = (cplx*)out;
+  p.n = n;
+  if (!n || !nchains) return PXM_OK;
+  const size_t npairs = (n + 1) / 2;
+  for (size_t c0c = 0; c0c < nchains; c0c += 65535) {
+    const size_t nc = std::min<size_t>(nchains - c0c, 65535);
+    const int per_chain = std::max(1, std::min(grid_for(npairs), (int)((148 * 16 + nc - 1) / nc)));
+    if (stage)
+      k_skrock_stage<<<dim3(per_chain, (unsigned)nc), 256, 0, st>>>(p, c0c);
+    else
+      k_skrock_shift<<<dim3(per_chain, (unsigned)nc), 256, 0, st>>>(p, c0c);
+    PXM_LAUNCHED();
+  }
+  return PXM_OK;
+}
+
 int pxm_launch_gather(int scatter, const void* in, const int* idx, const double* w, void* out, size_t nsel,
                       size_t nfull, size_t nchains, cudaStream_t st) {
   const size_t total = nsel * nchains;
@@ -928,6 +1127,8 @@ int pxm_elem_preload() {
   PXM_CUDA(cudaFuncGetAttributes(&a, k_reduce_stage2));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_gradlogpi));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_lincomb));
+  PXM_CUDA(cudaFuncGetAttributes(&a, k_skrock_shift));
+  PXM_CUDA(cudaFuncGetAttributes(&a, k_skrock_stage));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_gather_w));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_scatter_w));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_r2c));

@@ -1541,6 +1541,36 @@ int pxm_gradlogpi(const void* d_X, const void* d_prox, const double* d_T, double
                               (cudaStream_t)stream);
 }
 
+static bool skrock_noise_ok(int noise_mode, const double* d_z_re, const double* d_z_im) {
+  return noise_mode >= 0 && noise_mode <= 4 && (noise_mode < 1 || noise_mode > 2 || d_z_re != nullptr) &&
+         (noise_mode != 2 || d_z_im != nullptr);
+}
+
+int pxm_skrock_shift(const void* d_X, double c, const double* d_z_re, const double* d_z_im, int noise_mode,
+                     unsigned long long seed, unsigned long long step, const unsigned long long* d_step,
+                     unsigned int stream0, void* d_Y, long long n, long long nchains, void* stream) {
+  ProfScope _ps(2, (cudaStream_t)stream);
+  PXM_REQUIRE(d_X != nullptr && d_Y != nullptr && n >= 0 && nchains >= 0, "skrock_shift: bad argument");
+  PXM_REQUIRE(noise_mode >= 1 && skrock_noise_ok(noise_mode, d_z_re, d_z_im), "skrock_shift: noise_mode 1..4 with its arrays");
+  return pxm_launch_skrock(0, d_X, nullptr, nullptr, nullptr, nullptr, 0.0, 1.0, 0.0, 0.0, 0.0, 0.0, c, 0.0, d_z_re,
+                           d_z_im, noise_mode, seed, step, d_step, stream0, d_Y, (size_t)n, (size_t)nchains,
+                           (cudaStream_t)stream);
+}
+
+int pxm_skrock_stage(const void* d_U, const void* d_V, const void* d_gradg, const void* d_prox, const double* d_T,
+                     double T_scalar, double lmda, double a, double b, double c, double c0, double c_shift, double e,
+                     const double* d_z_re, const double* d_z_im, int noise_mode, unsigned long long seed,
+                     unsigned long long step, const unsigned long long* d_step, unsigned int stream0, void* d_out,
+                     long long n, long long nchains, void* stream) {
+  ProfScope _ps(2, (cudaStream_t)stream);
+  PXM_REQUIRE(d_U != nullptr && d_gradg != nullptr && d_out != nullptr && n >= 0 && nchains >= 0,
+              "skrock_stage: bad argument");
+  PXM_REQUIRE(skrock_noise_ok(noise_mode, d_z_re, d_z_im), "skrock_stage: noise_mode 0..4 with its arrays");
+  return pxm_launch_skrock(1, d_U, d_V, d_gradg, d_prox, d_T, T_scalar, lmda, a, b, c, c0, c_shift, e, d_z_re, d_z_im,
+                           noise_mode, seed, step, d_step, stream0, d_out, (size_t)n, (size_t)nchains,
+                           (cudaStream_t)stream);
+}
+
 int pxm_masked_gather(const void* d_full, const int* d_idx, const double* d_w, void* d_sel, long long nsel,
                       long long nfull, long long nchains, void* stream) {
   ProfScope _ps(2, (cudaStream_t)stream);

@@ -133,6 +133,11 @@ int pxm_launch_lincomb(int nx, const void* const* xs, const double* as, const do
                        void* out, size_t total, cudaStream_t st);
 int pxm_launch_gradlogpi(const void* X, const void* prox, const double* Tv, double Ts, const void* gradg, double lmda,
                          void* out, size_t n, size_t nchains, cudaStream_t st);
+int pxm_launch_skrock(int stage, const void* U, const void* V, const void* gradg, const void* prox, const double* Tv,
+                      double Ts, double lmda, double a, double b, double c, double c0, double cs, double e,
+                      const double* z_re, const double* z_im, int noise_mode, unsigned long long seed,
+                      unsigned long long step, const unsigned long long* d_step, unsigned int stream0, void* out, size_t n,
+                      size_t nchains, cudaStream_t st);
 int pxm_launch_gather(int scatter, const void* in, const int* idx, const double* w, void* out, size_t nsel,
                       size_t nfull, size_t nchains, cudaStream_t st);
 int pxm_launch_lm_convert(int to_internal, void* flm, double* H, const unsigned long long* d_slot_off,

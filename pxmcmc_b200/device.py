@@ -413,6 +413,43 @@ def gradlogpi_dev(X, prox, Tvec, Tscalar, gradg, lmda):
     return out[0] if was1 else out
 
 
+class SkrockNoise:
+    """the Z of one SKROCK step for pxm_skrock_shift / pxm_skrock_stage: injected real normals `re` [nchains, n] (and
+    `im` for complex chains), or, with re = None, the Philox normals pxm_philox_normal draws at (seed, stream0 + chain,
+    step) -- step read from the int64 device tensor `dstep` when given -- real or (`complex`) one 2n draw per chain"""
+
+    def __init__(self, re=None, im=None, *, complex=False, seed=0, step=0, stream0=0, dstep=None):
+        self.re, self.im = (None if re is None else to_dev_f(re)), (None if im is None else to_dev_f(im))
+        if self.re is None:
+            self.mode = 4 if complex else 3
+        else:
+            self.mode = 2 if self.im is not None else 1
+        self.seed, self.step, self.stream0, self.dstep = int(seed), int(step), int(stream0), dstep
+
+    def args(self):
+        return (ptr(self.re), ptr(self.im), self.mode, self.seed, self.step, ptr(self.dstep), self.stream0)
+
+
+def skrock_shift_dev(X, c, Z, out=None):
+    """Y = X + c Z ([nchains, n] complex; Z a `SkrockNoise`)"""
+    X2, was1 = batch2d(X)
+    out = torch.empty_like(X2) if out is None else batch2d(out)[0]
+    check(lib.pxm_skrock_shift(ptr(X2), float(c), *Z.args(), ptr(out), X2.shape[1], X2.shape[0], stream_ptr()))
+    return out[0] if was1 else out
+
+
+def skrock_stage_dev(U, V, gradg, prox, Tvec, Tscalar, lmda, a, b, c, c0, Z=None, c_shift=0.0, e=0.0, out=None):
+    """one SKROCK stage: a g + b U + c V + c0 (+ e Z), g = grad log pi at P = U (+ c_shift Z); see pxm_skrock_stage.
+    V = None is stage 1.  `out` may be U or V."""
+    U2, was1 = batch2d(U)
+    out = torch.empty_like(U2) if out is None else batch2d(out)[0]
+    zargs = Z.args() if Z is not None else (None, None, 0, 0, 0, None, 0)
+    check(lib.pxm_skrock_stage(ptr(U2), ptr(V), ptr(gradg), ptr(prox), ptr(Tvec), float(Tscalar), float(lmda), float(a),
+                               float(b), float(c), float(c0), float(c_shift), float(e), *zargs, ptr(out), U2.shape[1],
+                               U2.shape[0], stream_ptr()))
+    return out[0] if was1 else out
+
+
 def resid_dev(preds, data, invcov):
     p2, was1 = batch2d(preds)
     out = torch.empty_like(p2)

@@ -203,13 +203,16 @@ class PxMCMC:
         lp, l2, pr = self._logpi_dev(self._state(X), self._state(preds))
         return lp[0], l2[0], pr[0]
 
-    def _gradlogpi_dev(self, Xd, Pd=None):
+    def _gradg_at(self, Xd, Pd=None):
+        """gradg of the predictions of Xd (computed here unless `Pd` is given), as a device tensor"""
         if Pd is None and self._ring_mode():
-            gradg = self.forward.gradg_from_ring(self.forward.forward_ring(Xd))
-        else:
-            if Pd is None:
-                Pd = self._forward_dev(Xd)
-            gradg = D.to_dev_c(self._gradg_dev(self._pix(Pd)))
+            return self.forward.gradg_from_ring(self.forward.forward_ring(Xd))
+        if Pd is None:
+            Pd = self._forward_dev(Xd)
+        return D.to_dev_c(self._gradg_dev(self._pix(Pd)))
+
+    def _gradlogpi_dev(self, Xd, Pd=None):
+        gradg = self._gradg_at(Xd, Pd)
         fused = self._fused_prox()
         if fused is not None:
             return D.gradlogpi_dev(Xd, None, fused[0], fused[1], gradg, self.lmda)
@@ -1311,14 +1314,51 @@ class _GraphedSkrock:
 class SKROCK(PxMCMC):
     """Stochastic orthogonal Runge-Kutta-Chebyshev sampler (pxmcmc/mcmc.py:292-383).
     The reference evaluates K_s by naive recursion (4 059 gradient evaluations at
-    s=10); K_0..K_s are evaluated bottom-up here (s evaluations, identical values)."""
+    s=10); K_0..K_s are evaluated bottom-up here (s evaluations, identical values).
 
-    def __init__(self, forward, prox, mcmcparams=PxMCMCParams(), **kw):
+    `scheme` (keyword-only):
+    * "reference" (default): the recursion exactly as the reference codes it (ratio T_{j-1}(omega_0) / T_j(omega_1), a
+      scalar k_j = 1 added and K_{j-2} subtracted).  It reproduces the reference's chains, but its step multiplies the
+      state by about 1e8 at s = 10 whatever the step size: it does not sample.
+    * "published": SK-ROCK of Abdulle, Almuslimani & Vilmart (2018), as used by Pereyra, Vargas-Mieles & Zygalakis
+      (2020): K_j = mu_j delta grad log pi(K_{j-1}) + nu_j K_{j-1} + kappa_j K_{j-2} with the ratio
+      T_{j-1}(omega_0) / T_j(omega_0) and kappa_j = 1 - nu_j.  Stable for step sizes up to `stability_limit` / Lip,
+      about s^2 times MYULA's."""
+
+    def __init__(self, forward, prox, mcmcparams=PxMCMCParams(), *, scheme="reference", **kw):
+        if scheme not in ("reference", "published"):
+            raise ValueError(f"scheme must be 'reference' or 'published', got {scheme!r}")
+        self._scheme = scheme
         super().__init__(forward, prox, mcmcparams=mcmcparams, **kw)
         self.eta = 0.05
         self.omega_0 = 1 + self.eta / (self.s * self.s)
         self.omega_1 = chebyshev1(self.omega_0, self.s) / cheb1der(self.omega_0, self.s)
         self._recursion_coefs()
+
+    @property
+    def scheme(self):
+        """"reference" or "published" (read-only: the coefficients are fixed at construction)"""
+        return self._scheme
+
+    @property
+    def stability_limit(self):
+        """(omega_0 + 1) / omega_1: the published scheme is stable (|R(p)| <= 1, R(p) = T_s(omega_0 - omega_1 p) /
+        T_s(omega_0) the step's deterministic factor) for p = delta * Lip(grad log pi_lambda) <= stability_limit, where
+        Lip >= 1 / lmda from the Moreau-Yosida term.  17.4 at s = 3, 48.4 at s = 5, 193.6 at s = 10 (the bound usually
+        quoted, (s - 1/2)^2 (2 - 4 eta / 3) - 3/2, is a conservative version of it).  At it |R| = 1 / T_s(omega_0); |R|
+        passes 1 at 2 omega_0 / omega_1, (omega_0 - 1) / omega_1 further.  NaN for the
+        reference scheme, which is stable for no step size."""
+        return (self.omega_0 + 1) / self.omega_1 if self._scheme == "published" else float("nan")
+
+    def _save_ckpt(self, path, **fields):
+        super()._save_ckpt(path, scheme=self._scheme, **fields)
+
+    def _load_ckpt(self, path):
+        with np.load(path if path.endswith(".npz") else path + ".npz", allow_pickle=False) as f:
+            scheme = str(f["scheme"]) if "scheme" in f.files else "reference"  # files written before the option
+        if scheme != self._scheme:
+            raise ValueError(f"checkpoint was written by a SKROCK sampler with scheme={scheme!r}, not {self._scheme!r}")
+        return super()._load_ckpt(path)
 
     def run(self, start_point=None, *, checkpoint=None, checkpoint_every=0, resume=None):
         """the loop of pxmcmc/mcmc.py:308-336.  `checkpoint` / `checkpoint_every` / `resume` as in `MYULA.run`."""
@@ -1361,27 +1401,29 @@ class SKROCK(PxMCMC):
         print("\nDONE")
 
     def _chain_step_dev(self, Xd, Z=None, out=None):
-        """Z: real [nchains, n] normals, or a (real, imaginary) pair when `complex` (pxmcmc/mcmc.py:344-347)"""
+        """Z: real [nchains, n] normals, a (real, imaginary) pair when `complex` (pxmcmc/mcmc.py:344-347), or a
+        `device.SkrockNoise`; None draws it (host RNG, or Philox normals regenerated inside the stage kernels)"""
         n = Xd.shape[-1]
         nch = Xd.shape[0]
+        dstep = None
         if Z is None:
             if self.noise == "device":  # Philox normals, step counter on the host or (graph replays) on the device
                 dstep = getattr(self, "_dstep", None)
                 if dstep is None:
                     self._step_counter += 1
-                if self.complex:
-                    # one draw of 2n normals per chain: the first n are the real, the last n the imaginary parts
-                    z2 = D.philox_normal_dev(nch, 2 * n, self.seed, self._step_counter, self.stream0, dstep=dstep)
-                    Z = (z2[:, :n].contiguous(), z2[:, n:].contiguous())
-                else:
-                    Z = D.philox_normal_dev(nch, n, self.seed, self._step_counter, self.stream0, dstep=dstep)
-                if dstep is not None:
-                    D.check(D.lib.pxm_counter_add(D.ptr(dstep), 1, D.stream_ptr()))
+                # complex: one draw of 2n normals per chain, the first n the real, the last n the imaginary parts
+                Z = D.SkrockNoise(complex=self.complex, seed=self.seed, step=self._step_counter, stream0=self.stream0,
+                                  dstep=dstep)
             else:
                 Z = D.to_dev_f(np.random.randn(n * nch)).reshape(Xd.shape)
                 if self.complex:  # the reference's order: real part, then imaginary part
                     Z = (Z, D.to_dev_f(np.random.randn(n * nch)).reshape(Xd.shape))
-        return self._K_recursion(Xd, self.s, Z, out=out)
+        if not isinstance(Z, D.SkrockNoise):
+            Z = D.SkrockNoise(*Z) if isinstance(Z, tuple) else D.SkrockNoise(Z)
+        out = self._K_recursion(Xd, self.s, Z, out=out)
+        if dstep is not None:
+            D.check(D.lib.pxm_counter_add(D.ptr(dstep), 1, D.stream_ptr()))
+        return out
 
     def capture(self, X_curr):
         """One SKROCK step (s gradient evaluations, ~14 s launches) and its predictions as ONE CUDA graph; needs
@@ -1396,30 +1438,35 @@ class SKROCK(PxMCMC):
         return out if D.is_dev(X) else D.to_host(out[0])
 
     def _K_recursion(self, Xd, s, Z, out=None):
-        """K_s of pxmcmc/mcmc.py:349-368, memoised.  `out` (may be Xd) receives K_s."""
-        sq = np.sqrt(2 * self.delta)
-        K_prev2 = Xd
+        """K_s of pxmcmc/mcmc.py:349-368, memoised, one fused kernel per stage (and the shift Y = X + nu_1 sqrt(2 delta) Z
+        the first gradient is evaluated at).  Z: a `device.SkrockNoise`.  `out` (may be Xd) receives K_s."""
         if s == 0:
             return Xd if out is None else D.copy_into(out, Xd)
-        if isinstance(Z, tuple):  # complex noise: the imaginary part rides as a term with an imaginary unit folded in
-            Zc = torch.complex(Z[0], Z[1])
-            zterm = lambda c: ([(c, Zc)], None, 0.0)  # noqa: E731
-        else:
-            zterm = lambda c: ([], Z, c)  # noqa: E731
-        t, z, cz = zterm(self.nus[1] * sq)
-        Y = D.lincomb_dev([(1.0, Xd)] + t, z=z, cz=cz)
-        t, z, cz = zterm(self.ks[1] * sq)
-        K_prev = D.lincomb_dev([(1.0, Xd), (self.mus[1] * self.delta, self._gradlogpi_dev(Y))] + t, z=z, cz=cz,
-                               out=out if s == 1 else None)
+        sq = np.sqrt(2 * self.delta)
+        Y = D.skrock_shift_dev(Xd, self.nus[1] * sq, Z)
+        K_prev = D.skrock_stage_dev(Xd, None, *self._stage_inputs(Y), self.lmda, self.mus[1] * self.delta, 1.0, 0.0, 0.0,
+                                    Z=Z, c_shift=self.nus[1] * sq, e=self.ks[1] * sq, out=out if s == 1 else None)
+        K_prev2 = Xd
         for j in range(2, s + 1):
-            g = self._gradlogpi_dev(K_prev)
-            K = D.lincomb_dev([(self.mus[j] * self.delta, g), (self.nus[j], K_prev), (-1.0, K_prev2)], c0=self.ks[j],
-                              out=out if j == s else None)
+            # reference: ... + nu_j K_{j-1} + k_j - K_{j-2};  published: ... + nu_j K_{j-1} + kappa_j K_{j-2}
+            c, c0 = (-1.0, self.ks[j]) if self._scheme == "reference" else (self.ks[j], 0.0)
+            K = D.skrock_stage_dev(K_prev, K_prev2, *self._stage_inputs(K_prev), self.lmda, self.mus[j] * self.delta,
+                                   self.nus[j], c, c0, out=out if j == s else None)
             K_prev2, K_prev = K_prev, K
         return K_prev
 
+    def _stage_inputs(self, P):
+        """(gradg, prox, Tvec, Tscalar) of grad log pi at P for the stage kernel: the soft threshold is applied inside
+        it when the prior allows, else prox(P) is given"""
+        gradg = self._gradg_at(P)
+        fused = self._fused_prox()
+        if fused is not None:
+            return gradg, None, fused[0], fused[1]
+        return gradg, self._proxf_dev(P), None, 0.0
+
     def _recursion_coefs(self):
-        """coefficients exactly as the reference computes them (pxmcmc/mcmc.py:370-383)"""
+        """mu_j, nu_j and k_j (reference, exactly as pxmcmc/mcmc.py:370-383 computes them) or kappa_j (published);
+        stage 1 is the same in both schemes"""
         self.mus = np.zeros(self.s + 1)
         self.nus = np.zeros(self.s + 1)
         self.ks = np.zeros(self.s + 1)
@@ -1427,7 +1474,10 @@ class SKROCK(PxMCMC):
         self.nus[1] = self.s * self.omega_1 / 2
         self.ks[1] = self.s * self.omega_1 / self.omega_0
         for j in range(2, self.s + 1):
-            cheb_ratio = chebyshev1(self.omega_0, j - 1) / chebyshev1(self.omega_1, j)
+            if self._scheme == "reference":
+                cheb_ratio = chebyshev1(self.omega_0, j - 1) / chebyshev1(self.omega_1, j)
+            else:
+                cheb_ratio = chebyshev1(self.omega_0, j - 1) / chebyshev1(self.omega_0, j)
             self.mus[j] = 2 * self.omega_1 * cheb_ratio
             self.nus[j] = 2 * self.omega_0 * cheb_ratio
-            self.ks[j] = 1 - self.nus[0]
+            self.ks[j] = 1 - self.nus[0] if self._scheme == "reference" else 1 - self.nus[j]
