@@ -253,6 +253,17 @@ int pxm_skrock_stage(const void* d_U, const void* d_V, const void* d_gradg, cons
                      const double* d_z_re, const double* d_z_im, int noise_mode, unsigned long long seed,
                      unsigned long long step, const unsigned long long* d_step, unsigned int stream0, void* d_out,
                      long long n, long long nchains, void* stream);
+/* pxm_fista_update: one FISTA iteration (Beck & Teboulle 2009) of the synthesis-setting MAP for every chain:
+ *   x_{k+1} = soft(y_k - t gradg, T_scale T),  y_{k+1} = x_{k+1} + beta_k (x_{k+1} - x_k),
+ *   beta_k = (tau_k - 1)/tau_{k+1},  tau_{k+1} = (1 + sqrt(1 + 4 tau_k^2))/2
+ * with gradg the data-fidelity gradient at y_k (T: d_T of length n, or T_scalar).  d_state = {k, tau_k} (doubles;
+ * start from {0, 1}) is read on the device and advanced by the call, so a captured block of iterations replays
+ * unchanged.  d_hist[cap][nchains][2] receives, in slot k mod cap, |x_{k+1} - x_k|^2 and |x_{k+1}|^2 of every chain
+ * (deterministic two-level sums).  d_x_out / d_y_out may be d_x / d_y.  d_partial: scratch of
+ * nchains*pxm_reduce_scratch_elems() complex.  All vectors [nchains][n], nchains <= 65535. */
+int pxm_fista_update(const void* d_y, const void* d_gradg, const void* d_x, const double* d_T, double T_scalar,
+                     double T_scale, double t, double* d_state, void* d_x_out, void* d_y_out, double* d_hist,
+                     long long cap, long long n, long long nchains, void* d_partial, void* stream);
 /* masked gather / zero-filled scatter with optional per-datum weight:
  * WeakLensing.mask_forward/mask_adjoint/cov_weight (pxmcmc/measurements.py:242-304). */
 int pxm_masked_gather(const void* d_full, const int* d_idx, const double* d_w, void* d_sel, long long nsel,

@@ -91,7 +91,8 @@ SIGNATURES = {
     "pxm_skrock_shift": (_i, [_vp, _d, _vp, _vp, _i, _u64, _u64, _vp, _u32, _vp, _ll, _ll, _vp]),
     "pxm_skrock_stage": (_i, [_vp, _vp, _vp, _vp, _vp, _d, _d, _d, _d, _d, _d, _d, _d, _vp, _vp, _i, _u64, _u64, _vp,
                               _u32, _vp, _ll, _ll, _vp]),
-    "pxm_masked_gather": (_i, [_vp, _vp, _vp, _vp, _ll, _ll, _ll, _vp]),
+    "pxm_fista_update": (_i, [_vp, _vp, _vp, _vp, _d, _d, _d, _vp, _vp, _vp, _vp, _ll, _ll, _ll, _vp, _vp]),
+    "pxm_masked_gather":(_i, [_vp, _vp, _vp, _vp, _ll, _ll, _ll, _vp]),
     "pxm_masked_scatter": (_i, [_vp, _vp, _vp, _vp, _ll, _ll, _ll, _vp]),
     "pxm_real_to_complex": (_i, [_vp, _vp, _ll, _vp]),
     "pxm_csr_spmv": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _ll, _ll, _vp]),

@@ -615,6 +615,74 @@ __global__ void k_skrock_stage(SkrockArgs p, size_t chain0) {
 }
 
 // ---------------------------------------------------------------------------
+// FISTA (Beck & Teboulle 2009) for the synthesis-setting MAP, nchains independent problems:
+//   x_{k+1} = soft(y_k - t gradg(y_k), s T),   y_{k+1} = x_{k+1} + beta_k (x_{k+1} - x_k),
+//   beta_k = (tau_k - 1) / tau_{k+1},  tau_{k+1} = (1 + sqrt(1 + 4 tau_k^2)) / 2,  tau_0 = 1.
+// The iteration counter k and tau_k live in the device state block {k, tau_k}, so one captured block of iterations
+// replays unchanged.  Stage 1 also writes, per block, the partial sums of |x_{k+1} - x_k|^2 and |x_{k+1}|^2 (partial
+// [chain][PXM_REDUCE_PARTS], the scratch scheme of pxm_reduce); stage 2 sums them in a fixed order into history slot
+// k mod cap and advances the state.  y and x are read before they are written: x_out / y_out may be x_k / y_k.
+// ---------------------------------------------------------------------------
+struct FistaArgs {
+  const cplx* y;
+  const cplx* gradg;
+  const cplx* x;
+  const double* Tv;  // may be null -> Ts
+  double Ts, Tscale, t;
+  const double* state;  // {k, tau_k}
+  cplx* x_out;
+  cplx* y_out;
+  cplx* partial;  // [nchains][gridDim.x]: (sum |x_{k+1} - x_k|^2, sum |x_{k+1}|^2)
+  size_t n;
+};
+
+__device__ __forceinline__ double fista_next_tau(double tau) { return (1.0 + sqrt(1.0 + 4.0 * tau * tau)) / 2.0; }
+
+__global__ void k_fista_update(FistaArgs p) {
+  const double tau = p.state[1], tau1 = fista_next_tau(tau);
+  const double beta = (tau - 1.0) / tau1;
+  const size_t chain = blockIdx.y, off = chain * p.n;
+  cplx acc = make_double2(0.0, 0.0);
+  for (size_t e = blockIdx.x * (size_t)blockDim.x + threadIdx.x; e < p.n; e += (size_t)gridDim.x * blockDim.x) {
+    const size_t i = off + e;
+    const cplx y = p.y[i], g = p.gradg[i], xk = p.x[i];
+    const double T = (p.Tv ? p.Tv[e] : p.Ts) * p.Tscale;
+    const cplx xn = soft_c(make_double2(y.x - p.t * g.x, y.y - p.t * g.y), T);
+    const double dx = xn.x - xk.x, dy = xn.y - xk.y;
+    p.x_out[i] = xn;
+    p.y_out[i] = make_double2(xn.x + beta * dx, xn.y + beta * dy);
+    acc.x += dx * dx + dy * dy;
+    acc.y += xn.x * xn.x + xn.y * xn.y;
+  }
+  acc = block_sum(acc);
+  if (threadIdx.x == 0) p.partial[chain * gridDim.x + blockIdx.x] = acc;
+}
+
+// one CTA: every chain's partials in order, then the state advances (after every read of it in this launch)
+__global__ void k_fista_finish(const cplx* __restrict__ partial, int nparts, int nchains, double* state, double* hist,
+                               long long cap) {
+  const long long slot = (long long)state[0] % cap;
+  for (int c = 0; c < nchains; ++c) {
+    cplx acc = make_double2(0.0, 0.0);
+    for (int i = threadIdx.x; i < nparts; i += blockDim.x) {
+      const cplx v = partial[(size_t)c * nparts + i];
+      acc.x += v.x;
+      acc.y += v.y;
+    }
+    acc = block_sum(acc);
+    if (threadIdx.x == 0) {
+      hist[(slot * nchains + c) * 2] = acc.x;
+      hist[(slot * nchains + c) * 2 + 1] = acc.y;
+    }
+  }
+  if (threadIdx.x == 0) {
+    const double tau = state[1];
+    state[0] += 1.0;
+    state[1] = fista_next_tau(tau);
+  }
+}
+
+// ---------------------------------------------------------------------------
 // masked gather / scatter with covariance weighting (weak lensing,
 // /root/reference/pxmcmc/measurements.py:242-304)
 // ---------------------------------------------------------------------------
@@ -1099,6 +1167,30 @@ int pxm_launch_skrock(int stage, const void* U, const void* V, const void* gradg
   return PXM_OK;
 }
 
+int pxm_launch_fista(const void* y, const void* gradg, const void* x, const double* Tv, double Ts, double Tscale,
+                     double t, double* state, void* x_out, void* y_out, double* hist, long long cap, size_t n,
+                     size_t nchains, void* partial, cudaStream_t st) {
+  FistaArgs p;
+  p.y = (const cplx*)y;
+  p.gradg = (const cplx*)gradg;
+  p.x = (const cplx*)x;
+  p.Tv = Tv;
+  p.Ts = Ts;
+  p.Tscale = Tscale;
+  p.t = t;
+  p.state = state;
+  p.x_out = (cplx*)x_out;
+  p.y_out = (cplx*)y_out;
+  p.partial = (cplx*)partial;
+  p.n = n;
+  if (!nchains) return PXM_OK;
+  k_fista_update<<<dim3(PXM_REDUCE_PARTS, (unsigned)nchains), 256, 0, st>>>(p);
+  PXM_LAUNCHED();
+  k_fista_finish<<<1, 256, 0, st>>>((const cplx*)partial, PXM_REDUCE_PARTS, (int)nchains, state, hist, cap);
+  PXM_LAUNCHED();
+  return PXM_OK;
+}
+
 int pxm_launch_gather(int scatter, const void* in, const int* idx, const double* w, void* out, size_t nsel,
                       size_t nfull, size_t nchains, cudaStream_t st) {
   const size_t total = nsel * nchains;
@@ -1129,6 +1221,8 @@ int pxm_elem_preload() {
   PXM_CUDA(cudaFuncGetAttributes(&a, k_lincomb));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_skrock_shift));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_skrock_stage));
+  PXM_CUDA(cudaFuncGetAttributes(&a, k_fista_update));
+  PXM_CUDA(cudaFuncGetAttributes(&a, k_fista_finish));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_gather_w));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_scatter_w));
   PXM_CUDA(cudaFuncGetAttributes(&a, k_r2c));

@@ -1571,6 +1571,17 @@ int pxm_skrock_stage(const void* d_U, const void* d_V, const void* d_gradg, cons
                            (cudaStream_t)stream);
 }
 
+int pxm_fista_update(const void* d_y, const void* d_gradg, const void* d_x, const double* d_T, double T_scalar,
+                     double T_scale, double t, double* d_state, void* d_x_out, void* d_y_out, double* d_hist,
+                     long long cap, long long n, long long nchains, void* d_partial, void* stream) {
+  ProfScope _ps(2, (cudaStream_t)stream);
+  PXM_REQUIRE(d_y && d_gradg && d_x && d_state && d_x_out && d_y_out && d_hist && d_partial && n >= 0 && cap >= 1 &&
+                  nchains >= 0 && nchains <= 65535,
+              "fista_update: bad argument");
+  return pxm_launch_fista(d_y, d_gradg, d_x, d_T, T_scalar, T_scale, t, d_state, d_x_out, d_y_out, d_hist, cap,
+                          (size_t)n, (size_t)nchains, d_partial, (cudaStream_t)stream);
+}
+
 int pxm_masked_gather(const void* d_full, const int* d_idx, const double* d_w, void* d_sel, long long nsel,
                       long long nfull, long long nchains, void* stream) {
   ProfScope _ps(2, (cudaStream_t)stream);

@@ -138,6 +138,9 @@ int pxm_launch_skrock(int stage, const void* U, const void* V, const void* gradg
                       const double* z_re, const double* z_im, int noise_mode, unsigned long long seed,
                       unsigned long long step, const unsigned long long* d_step, unsigned int stream0, void* out, size_t n,
                       size_t nchains, cudaStream_t st);
+int pxm_launch_fista(const void* y, const void* gradg, const void* x, const double* Tv, double Ts, double Tscale,
+                     double t, double* state, void* x_out, void* y_out, double* hist, long long cap, size_t n,
+                     size_t nchains, void* partial, cudaStream_t st);
 int pxm_launch_gather(int scatter, const void* in, const int* idx, const double* w, void* out, size_t nsel,
                       size_t nfull, size_t nchains, cudaStream_t st);
 int pxm_launch_lm_convert(int to_internal, void* flm, double* H, const unsigned long long* d_slot_off,

@@ -450,6 +450,22 @@ def skrock_stage_dev(U, V, gradg, prox, Tvec, Tscalar, lmda, a, b, c, c0, Z=None
     return out[0] if was1 else out
 
 
+def fista_update_dev(Y, gradg, X, Tvec, Tscalar, Tscale, t, state, hist, out=None):
+    """one FISTA iteration (pxm_fista_update) of the [nchains, n] complex tensors: (x_{k+1}, y_{k+1}) written to `out`
+    (X, Y themselves are allowed) or to new tensors; `state` = float64 device tensor {k, tau_k}, advanced by the call;
+    `hist` = float64 [cap, nchains, 2] receives |x_{k+1} - x_k|^2 and |x_{k+1}|^2 in slot k mod cap"""
+    nb, n = Y.shape
+    if hist.dim() != 3 or hist.shape[1:] != (nb, 2) or hist.dtype != FDT:
+        raise ValueError("fista_update: hist must be a float64 [cap, nchains, 2] tensor")
+    Xo, Yo = (torch.empty_like(Y), torch.empty_like(Y)) if out is None else out
+    key = (nb, Y.device, torch.cuda.current_stream().cuda_stream)
+    if key not in _scratch:
+        _scratch[key] = torch.empty(nb * lib.pxm_reduce_scratch_elems(), dtype=CDT, device=Y.device)
+    check(lib.pxm_fista_update(ptr(Y), ptr(gradg), ptr(X), ptr(Tvec), float(Tscalar), float(Tscale), float(t), ptr(state),
+                               ptr(Xo), ptr(Yo), ptr(hist), hist.shape[0], n, nb, ptr(_scratch[key]), stream_ptr()))
+    return Xo, Yo
+
+
 def resid_dev(preds, data, invcov):
     p2, was1 = batch2d(preds)
     out = torch.empty_like(p2)

@@ -266,6 +266,77 @@ class ForwardOperator:
         op._is_paired = True
         return op
 
+    # ------------------------------------------------------------------ Lipschitz constant of the data-fidelity gradient
+    def _real_positive_ic(self):
+        """None when the inverse covariance is diagonal, real and positive (the data fidelity is then the real
+        quadratic 1/2 (Phi Psi x - d)^dagger IC (Phi Psi x - d) and gradg its gradient), else the reason why not"""
+        if self._diag is None:
+            return None
+        d = np.asarray(self._diag)
+        if np.any(d.imag != 0) or np.any(d.real <= 0):
+            return ("the inverse covariance is not real and positive, so gradg is not the gradient of a real data "
+                    "fidelity (a real sigma with complex data is turned into the variance var (1 + i) / sqrt 2, "
+                    "pxmcmc/forward.py:80-82); pass sigma as a complex array (np.asarray(sigma, dtype=complex)) to skip "
+                    "that rule")
+        return None
+
+    def _zero_data(self):
+        """shadow copy with zero data (same transform, measurement and covariance; data-dependent caches dropped, as in
+        `paired`): its gradg is the linear part Psi^dagger Phi^dagger IC Phi Psi of this operator's"""
+        import copy
+
+        op = copy.copy(self)
+        op.data = np.zeros_like(np.asarray(self.data))
+        op._dev = None
+        for c in ("_ring_data_cache", "_harm_b_cache", "_ic_rings_cache"):
+            if hasattr(op, c):
+                delattr(op, c)
+        return op
+
+    def _normal_apply(self, X):
+        """gradg(forward(X)) through the library's device path: the carried ring / Gram form when it applies, else
+        forward + calc_gradg (X: [nchains, n] complex device tensor)"""
+        if self._pxm_native and self._ring_fusable():
+            return self.gradg_from_ring(self.forward_ring(X))
+        if self._pxm_native:
+            return D.to_dev_c(self.calc_gradg(self.forward(X)))
+        x = D.to_host(X)
+        return D.to_dev_c(np.stack([np.asarray(self.calc_gradg(self.forward(v))) for v in x]))
+
+    def lipschitz(self, tol=1e-10):
+        """L_f = lambda_max(Psi^dagger Phi^dagger IC Phi Psi): the Lipschitz constant of gradg, the largest eigenvalue of
+        its linear part, by ARPACK (scipy.sparse.linalg.eigsh, which="LA", relative accuracy `tol`) with the library's
+        own device path as the matrix-vector product (on a zero-data copy of this operator).  Cached per inverse
+        covariance.  Synthesis setting with a real, positive, diagonal inverse covariance only (ValueError /
+        NotImplementedError with the reason otherwise)."""
+        if self.setting != "synthesis":
+            raise NotImplementedError("lipschitz: the synthesis setting only")
+        if self._diag is None:
+            raise NotImplementedError("lipschitz: a full covariance matrix is not supported (diagonal covariances only)")
+        if getattr(self, "_pxm_allreduce", None) is not None:
+            raise NotImplementedError("lipschitz: m-sharded operators are not supported")
+        why = self._real_positive_ic()
+        if why is not None:
+            raise ValueError("lipschitz: " + why)
+        c = getattr(self, "_lipschitz_cache", None)
+        if c is not None and c[0] is self._diag and c[1] <= tol:
+            return c[2]
+        from scipy.sparse.linalg import LinearOperator, eigsh
+
+        op = self._zero_data()
+        n = int(self.nparams)
+        counter = [0]
+
+        def matvec(v):
+            counter[0] += 1
+            return D.to_host(op._normal_apply(D.to_dev_c(np.ravel(v)).reshape(1, n))[0])
+
+        A = LinearOperator((n, n), matvec=matvec, dtype=np.complex128)
+        v0 = np.random.default_rng(0).standard_normal(n).astype(np.complex128)
+        lam = float(eigsh(A, k=1, which="LA", tol=tol, v0=v0, return_eigenvectors=False)[0])
+        self._lipschitz_cache = (self._diag, float(tol), lam, counter[0])
+        return lam
+
     def _forward_synthesis(self, X):
         if self._fused():
             return self.measurement._forward_from_harmonic(self.transform._inverse_harmonic(X))

@@ -256,6 +256,125 @@ class PxMCMC:
         Xd = self._state(X)
         return Xd, (D.to_dev_c(self._forward_dev(Xd)) if want_preds else None)
 
+    # ------------------------------------------------------------------ MAP estimate (FISTA), step-size bound
+    _FISTA_BLOCK = 50  # iterations between two convergence reads (one CUDA graph replay when graphed)
+
+    # p = delta * Lip(grad log pi) up to which one step is stable (the samplers that have such a bound override it)
+    stability_limit = float("nan")
+
+    def max_stable_delta(self):
+        """stability_limit / (L_f + 1 / lmda): the largest step size delta for which one step of the sampler is stable
+        (its deterministic factor on a quadratic stays within [-1, 1]), with L_f = `forward.lipschitz()` the Lipschitz
+        constant of gradg and 1 / lmda that of the Moreau-Yosida term.  A stability bound, not an accuracy
+        recommendation: the chain's bias grows with delta below it too.  Synthesis setting, library L1 prior,
+        real positive inverse covariance (the refusals of `map_estimate`).  NaN when the sampler has no stability
+        limit (SKROCK's reference scheme)."""
+        if np.isnan(self.stability_limit):
+            return float("nan")
+        self._check_map_problem("max_stable_delta")
+        return self.stability_limit / (self.forward.lipschitz() + 1.0 / self.lmda)
+
+    def _check_map_problem(self, what):
+        """raise unless the drift -(x - prox x)/lmda - gradg(x) is the Moreau-Yosida gradient flow of the real objective
+        F(x) = 1/2 (Phi Psi x - d)^dagger IC (Phi Psi x - d) + mu sum_i w_i |x_i| (see `map_estimate`)"""
+        if self.forward.setting != "synthesis" or getattr(self.prior, "setting", None) != "synthesis":
+            raise NotImplementedError(
+                f"{what}: the analysis setting is not supported (the reference's analysis prox X + Psi(soft(Psi^dagger X) "
+                "- Psi^dagger X) is not the prox of mu ||w Psi^dagger x||_1)")
+        if not is_library_l1(self.prior):
+            raise NotImplementedError(f"{what}: a user-overridden prox / prior is not supported (the library's L1 "
+                                      "priors only: the prox must be the soft threshold)")
+        if getattr(self.forward, "_diag", None) is None:
+            raise NotImplementedError(f"{what}: a full covariance matrix is not supported (diagonal covariances only)")
+        if getattr(self.forward, "_pxm_allreduce", None) is not None:
+            raise NotImplementedError(f"{what}: m-sharded operators are not supported")
+        why = self.forward._real_positive_ic()
+        if why is not None:
+            raise ValueError(f"{what}: {why}")
+
+    def _map_objective(self, Xd):
+        """F of every chain of Xd [nchains, n] as a float64 device tensor: 1/2 L2 + mu prior (pxm_reduce kinds 1, 0).
+        The tracked logPi = -mu prior - L2 has no 1/2 (as in the reference), so F is not -logPi."""
+        L2, pr = self._logpi_terms_dev(Xd, D.to_dev_c(self._forward_dev(Xd)))
+        return 0.5 * L2.real + self.mu * pr
+
+    def map_estimate(self, start_point=None, *, tol=1e-8, maxiter=100_000):
+        """MAP estimate of the synthesis-setting posterior by FISTA (Beck & Teboulle 2009) on the device: the minimiser
+        of F(x) = 1/2 (Phi Psi x - d)^dagger IC (Phi Psi x - d) + mu sum_i w_i |x_i| (|.| the complex modulus, as the
+        soft threshold), whose Moreau-Yosida gradient flow is the samplers' drift -(x - prox(x))/lmda - gradg(x) when
+        the prior's threshold is T = lmda mu w (the library's L1 priors, is_library_l1).  F carries the 1/2 the tracked
+        log posterior (-mu prior - L2, as in the reference) does not have: F is not -logPi.
+
+        Step t = 1 / L_f (`forward.lipschitz()`), threshold (t / lmda) T.  `start_point`: None (a Laplace draw) or a
+        start point, with the conventions of `run`; every chain is solved independently.  Stops when the largest
+        relative change |x_{k+1} - x_k| / |x_{k+1}| over the chains is below `tol`, read once every block of
+        iterations (one small device -> host copy), or after `maxiter` iterations.  A block is one CUDA graph when the
+        operator and prior are native, else it runs eagerly; both give the same iterates bit for bit.  With
+        `real_pairs=True` the problem is solved on the operator given to the sampler.
+
+        Returns (x, info): x complex [n] (one chain) or [nchains, n], a valid `run(start_point=x)`; info = {"F":
+        objective per chain at x, "iterations", "converged", "relative_change": [blocks, nchains] at the end of every
+        block, "F_history": [blocks, nchains], "lipschitz": L_f, "step": t}.
+
+        Raises NotImplementedError in the analysis setting, for a user-overridden prox or prior, a full covariance
+        matrix or an m-sharded operator, and ValueError when the inverse covariance is not real and positive (the
+        reference's rule var (1 + i) / sqrt 2 for a real sigma with complex data: pass sigma as a complex array)."""
+        self._check_map_problem("map_estimate")
+        Lf = self.forward.lipschitz()
+        t = 1.0 / Lf
+        Tv, Ts = self._fused_prox()
+        X, _ = self._initial_sample(start_point, want_preds=False)
+        X = X.clone()
+        Y = X.clone()
+        nch = X.shape[0]
+        K = self._FISTA_BLOCK
+        state = torch.tensor([0.0, 1.0], dtype=D.FDT, device=X.device)
+        hist = torch.zeros((K, nch, 2), dtype=D.FDT, device=X.device)
+
+        def iteration(x, y, st, h):
+            D.fista_update_dev(y, self._gradg_at(y), x, Tv, Ts, t / self.lmda, t, st, h, out=(x, y))
+
+        graph = None
+        if self._native() and maxiter >= K:
+            # warm-up on copies (tables, allocator pools) before the capture; the state of the solve is not touched
+            side = torch.cuda.Stream()
+            side.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(side):
+                xw, yw, sw, hw = X.clone(), Y.clone(), state.clone(), hist.clone()
+                for _ in range(2):
+                    iteration(xw, yw, sw, hw)
+            torch.cuda.current_stream().wait_stream(side)
+            torch.cuda.synchronize()
+            del xw, yw, sw, hw
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.stream(side):
+                with torch.cuda.graph(graph, stream=side):
+                    for _ in range(K):
+                        iteration(X, Y, state, hist)
+            torch.cuda.current_stream().wait_stream(side)
+        its, converged, rel, Fh = 0, False, [], []
+        while its < maxiter and not converged:
+            k = min(K, maxiter - its)
+            if graph is not None and k == K:
+                graph.replay()
+            else:
+                for _ in range(k):
+                    iteration(X, Y, state, hist)
+            its += k
+            F = self._map_objective(X)
+            v = torch.cat([hist[(its - 1) % K].reshape(-1), F]).cpu().numpy()
+            dx2, x2 = v[0:2 * nch:2], v[1:2 * nch:2]
+            r = np.sqrt(dx2) / np.maximum(np.sqrt(x2), np.finfo(float).tiny)
+            rel.append(r)
+            Fh.append(v[2 * nch:])
+            converged = bool(np.max(r) < tol)
+        out = D.to_host(X)
+        if self.nchains == 1:
+            out = out[0]
+        info = {"F": Fh[-1] if nch > 1 else float(Fh[-1][0]), "iterations": its, "converged": converged,
+                "relative_change": np.array(rel), "F_history": np.array(Fh), "lipschitz": Lf, "step": t}
+        return out, info
+
     def _initialise_tracking_arrays(self):
         """pxmcmc/mcmc.py:113-128 (leading chain axis only when nchains > 1)"""
         lead = (self.nchains,) if self.nchains > 1 else ()
@@ -539,6 +658,9 @@ class MYULA(PxMCMC):
     """Moreau-Yosida unadjusted Langevin algorithm (pxmcmc/mcmc.py:143-201)."""
 
     graph_run = True  # run(): replay the iteration as a CUDA graph when the noise is generated on the device
+    # one step on a quadratic multiplies the deviation from the mode by 1 - p, p = delta * Lip(grad log pi): within
+    # [-1, 1] for p <= 2
+    stability_limit = 2.0
 
     def __init__(self, forward, prox, mcmcparams=PxMCMCParams(), *, real_pairs=False, **kw):
         """`real_pairs=True` (extension; an even number of chains, real data, real noise level, `complex=False`, the
