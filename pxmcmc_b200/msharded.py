@@ -385,6 +385,11 @@ def sharded_s2_wavelets_l1(transform, T, L, B, J_min, cls=None, **kw):
     full.T = np.ascontiguousarray(np.asarray(full.T)[idx])
     full.map_weights = np.ascontiguousarray(np.asarray(full.map_weights)[idx])
     full._Tdev = full._wdev = None
+    # uploaded now, not on first use: a host -> device copy waits for the stream it is issued on, and inside an
+    # iteration that stream holds a peer barrier (with all ranks on one GPU, `SimulatedRanks`, the peers that barrier
+    # waits for are not even enqueued yet: the first iteration would end in the barrier's time-out)
+    full._T_args()
+    full._weights_dev()
     return full
 
 
