@@ -378,7 +378,7 @@ long long pxm_launch_count(void);
 
 /* ---- debugging aids (tests only) ---------------------------------------------- */
 int pxm_debug_set_naive(int on); /* route Legendre contractions through the plain kernel */
-int pxm_debug_set_fft_multipass(int mode); /* ring FFT kernel choice: 0 by grid size (default), 1 always the multi-pass kernel, 2 always the two-pass kernel (Bluestein lengths <= 1024), 3 two-pass with the persistent TMA-staged kernel for lengths 512 / 1024 whatever the grid size (4: the same; selects the two-CTA kernel in development builds with -DPXM_FFT_PINGPONG) */
+int pxm_debug_set_fft_multipass(int mode); /* ring FFT kernel choice: 0 by grid size (default), 1 always the multi-pass kernel, 2 always the two-pass kernel (Bluestein lengths <= 1024), 3 two-pass with the persistent TMA-staged kernel for lengths 512 / 1024 whatever the grid size (the one-CTA-per-SM kernel pxm_ring_fft6_kernel, as mode 0 picks for large grids); 4 as 3 with the two-CTA kernel pxm_ring_fft3_kernel it replaced */
 int pxm_debug_wigner_row_host(int grid_L, int ring, int m, int spin, int lmax, double* out); /* host, no GPU */
 
 #ifdef __cplusplus

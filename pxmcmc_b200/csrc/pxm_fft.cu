@@ -718,16 +718,17 @@ __device__ __forceinline__ double flip_sign(double x, int mask_hi) {
 }
 
 // chirp_s: this group's chirp times sqrt(scale / M) in shared memory (pass 1 and pass 3 each apply it once)
-template <int DIR, int R1, int R2>
+// NG: item groups per CTA (the threads of a group are blockDim.x / NG consecutive threads; tid: index within the group)
+template <int DIR, int R1, int R2, int NG>
 __device__ __forceinline__ void ring_fft3_pass1(const PxmFftGroup& gr, const Fft3Item& it, cplx* __restrict__ s,
                                                 const unsigned char* __restrict__ stage,
-                                                const cplx* __restrict__ chirp_s, const cplx* __restrict__ arena) {
+                                                const cplx* __restrict__ chirp_s, const cplx* __restrict__ arena, int tid) {
   constexpr int H1 = R1 / 2;
   const int n = gr.n, rings = gr.rings, ell = gr.ell;
   const int nr = 1 << gr.pad;
   const int RS = ring_stride2(R1, R2);
   const cplx* __restrict__ tw2 = arena + gr.tw2_off;  // [k1][j2]
-  for (int idx = threadIdx.x; idx < nr * R2; idx += blockDim.x) {
+  for (int idx = tid; idx < nr * R2; idx += blockDim.x / NG) {
     // 4 rings of a row-group on adjacent lanes, 8 values of j2 per warp: the chirp / twiddle reads are
     // broadcasts over the rings, the ring-array accesses are 32-byte sectors, the pixel rows 128-byte pieces
     const int rhi = idx / (4 * R2), rem = idx - rhi * 4 * R2;
@@ -781,14 +782,14 @@ __device__ __forceinline__ void ring_fft3_pass1(const PxmFftGroup& gr, const Fft
   }
 }
 
-template <int R1, int R2>
-__device__ __forceinline__ void ring_fft3_middle(const PxmFftGroup& gr, cplx* __restrict__ s,
-                                                 const cplx* __restrict__ arena) {
+// bhat: the group's filter spectrum in natural order [k2 R1 + k1], in global (two-CTA kernel) or shared memory
+template <int R1, int R2, int NG>
+__device__ __forceinline__ void ring_fft3_middle(const PxmFftGroup& gr, cplx* __restrict__ s, const cplx* __restrict__ bhat,
+                                                 const cplx* __restrict__ arena, int tid) {
   const int nr = 1 << gr.pad;
   const int RS = ring_stride2(R1, R2);
-  const cplx* __restrict__ bhat = arena + gr.bhat2_off;
   const cplx* __restrict__ tw2t = arena + gr.tw2_off + R1 * R2;  // [j2][k1]
-  for (int idx = threadIdx.x; idx < nr * R1; idx += blockDim.x) {
+  for (int idx = tid; idx < nr * R1; idx += blockDim.x / NG) {
     // 4 rings on adjacent lanes, 8 values of k1 per warp: the filter-spectrum and twiddle loads are
     // broadcasts over the rings (a quarter of the L1 wavefronts), the row accesses stay conflict free
     const int rhi = idx / (4 * R1), rem = idx - rhi * 4 * R1;
@@ -821,16 +822,16 @@ __device__ __forceinline__ void ring_fft3_middle(const PxmFftGroup& gr, cplx* __
   }
 }
 
-template <int DIR, int R1, int R2>
+template <int DIR, int R1, int R2, int NG>
 __device__ __forceinline__ void ring_fft3_pass3(const PxmFftGroup& gr, const Fft3Item& it, const cplx* __restrict__ s,
                                                 const cplx* __restrict__ chirp_s, cplx* __restrict__ pix,
-                                                size_t pix_chain_stride, double* __restrict__ F, int nld) {
+                                                size_t pix_chain_stride, double* __restrict__ F, int nld, int tid) {
   constexpr int H1 = R1 / 2;
   const int n = gr.n, rings = gr.rings, ell = gr.ell;
   const int nr = 1 << gr.pad;
   const int RS = ring_stride2(R1, R2);
   const size_t col0 = (size_t)it.chain * 4;  // paired layout only (the launcher checks)
-  for (int idx = threadIdx.x; idx < nr * R2; idx += blockDim.x) {
+  for (int idx = tid; idx < nr * R2; idx += blockDim.x / NG) {
     // 4 rings of a row-group on adjacent lanes, 8 values of j2 per warp: the chirp / twiddle reads are
     // broadcasts over the rings, the ring-array accesses are 32-byte sectors, the pixel rows 128-byte pieces
     const int rhi = idx / (4 * R2), rem = idx - rhi * 4 * R2;
@@ -939,9 +940,9 @@ pxm_ring_fft3_kernel(const __grid_constant__ PxmFftGroupTable tab, const __grid_
     phase ^= 1;
     FFT3_T(0);
     if (big)
-      ring_fft3_pass1<DIR, 32, 32>(gr, cur, s, stage, chirp_s, arena);
+      ring_fft3_pass1<DIR, 32, 32, 1>(gr, cur, s, stage, chirp_s, arena, threadIdx.x);
     else
-      ring_fft3_pass1<DIR, 16, 32>(gr, cur, s, stage, chirp_s, arena);
+      ring_fft3_pass1<DIR, 16, 32, 1>(gr, cur, s, stage, chirp_s, arena, threadIdx.x);
     FFT3_T(1);
     __syncthreads();
     FFT3_T(2);
@@ -957,18 +958,134 @@ pxm_ring_fft3_kernel(const __grid_constant__ PxmFftGroupTable tab, const __grid_
     }
     FFT3_T(3);
     if (big)
-      ring_fft3_middle<32, 32>(gr, s, arena);
+      ring_fft3_middle<32, 32, 1>(gr, s, arena + gr.bhat2_off, arena, threadIdx.x);
     else
-      ring_fft3_middle<16, 32>(gr, s, arena);
+      ring_fft3_middle<16, 32, 1>(gr, s, arena + gr.bhat2_off, arena, threadIdx.x);
     FFT3_T(4);
     __syncthreads();
     FFT3_T(5);
     if (big)
-      ring_fft3_pass3<DIR, 32, 32>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld);
+      ring_fft3_pass3<DIR, 32, 32, 1>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld, threadIdx.x);
     else
-      ring_fft3_pass3<DIR, 16, 32>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld);
+      ring_fft3_pass3<DIR, 16, 32, 1>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld, threadIdx.x);
     FFT3_T(6);
     cur = nxt;
+  }
+}
+
+// =============================================================================================
+// The persistent staged transform with ONE CTA of 256 threads per SM (pxm_ring_fft6_kernel, what the launcher
+// picks for the radix-32 class): two groups of 4 warps, each running exactly the per-item code of
+// pxm_ring_fft3_kernel -- its own TMA stage, mbarrier and work buffer, synchronised on its own named barrier --
+// with no hand-over between the groups.  Items are dealt in chain pairs: group g takes chain 2k + g of a ring
+// block, so both groups always work in the same Bluestein group and the CTA holds ONE copy of the chirp and ONE
+// of the filter spectrum, in shared memory.  The middle pass then reads its 32 filter-spectrum values per thread
+// and item from shared memory (broadcasts over the 4 rings of a quarter-warp) instead of from L2: next to the
+// shared memory of two CTAs of the two-CTA kernel about 28 KB of L1 remained, with a 13 % load hit rate.
+// The tables change a few times per launch (the blocks of a group are consecutive items), behind CTA barriers
+// that both groups reach in the same iterations: they walk the same sequence of chain pairs.
+// =============================================================================================
+constexpr int PXM_FFT6_WORK0 = 2 * PXM_FFT3_STAGE;  // the two stages first: 1024-byte aligned for the TMA swizzle
+constexpr int PXM_FFT6_CHIRP0 = PXM_FFT6_WORK0 + 2 * PXM_FFT3_WORK;
+constexpr int PXM_FFT6_BHAT0 = PXM_FFT6_CHIRP0 + PXM_FFT3_CHIRP;
+constexpr int PXM_FFT6_BAR0 = PXM_FFT6_BHAT0 + 1024 * 16;
+constexpr int PXM_FFT6_SMEM = PXM_FFT6_BAR0 + 2 * 8;  // 225 808 bytes
+static_assert(PXM_FFT6_SMEM <= 232448, "one CTA per SM: the opt-in shared memory of a block");
+
+__device__ __forceinline__ void grp_sync(int g) { asm volatile("bar.sync %0, 128;" ::"r"(1 + g) : "memory"); }
+
+template <int DIR>
+__global__ void __launch_bounds__(256, 1)
+pxm_ring_fft6_kernel(const __grid_constant__ PxmFftGroupTable tab, const __grid_constant__ Fft3Blocks blocks,
+                     const __grid_constant__ Fft3Maps maps, cplx* __restrict__ pix, size_t pix_chain_stride,
+                     double* __restrict__ F, int nld, const cplx* __restrict__ arena, int nchains, long long npairs) {
+  extern __shared__ __align__(1024) unsigned char fsm6[];
+  const int g = threadIdx.x >> 7, tid = threadIdx.x & 127;  // 256 threads: two groups of 128
+  unsigned char* stage = fsm6 + g * PXM_FFT3_STAGE;
+  cplx* s = reinterpret_cast<cplx*>(fsm6 + PXM_FFT6_WORK0 + g * PXM_FFT3_WORK);
+  cplx* chirp_s = reinterpret_cast<cplx*>(fsm6 + PXM_FFT6_CHIRP0);
+  cplx* bhat_s = reinterpret_cast<cplx*>(fsm6 + PXM_FFT6_BHAT0);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(fsm6 + PXM_FFT6_BAR0) + g;
+  long long pair = blockIdx.x;
+  if (pair >= npairs) return;
+  if (tid == 0) {
+    if (smem_u32(fsm6) & 1023) __trap();
+    mbar_init(bar, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  // (block, chain pair) of the pair, advanced without divisions; with an odd chain count the last pair of a
+  // block has no chain for group 1, which then skips the item
+  const int npc = (nchains + 1) >> 1;
+  int ib = (int)(pair / npc), ik = (int)(pair - (long long)ib * npc);
+  const int db = (int)gridDim.x / npc, dk = (int)gridDim.x - db * npc;
+  uint32_t phase = 0;
+  Fft3Item cur, nxt;
+  fft3_find(tab, blocks, ib, 2 * ik + g, &cur);
+  bool have = cur.chain < nchains;
+  if (have && tid == 0)
+    fft3_stage_one<DIR>(tab.g[cur.gi], cur, stage, bar, pix, pix_chain_stride, &maps.m[blocks.map_of_group[cur.gi]]);
+  nxt = cur;
+  int table_group = -1;
+  for (; pair < npairs; pair += gridDim.x) {
+    const PxmFftGroup& gr = tab.g[cur.gi];
+    const bool big = gr.logM == 10;
+    if (cur.gi != table_group) {
+      __syncthreads();  // both groups have finished with the old chirp (pass 3) and filter spectrum (middle pass)
+      const cplx* __restrict__ chirp = arena + gr.chirp_off;
+      const double rs = sqrt(gr.scale / (double)gr.M);
+      for (int j = threadIdx.x; j < gr.n; j += blockDim.x) {
+        const cplx c = chirp[j];
+        chirp_s[j] = make_double2(c.x * rs, c.y * rs);
+      }
+#ifndef PXM_ABL_FFT6_GLOBAL_BHAT
+      const cplx* __restrict__ bhat = arena + gr.bhat2_off;
+      for (int k = threadIdx.x; k < gr.M; k += blockDim.x) bhat_s[k] = bhat[k];
+#endif
+      table_group = cur.gi;
+      __syncthreads();
+    }
+#ifdef PXM_ABL_FFT6_GLOBAL_BHAT
+    const cplx* bh = arena + gr.bhat2_off;
+#else
+    const cplx* bh = bhat_s;
+#endif
+    if (have) {
+      grp_sync(g);            // pass 3 of the group's previous item has left the work buffer
+      mbar_wait(bar, phase);  // the staged inputs have landed
+      phase ^= 1;
+      if (big)
+        ring_fft3_pass1<DIR, 32, 32, 2>(gr, cur, s, stage, chirp_s, arena, tid);
+      else
+        ring_fft3_pass1<DIR, 16, 32, 2>(gr, cur, s, stage, chirp_s, arena, tid);
+      grp_sync(g);
+    }
+    bool have_next = false;
+    if (pair + gridDim.x < npairs) {
+      ib += db;
+      ik += dk;
+      if (ik >= npc) {
+        ik -= npc;
+        ++ib;
+      }
+      fft3_find(tab, blocks, ib, 2 * ik + g, &nxt);
+      have_next = nxt.chain < nchains;
+      if (have_next && tid == 0)  // the stage is free: pass 1 has read it, or the group had no item
+        fft3_stage_one<DIR>(tab.g[nxt.gi], nxt, stage, bar, pix, pix_chain_stride, &maps.m[blocks.map_of_group[nxt.gi]]);
+    }
+    if (have) {
+      if (big)
+        ring_fft3_middle<32, 32, 2>(gr, s, bh, arena, tid);
+      else
+        ring_fft3_middle<16, 32, 2>(gr, s, bh, arena, tid);
+      grp_sync(g);
+      if (big)
+        ring_fft3_pass3<DIR, 32, 32, 2>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld, tid);
+      else
+        ring_fft3_pass3<DIR, 16, 32, 2>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld, tid);
+    }
+    cur = nxt;
+    have = have_next;
   }
 }
 
@@ -1287,290 +1404,6 @@ pxm_ring_fft5_kernel(const __grid_constant__ PxmFftGroupTable tab, const __grid_
 
 #endif  // PXM_FFT_PAIRSPLIT
 
-#ifdef PXM_FFT_PINGPONG
-// =============================================================================================
-// DEVELOPMENT VARIANT, compiled only with -DPXM_FFT_PINGPONG (measured SLOWER: 1.31 vs 1.17 ms per 64-chain step,
-// gpurun_out/r2k_tests.log / DESIGN.md 7c: with one warp per scheduler in the FP64 section the filter-spectrum loads are exposed).
-// Ping-pong variant of the persistent staged transform: ONE CTA of 256 threads per SM made of two
-// groups of 4 warps.  Each group is what a CTA of pxm_ring_fft3_kernel was -- its own work items,
-// staging buffer, work buffer, chirp copy, TMA barrier -- but the groups hand a token back and forth so
-// that the FP64 section of a pass (register DFTs, twiddles, filter) of one group runs while the other
-// group is in the shared-memory / global-memory section of its pass (stores of the previous pass, group
-// barrier, loads of the next one).  Two independent CTAs per SM ran those sections in lockstep: measured
-// time = memory time + FP64 time (ablations in DESIGN.md); with the hand-over it is close to the larger
-// of the two.  The token is a pair of named barriers used as producer / consumer barriers
-// (bar.sync by the group that waits, bar.arrive by the group that releases).
-// Inter-pass twiddles W_M^(k1 j2) are formed from one table entry per thread by a power tree
-// (twiddle_tree) instead of R - 1 table loads: the loads sat on the critical path of the FP64 section.
-// =============================================================================================
-constexpr int PXM_FFT4_GROUP = ((PXM_FFT3_STAGE + PXM_FFT3_WORK + PXM_FFT3_CHIRP + 1023) / 1024) * 1024;
-constexpr int PXM_FFT4_SMEM = 2 * PXM_FFT4_GROUP + 64;
-
-__device__ __forceinline__ void grp_sync(int g) { asm volatile("bar.sync %0, 128;" ::"r"(1 + g) : "memory"); }
-__device__ __forceinline__ void tok_acquire(int g) { asm volatile("bar.sync %0, 256;" ::"r"(3 + g) : "memory"); }
-__device__ __forceinline__ void tok_release_to(int g) { asm volatile("bar.arrive %0, 256;" ::"r"(3 + g) : "memory"); }
-
-struct Fft4Tok {
-  int g;        // this group
-  bool last;    // the very last release of the launch is skipped (nobody waits for it)
-  __device__ __forceinline__ void acquire() const { tok_acquire(g); }
-  __device__ __forceinline__ void release(bool final_pass) const {
-    if (!(last && final_pass)) tok_release_to(g ^ 1);
-  }
-};
-
-template <int DIR, int R1, int R2>
-__device__ __forceinline__ void ring_fft4_pass1(const PxmFftGroup& gr, const Fft3Item& it, cplx* __restrict__ s,
-                                                const unsigned char* __restrict__ stage,
-                                                const cplx* __restrict__ chirp_s, const cplx* __restrict__ arena,
-                                                int tid, const Fft4Tok& tok, bool have) {
-  constexpr int H1 = R1 / 2;
-  const int n = gr.n, rings = gr.rings, ell = gr.ell;
-  const int nr = 1 << gr.pad;
-  const int RS = ring_stride2(R1, R2);
-  const cplx* __restrict__ tw2 = arena + gr.tw2_off;  // [k1][j2]
-  // nr * R2 is 128 (M = 1024) or 256 (M = 512): every thread runs the same one or two trips; a group without an
-  // item (have == false) transforms zeros into its own work buffer so that the token changes hands all the same
-  const int padded = nr * R2;
-  for (int idx = tid; idx < padded; idx += 128) {
-    const int rhi = idx / (4 * R2), rem = idx - rhi * 4 * R2;
-    const int r = rhi * 4 + (rem & 3), j2 = rem >> 2;
-    const int nj = (have && it.t0 + r < rings) ? n : 0;  // rows past the end of the grid are zeros
-    cplx x[R1];
-    // ---- memory section: staged inputs -> registers
-    {
-      if (DIR == 0) {
-        const cplx* row = reinterpret_cast<const cplx*>(stage) + r * n;
-#pragma unroll
-        for (int j1 = 0; j1 < H1; ++j1) {
-          const int j = j1 * R2 + j2;
-          x[j1] = (j < nj) ? row[j] : make_double2(0.0, 0.0);
-        }
-      } else {
-        const unsigned char* grp = stage + (size_t)(r >> 2) * ((ell * 128 + 1023) & ~1023);
-        const int rl = r & 3;
-#pragma unroll
-        for (int j1 = 0; j1 < H1; ++j1) {
-          const int j = j1 * R2 + j2;
-          cplx v = make_double2(0.0, 0.0);
-          if (j < nj) {
-            const bool minus = j >= ell;  // order m = j - n < 0: second half of the 128-byte row
-            const int am = minus ? n - j : j;
-            const int d = (minus ? 8 : 0) + rl;  // re at double d, im at d + 4 (two chunks further)
-            const unsigned char* row = grp + am * 128 + (d & 1) * 8;
-            const int sw = am & 7, ch = d >> 1;
-            const double re = *reinterpret_cast<const double*>(row + ((ch ^ sw) << 4));
-            const double im = *reinterpret_cast<const double*>(row + (((ch + 2) ^ sw) << 4));
-            const int neg = (minus && (am & 1)) ? (int)0x80000000 : 0;
-            // (-1)^m of the paired layout and the conjugation on load (x_p = conj(DFT(conj F))) are sign-bit flips
-            v = make_double2(flip_sign(re, neg), flip_sign(im, neg ^ (int)0x80000000));
-          }
-          x[j1] = v;
-        }
-      }
-    }
-    if (idx == tid) tok.acquire();
-    // ---- FP64 section
-    {
-#pragma unroll
-      for (int j1 = 0; j1 < H1; ++j1) {
-        const int j = j1 * R2 + j2;
-        x[j1] = cmul(x[j1], chirp_s[j < n ? j : 0]);
-      }
-      dft_half_in<R1>(x);
-      twiddle_tree<R1, false>(x, tw2[R2 + j2]);  // W_M^(k1 j2), k1 < R1, from W_M^(j2)
-    }
-    if (idx + 128 >= padded) tok.release(false);
-    // ---- memory section: registers -> work buffer
-    {
-      cplx* dst = s + r * RS + j2;
-#pragma unroll
-      for (int k1 = 0; k1 < R1; ++k1) dst[k1 * (R2 + 1)] = x[k1];
-    }
-  }
-}
-
-template <int R1, int R2>
-__device__ __forceinline__ void ring_fft4_middle(const PxmFftGroup& gr, cplx* __restrict__ s,
-                                                 const cplx* __restrict__ arena, int tid, const Fft4Tok& tok, bool have) {
-  const int nr = 1 << gr.pad;
-  const int RS = ring_stride2(R1, R2);
-  const cplx* __restrict__ bhat = arena + gr.bhat2_off;
-  const cplx* __restrict__ tw2t = arena + gr.tw2_off + R1 * R2;  // [j2][k1]
-  const int padded = nr * R1;  // 128 for both radix pairs
-  for (int idx = tid; idx < padded; idx += 128) {
-    const int rhi = idx / (4 * R1), rem = idx - rhi * 4 * R1;
-    const int r = rhi * 4 + (rem & 3), k1 = rem >> 2;
-    cplx* row = s + r * RS + k1 * (R2 + 1);
-    cplx x[R2];
-#pragma unroll
-    for (int j2 = 0; j2 < R2; ++j2) x[j2] = row[j2];
-    if (idx == tid) tok.acquire();
-    {
-      dftN<R2, false>(x);
-      prefetched<R2, PXM_PF2>([&](int k2) { return bhat[k2 * R1 + k1]; }, [&](int k2, cplx b) { x[k2] = cmul(x[k2], b); });
-      dftN<R2, true>(x);
-      twiddle_tree<R2, true>(x, tw2t[R1 + k1]);  // conj W_M^(j2 k1), j2 < R2, from W_M^(k1)
-    }
-    if (idx + 128 >= padded) tok.release(false);
-#pragma unroll
-    for (int j2 = 0; j2 < R2; ++j2) row[j2] = x[j2];
-  }
-}
-
-template <int DIR, int R1, int R2>
-__device__ __forceinline__ void ring_fft4_pass3(const PxmFftGroup& gr, const Fft3Item& it, const cplx* __restrict__ s,
-                                                const cplx* __restrict__ chirp_s, cplx* __restrict__ pix,
-                                                size_t pix_chain_stride, double* __restrict__ F, int nld, int tid,
-                                                const Fft4Tok& tok, bool have) {
-  constexpr int H1 = R1 / 2;
-  const int n = gr.n, rings = gr.rings, ell = gr.ell;
-  const int nr = 1 << gr.pad;
-  const int RS = ring_stride2(R1, R2);
-  const size_t col0 = (size_t)it.chain * 4;  // paired layout only (the launcher checks)
-  const int padded = nr * R2;
-  for (int idx = tid; idx < padded; idx += 128) {
-    const int rhi = idx / (4 * R2), rem = idx - rhi * 4 * R2;
-    const int r = rhi * 4 + (rem & 3), j2 = rem >> 2;
-    const int t = it.t0 + r;
-    const bool act = have && t < rings;
-    cplx x[R1];
-    {
-      const cplx* src = s + r * RS + j2;
-#pragma unroll
-      for (int k1 = 0; k1 < R1; ++k1) x[k1] = src[k1 * (R2 + 1)];
-    }
-    if (idx == tid) tok.acquire();
-    {
-      dft_half_out<R1>(x);
-#pragma unroll
-      for (int j1 = 0; j1 < H1; ++j1) {
-        const int j = j1 * R2 + j2;
-        x[j1] = cmul(x[j1], chirp_s[j < n ? j : 0]);
-      }
-    }
-    if (idx + 128 >= padded) tok.release(true);
-    if (act) {
-      if (DIR == 0) {
-        double* frow = F + gr.f_off + ((size_t)(t >> 2) * (size_t)nld + col0) * 4 + (size_t)(t & 3);
-        const size_t ss = gr.slot_stride;
-#pragma unroll
-        for (int j1 = 0; j1 < H1; ++j1) {
-          const int j = j1 * R2 + j2;
-          if (j < n) {
-            const bool minus = j >= ell;
-            const int am = minus ? n - j : j;
-            double* dst = frow + (size_t)am * ss + (minus ? 8 : 0);
-            const int neg = (minus && (am & 1)) ? (int)0x80000000 : 0;
-            dst[0] = flip_sign(x[j1].x, neg);
-            dst[4] = flip_sign(x[j1].y, neg);  // next column of the k4-interleaved layout
-          }
-        }
-      } else {
-        cplx* row = pix + (size_t)it.chain * pix_chain_stride + gr.pix_off + (size_t)(t - gr.ring0) * n;
-#pragma unroll
-        for (int j1 = 0; j1 < H1; ++j1) {
-          const int j = j1 * R2 + j2;
-          if (j < n) row[j] = make_double2(x[j1].x, flip_sign(x[j1].y, (int)0x80000000));
-        }
-      }
-    }
-  }
-}
-
-template <int DIR>
-__global__ void __launch_bounds__(256, 1)
-pxm_ring_fft4_kernel(const __grid_constant__ PxmFftGroupTable tab, const __grid_constant__ Fft3Blocks blocks,
-                     const __grid_constant__ Fft3Maps maps, cplx* __restrict__ pix, size_t pix_chain_stride,
-                     double* __restrict__ F, int nld, const cplx* __restrict__ arena, int nchains, long long nitems) {
-  extern __shared__ __align__(1024) unsigned char fsm4[];
-  const int g = threadIdx.x >> 7, tid = threadIdx.x & 127;
-  unsigned char* base = fsm4 + g * PXM_FFT4_GROUP;
-  unsigned char* stage = base;  // 1024-byte aligned: the TMA swizzle phase is (row & 7)
-  cplx* s = reinterpret_cast<cplx*>(base + PXM_FFT3_STAGE);
-  cplx* chirp_s = reinterpret_cast<cplx*>(base + PXM_FFT3_STAGE + PXM_FFT3_WORK);
-  uint64_t* bar = reinterpret_cast<uint64_t*>(fsm4 + 2 * PXM_FFT4_GROUP) + g;
-  if (tid == 0) {
-    if (smem_u32(fsm4) & 1023) __trap();
-    mbar_init(bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  // both groups run the same number of rounds (the token must change hands a fixed number of times)
-  const long long stride = 2LL * gridDim.x;
-  const long long rounds = (nitems + stride - 1) / stride;
-  long long item = 2LL * blockIdx.x + g;
-  uint32_t phase = 0;
-  Fft3Item cur, nxt;
-  int ib = (int)(item / nchains), ic = (int)(item - (long long)ib * nchains);
-  const int db = (int)(stride / nchains), dc = (int)(stride - (long long)db * nchains);
-  bool have = item < nitems;
-  if (have) {
-    fft3_find(tab, blocks, ib, ic, &cur);
-    if (tid == 0) fft3_stage_one<DIR>(tab.g[cur.gi], cur, stage, bar, pix, pix_chain_stride, &maps.m[blocks.map_of_group[cur.gi]]);
-  } else {
-    // a group without work still takes its turns with the token: it transforms zeros of the launch's first
-    // (radix-32 class) group into its own work buffer and stores nothing
-    cur.gi = blocks.gi[0];
-    cur.t0 = 0;
-    cur.chain = 0;
-  }
-  nxt = cur;
-  if (g == 1) tok_release_to(0);  // group 0 computes first
-  int chirp_group = -1;
-  for (long long rd = 0; rd < rounds; ++rd, item += stride) {
-    const PxmFftGroup& gr = tab.g[cur.gi];
-    const bool big = gr.logM == 10;
-    Fft4Tok tok;
-    tok.g = g;
-    tok.last = (g == 1) && (rd + 1 == rounds);
-    if (have && cur.gi != chirp_group) {  // a few times per launch: the blocks of a group are consecutive items
-      grp_sync(g);                        // pass 3 of the previous item has finished with the old chirp
-      const cplx* __restrict__ chirp = arena + gr.chirp_off;
-      const double rs = sqrt(gr.scale / (double)gr.M);
-      for (int j = tid; j < gr.n; j += 128) {
-        const cplx c = chirp[j];
-        chirp_s[j] = make_double2(c.x * rs, c.y * rs);
-      }
-      chirp_group = cur.gi;
-    }
-    grp_sync(g);  // pass 3 of the previous item has left the work buffer; the chirp copy is complete
-    if (have) {
-      mbar_wait(bar, phase);  // the staged inputs have landed
-      phase ^= 1;
-    }
-    if (big)
-      ring_fft4_pass1<DIR, 32, 32>(gr, cur, s, stage, chirp_s, arena, tid, tok, have);
-    else
-      ring_fft4_pass1<DIR, 16, 32>(gr, cur, s, stage, chirp_s, arena, tid, tok, have);
-    grp_sync(g);
-    bool have_next = false;
-    if (item + stride < nitems) {
-      have_next = true;
-      ib += db;
-      ic += dc;
-      if (ic >= nchains) {
-        ic -= nchains;
-        ++ib;
-      }
-      fft3_find(tab, blocks, ib, ic, &nxt);
-      if (tid == 0) fft3_stage_one<DIR>(tab.g[nxt.gi], nxt, stage, bar, pix, pix_chain_stride, &maps.m[blocks.map_of_group[nxt.gi]]);
-    }
-    if (big)
-      ring_fft4_middle<32, 32>(gr, s, arena, tid, tok, have);
-    else
-      ring_fft4_middle<16, 32>(gr, s, arena, tid, tok, have);
-    grp_sync(g);
-    if (big)
-      ring_fft4_pass3<DIR, 32, 32>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld, tid, tok, have);
-    else
-      ring_fft4_pass3<DIR, 16, 32>(gr, cur, s, chirp_s, pix, pix_chain_stride, F, nld, tid, tok, have);
-    cur = nxt;
-    have = have_next;
-  }
-}
-
-#endif  // PXM_FFT_PINGPONG
 
 constexpr int PXM_FFT2_SMEM = (16 * (16 * 17 + 2)) * 16 > (4 * (32 * 33 + 2)) * 16 ? (16 * (16 * 17 + 2)) * 16
                                                                                   : (4 * (32 * 33 + 2)) * 16;
@@ -1633,7 +1466,7 @@ int pxm_fft_rings_per_cta_log(int M) {
 
 static int g_fft_legacy = 0;
 static int g_fft_pair = 0;      // persistent class: the pair-split kernel (16 points per thread, 16 warps per SM)
-static int g_fft_pingpong = 1;  // builds with -DPXM_FFT_PINGPONG: the ping-pong kernel (1) or the two-CTA kernel (0)
+static int g_fft_two_cta = 0;  // persistent class: the two-CTA kernel pxm_ring_fft3_kernel instead of pxm_ring_fft6_kernel
 constexpr int PXM_FFT_SMEM = (4096 + 256 + 32) * 16;  // up to 4096 complex points (+1/16 padding) per CTA
 
 int pxm_fft_setup_tables(const PxmFftGroup* d_groups, const PxmFftGroup* h_groups, int ngroups, void* d_arena,
@@ -1653,10 +1486,8 @@ int pxm_fft_setup_tables(const PxmFftGroup* d_groups, const PxmFftGroup* h_group
     PXM_CUDA(cudaFuncSetAttribute(pxm_ring_fft5_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PXM_FFT3_SMEM));
     PXM_CUDA(cudaFuncSetAttribute(pxm_ring_fft5_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PXM_FFT3_SMEM));
 #endif
-#ifdef PXM_FFT_PINGPONG
-    PXM_CUDA(cudaFuncSetAttribute(pxm_ring_fft4_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PXM_FFT4_SMEM));
-    PXM_CUDA(cudaFuncSetAttribute(pxm_ring_fft4_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PXM_FFT4_SMEM));
-#endif
+    PXM_CUDA(cudaFuncSetAttribute(pxm_ring_fft6_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, PXM_FFT6_SMEM));
+    PXM_CUDA(cudaFuncSetAttribute(pxm_ring_fft6_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PXM_FFT6_SMEM));
     configured = true;
   }
   if (ngroups <= 0) return PXM_OK;  // a rank of an m-sharded plan that owns no ring
@@ -1780,19 +1611,17 @@ int pxm_fft_launch(int dir, const PxmFftGroup* d_groups, const PxmFftGroup* h_gr
                                                                     nitems);
       } else
 #endif
-#ifdef PXM_FFT_PINGPONG
-      if (g_fft_pingpong) {
-        // one 256-thread CTA per SM whose two 4-warp groups alternate between FP64 and memory sections
-        const int g4 = (int)std::min<long long>((nitems + 1) / 2, (long long)nsm);
+      if (!g_fft_two_cta) {
+        // one 256-thread CTA per SM: two groups of 4 warps on chain pairs, one shared chirp and filter spectrum
+        const long long npairs = n1 * ((nchains + 1) / 2);
+        const int g6 = (int)std::min<long long>(npairs, (long long)nsm);
         if (dir == 0)
-          pxm_ring_fft4_kernel<0><<<g4, 256, PXM_FFT4_SMEM, stream>>>(tab, blocks, maps, px, pix_chain_stride, F, nld, ar, nchains,
-                                                                    nitems);
+          pxm_ring_fft6_kernel<0><<<g6, 256, PXM_FFT6_SMEM, stream>>>(tab, blocks, maps, px, pix_chain_stride, F, nld, ar, nchains,
+                                                                    npairs);
         else
-          pxm_ring_fft4_kernel<1><<<g4, 256, PXM_FFT4_SMEM, stream>>>(tab, blocks, maps, px, pix_chain_stride, F, nld, ar, nchains,
-                                                                    nitems);
-      } else
-#endif
-      if (dir == 0)
+          pxm_ring_fft6_kernel<1><<<g6, 256, PXM_FFT6_SMEM, stream>>>(tab, blocks, maps, px, pix_chain_stride, F, nld, ar, nchains,
+                                                                    npairs);
+      } else if (dir == 0)
         pxm_ring_fft3_kernel<0><<<g3, 128, PXM_FFT3_SMEM, stream>>>(tab, blocks, maps, px, pix_chain_stride, F, nld, ar, nchains,
                                                                   nitems);
       else
@@ -1823,10 +1652,10 @@ int pxm_fft_launch(int dir, const PxmFftGroup* d_groups, const PxmFftGroup* h_gr
 
 // 0: choose by grid size, 1: always the multi-pass kernel, 2: always the two-pass kernel (where it applies),
 // 3: two-pass, with the persistent staged kernel for the radix-32 class (what 0 picks for large grids)
-// 4: like 3 but with the two-CTA persistent kernel instead of the ping-pong one; any other value re-enables it
+// 4: like 3 but with the two-CTA persistent kernel pxm_ring_fft3_kernel instead of pxm_ring_fft6_kernel
 // 5: like 3 with the pair-split persistent kernel, 6: like 3 with the 32-points-per-thread persistent kernel
 void pxm_fft_set_legacy(int on) {
-  g_fft_pingpong = on != 4;
+  g_fft_two_cta = on == 4;
   if (on == 5) g_fft_pair = 1;
   if (on == 6) g_fft_pair = 0;
   g_fft_legacy = (on >= 4) ? 3 : on;

@@ -17,7 +17,7 @@ for s in m.SOURCES:
         if r.returncode:
             sys.exit(r.stderr)
         for line in (r.stdout + r.stderr).splitlines():
-            if "fft3_kernel" in line:
+            if "fft3_kernel" in line or "fft6_kernel" in line:
                 want = True
             elif "Compiling" in line:
                 want = False

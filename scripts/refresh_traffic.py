@@ -45,7 +45,7 @@ def main():
     # the first steps (the Legendre kernel also builds the quadrature tables at plan creation: skip generously)
     # (the bench carries the predictions in harmonic form: 2 persistent ring-FFT launches and 3 Legendre launches per step;
     # two consecutive steps are captured)
-    fft, log = ncu(chains, "pxm_ring_fft3_kernel", 12, 4)
+    fft, log = ncu(chains, "pxm_ring_fft6_kernel", 12, 4)
     logs.append(log)
     leg, log = ncu(chains, "pxm_legendre_kernel", 60, 6)
     logs.append(log)
