@@ -121,11 +121,12 @@ class PxMCMC:
         f = getattr(self.forward, "_ring_fusable", None)
         return bool(f is not None and getattr(self.forward, "_pxm_native", False) and f())
 
-    def _initial_preds(self, Xd):
-        """predictions of the state(s) in the form the run loops carry them: `RingPreds` in ring mode, else pixels"""
-        if self._ring_mode():
+    def _initial_preds(self, Xd, P=None):
+        """predictions of the state(s) in the form the run loops carry them: `RingPreds` in ring mode, else pixels.
+        `P`: the predictions of Xd when known, kept unless they are pixels and the loops carry ring coefficients"""
+        if self._ring_mode() and not isinstance(P, RingPreds):
             return self.forward.forward_ring(Xd)
-        return D.to_dev_c(self._forward_dev(Xd))
+        return D.to_dev_c(self._forward_dev(Xd)) if P is None else P
 
     @staticmethod
     def _pix(P):
@@ -194,8 +195,91 @@ class PxMCMC:
         return np.vdot(diff, self.forward.invcov @ diff)
 
     # ------------------------------------------------------------------ reference API
-    def run(self, start_point=None):
-        raise NotImplementedError
+    graph_run = True  # run(): replay the iteration as one CUDA graph when it can be recorded (`_graphed`)
+    _burn_in_line = False  # run() prints "Burning in..." at the progress steps of the burn-in (the reference's MYULA)
+    _pair_engine = None  # MYULA(real_pairs=True): the sampler that iterates on the packed chains
+
+    @property
+    def engine(self):
+        """the sampler whose `iterate` / `capture` / `iterate_host` act on the device representation of the chains:
+        the packed one in `real_pairs` mode, else this sampler itself"""
+        return self._pair_engine if self._pair_engine is not None else self
+
+    def _graphed(self):
+        """True when run() replays the iteration as one CUDA graph: `graph_run`, Philox noise (host draws cannot be
+        recorded) and every operation of the iteration on the device (native operator and prior, not m-sharded).
+        Small bandlimits are launch-latency bound: 85 -> 63 us per MYULA iteration at L = 32."""
+        eng = self.engine
+        return bool(self.graph_run and self.noise == "device" and eng._native()
+                    and getattr(eng.forward, "_pxm_allreduce", None) is None)
+
+    def run(self, start_point=None, *, checkpoint=None, checkpoint_every=0, resume=None):
+        """the loop of pxmcmc/mcmc.py:150-183 (MYULA) and :308-336 (SKROCK) on the device state `engine` iterates.
+        Extensions (keyword-only): `checkpoint` = file written every `checkpoint_every` iterations (and at the end);
+        `resume` = such a file: the chain continues exactly as if it had never stopped (same Philox steps / same numpy
+        RNG stream, tracked arrays restored).  In `real_pairs` mode samples are unpacked where they are tracked or
+        checkpointed (every `ngap`-th iteration), so the tracked arrays are the ordinary ones; the summaries take the
+        packed chains."""
+        eng = self.engine
+        pairs = eng is not self
+        i = 0
+        j = 0
+        self._stats_begin(eng.nchains, pairs=pairs)
+        if resume is not None:
+            i, j, X, P = self.load_checkpoint(resume)
+        else:
+            X, P = self._initial_sample(start_point, want_preds=False)
+        if pairs:  # the packed engine computes its own predictions
+            eng._step_counter = self._step_counter
+            X, P = self.pack(X), None
+        P = eng._initial_preds(X, P)
+
+        def outer(X, P):
+            """state and predictions as the tracked arrays and checkpoints hold them"""
+            return (self.unpack(X), self.unpack(eng._pix(P))) if pairs else (X, P)
+
+        graphed = eng.capture(X, P) if self._graphed() else None
+        while j < self.nsamples:
+            if graphed is not None:
+                graphed.step()
+                X, P = graphed._state_raw()
+            else:
+                X, P = eng.iterate(X, P)
+            self._step_counter = eng._step_counter
+            if self._on_grid(i):
+                P_pix = eng._pix(P)
+                self._track_dev(j, *outer(X, P_pix))
+                self._stats_push(X, P_pix, j)
+                j += 1
+            if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
+                if i >= self.nburn:
+                    self._track_flush()
+                    self._print_progress(j - 1, np.ravel(self.logPi)[j - 1], L2=np.ravel(self.L2s)[j - 1],
+                                         prior=np.ravel(self.priors)[j - 1])
+                elif self._burn_in_line:
+                    print("Burning in...")
+            i += 1
+            if checkpoint is not None and checkpoint_every and i % checkpoint_every == 0:
+                self.save_checkpoint(checkpoint, i, j, *outer(X, P))
+        if checkpoint is not None:
+            self.save_checkpoint(checkpoint, i, j, *outer(X, P))
+        self._track_flush()
+        self._stats_end()
+        self._final_state = outer(X, eng._pix(P))
+        if graphed is not None:
+            graphed.release()
+        print("\nDONE")
+
+    def capture(self, X, P=None, iterations=1):
+        """Record `iterations` passes of `iterate` as ONE CUDA graph on private copies of the state and return a
+        `GraphedChain`: `.step()` replays it (a single launch instead of ~10-40 kernel launches per MYULA iteration and
+        ~14 per stage of a SKROCK step: single-chain runs are launch-latency bound, SURVEY.md 7.2), `.state()` returns the
+        current (X, preds).  `P`: the predictions of X (computed here when None).  Needs `noise="device"` (the Philox
+        step then lives in device memory and is advanced inside the graph; the noise stream is the same as without the
+        graph)."""
+        if self.noise != "device":
+            raise ValueError("capture() needs noise='device' (host RNG draws cannot be recorded)")
+        return GraphedChain(self, X, P, iterations)
 
     def logpi(self, X, preds):
         """log posterior, L2 misfit and prior of a model (pxmcmc/mcmc.py:71-82):
@@ -334,24 +418,19 @@ class PxMCMC:
         def iteration(x, y, st, h):
             D.fista_update_dev(y, self._gradg_at(y), x, Tv, Ts, t / self.lmda, t, st, h, out=(x, y))
 
+        def warm_up():  # on copies: the state of the solve is not touched
+            xw, yw, sw, hw = X.clone(), Y.clone(), state.clone(), hist.clone()
+            for _ in range(2):
+                iteration(xw, yw, sw, hw)
+
+        def block():
+            for _ in range(K):
+                iteration(X, Y, state, hist)
+
         graph = None
         if self._native() and maxiter >= K:
-            # warm-up on copies (tables, allocator pools) before the capture; the state of the solve is not touched
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                xw, yw, sw, hw = X.clone(), Y.clone(), state.clone(), hist.clone()
-                for _ in range(2):
-                    iteration(xw, yw, sw, hw)
-            torch.cuda.current_stream().wait_stream(side)
-            torch.cuda.synchronize()
-            del xw, yw, sw, hw
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.stream(side):
-                with torch.cuda.graph(graph, stream=side):
-                    for _ in range(K):
-                        iteration(X, Y, state, hist)
-            torch.cuda.current_stream().wait_stream(side)
+            _warm_up(warm_up)
+            graph = _record_graph(block)
         its, converged, rel, Fh = 0, False, [], []
         while its < maxiter and not converged:
             k = min(K, maxiter - its)
@@ -397,29 +476,29 @@ class PxMCMC:
         if "prior" in self.track:
             self.priors = np.zeros(lead + (self.nsamples,), dtype=float)
 
-    def _tracking(self, j, X_curr, curr_preds, logPi, L2, prior):
-        """store sample j; complex values are truncated to their real part exactly
-        as numpy does when the reference assigns them into float arrays
-        (pxmcmc/mcmc.py:130-140)"""
-        def put(arr, val):
-            val = np.asarray(val)
-            if not np.iscomplexobj(arr):
-                val = val.real
-            if self.nchains > 1:
-                arr[:, j] = val
-            else:
-                arr[j] = val[0] if val.ndim and val.shape[0] == 1 else val
+    def _put(self, arr, j, val, c=slice(None)):
+        """store sample j of chain(s) `c` (all by default) in a tracked array; complex values are truncated to their
+        real part exactly as numpy does when the reference assigns them into float arrays (pxmcmc/mcmc.py:130-140)"""
+        val = np.asarray(val)
+        if not np.iscomplexobj(arr):
+            val = val.real
+        if self.nchains > 1:
+            arr[c, j] = val
+        else:
+            arr[j] = val[0] if val.ndim and val.shape[0] == 1 else val
 
+    def _tracking(self, j, X_curr, curr_preds, logPi, L2, prior):
+        """store sample j of every chain (pxmcmc/mcmc.py:130-140)"""
         if hasattr(self, "logPi"):
-            put(self.logPi, logPi)
+            self._put(self.logPi, j, logPi)
         if hasattr(self, "L2s"):
-            put(self.L2s, L2)
+            self._put(self.L2s, j, L2)
         if hasattr(self, "priors"):
-            put(self.priors, prior)
+            self._put(self.priors, j, prior)
         if hasattr(self, "preds"):
-            put(self.preds, D.to_host(curr_preds) if D.is_dev(curr_preds) else curr_preds)
+            self._put(self.preds, j, D.to_host(curr_preds) if D.is_dev(curr_preds) else curr_preds)
         if hasattr(self, "chain"):
-            put(self.chain, D.to_host(X_curr) if D.is_dev(X_curr) else X_curr)
+            self._put(self.chain, j, D.to_host(X_curr) if D.is_dev(X_curr) else X_curr)
 
     def _track_dev(self, j, X_curr, curr_preds):
         """sample j of a device-resident chain: log posterior terms and the tracked vectors.  With `async_spill` nothing
@@ -657,7 +736,7 @@ class _Spill:
 class MYULA(PxMCMC):
     """Moreau-Yosida unadjusted Langevin algorithm (pxmcmc/mcmc.py:143-201)."""
 
-    graph_run = True  # run(): replay the iteration as a CUDA graph when the noise is generated on the device
+    _burn_in_line = True
     # one step on a quadratic multiplies the deviation from the mode by 1 - p, p = delta * Lip(grad log pi): within
     # [-1, 1] for p <= 2
     stability_limit = 2.0
@@ -693,12 +772,6 @@ class MYULA(PxMCMC):
         eng.real_pairs, eng._pair_engine, eng._is_pair_engine = False, None, True
         eng._spill = None
         return eng
-
-    @property
-    def engine(self):
-        """the sampler whose `iterate` / `capture` / `iterate_host` act on the device representation of the chains:
-        the packed one in `real_pairs` mode, else this sampler itself"""
-        return self._pair_engine if self._pair_engine is not None else self
 
     @staticmethod
     def pack(X):
@@ -756,109 +829,6 @@ class MYULA(PxMCMC):
                                      stream0=self.stream0 + (2 if pair else 1) * (off or 0), out=out)
         return out
 
-    def run(self, start_point=None, *, checkpoint=None, checkpoint_every=0, resume=None):
-        """the loop of pxmcmc/mcmc.py:150-183.  Extensions (keyword-only): `checkpoint` = file written every
-        `checkpoint_every` iterations (and at the end); `resume` = such a file: the chain continues exactly as if it
-        had never stopped (same Philox steps / same numpy RNG stream, tracked arrays restored)."""
-        if self._pair_engine is not None:
-            return self._run_pairs(start_point, checkpoint, checkpoint_every, resume)
-        i = 0
-        j = 0
-        self._stats_begin()
-        if resume is not None:
-            i, j, X_curr, curr_preds = self.load_checkpoint(resume)
-        else:
-            X_curr, curr_preds = self._initial_sample(start_point)
-        if self._ring_mode() and not isinstance(curr_preds, RingPreds):
-            # predictions carried as ring coefficients: the pixel-side FFT pair of every iteration cancels
-            curr_preds = self.forward.forward_ring(X_curr)
-        # Philox noise and a native operator: the iteration is replayed as one CUDA graph (small bandlimits are
-        # launch-latency bound: 85 -> 63 us per iteration at L = 32); the noise stream is the eager one
-        graphed = None
-        if self.graph_run and self.noise == "device" and self._native() and getattr(self.forward, "_pxm_allreduce", None) is None:
-            graphed = self.capture(X_curr, curr_preds, iterations=1)
-        while j < self.nsamples:
-            if graphed is not None:
-                graphed.step()
-                X_curr, curr_preds = graphed._state_raw()
-            else:
-                X_curr, curr_preds = self.iterate(X_curr, curr_preds)
-            if i >= self.nburn:
-                if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
-                    P_pix = self._pix(curr_preds) if "predictions" in self._summarise + self._credible else curr_preds
-                    self._track_dev(j, X_curr, P_pix)
-                    self._stats_push(X_curr, P_pix, j)
-                    j += 1
-                if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
-                    self._track_flush()
-                    self._print_progress(j - 1, np.ravel(self.logPi)[j - 1], L2=np.ravel(self.L2s)[j - 1],
-                                         prior=np.ravel(self.priors)[j - 1])
-            else:
-                if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
-                    print("Burning in...")
-            i += 1
-            if checkpoint is not None and checkpoint_every and i % checkpoint_every == 0:
-                self.save_checkpoint(checkpoint, i, j, X_curr, curr_preds)
-        if checkpoint is not None:
-            self.save_checkpoint(checkpoint, i, j, X_curr, curr_preds)
-        self._track_flush()
-        self._stats_end()
-        curr_preds = self._pix(curr_preds)
-        if graphed is not None:
-            X_curr, curr_preds = X_curr.clone(), curr_preds.clone()
-            graphed.release()
-        self._final_state = (X_curr, curr_preds)
-        print("\nDONE")
-
-    def _run_pairs(self, start_point, checkpoint, checkpoint_every, resume):
-        """`run()` in `real_pairs` mode: the loop of pxmcmc/mcmc.py:150-183 on the packed state; samples are unpacked
-        where they are tracked or checkpointed (every `ngap`-th iteration), so the tracked arrays are the ordinary ones"""
-        eng = self._pair_engine
-        i = 0
-        j = 0
-        self._stats_begin(eng.nchains, pairs=True)  # on the packed chains: no unpack copy
-        if resume is not None:
-            i, j, X_curr, _ = self.load_checkpoint(resume)
-        else:
-            X_curr, _ = self._initial_sample(start_point, want_preds=False)  # the packed engine computes its own
-        eng._step_counter = self._step_counter
-        Xp = self.pack(X_curr)
-        Pp = eng._initial_preds(Xp)
-        graphed = None
-        if self.graph_run and self.noise == "device" and eng._native():
-            graphed = eng.capture(Xp, Pp, iterations=1)
-        while j < self.nsamples:
-            if graphed is not None:
-                graphed.step()
-                Xp, Pp = graphed._state_raw()
-            else:
-                Xp, Pp = eng.iterate(Xp, Pp)
-            if i >= self.nburn:
-                if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
-                    Pp_pix = eng._pix(Pp)
-                    self._track_dev(j, self.unpack(Xp), self.unpack(Pp_pix))
-                    self._stats_push(Xp, Pp_pix, j)
-                    j += 1
-                if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
-                    self._track_flush()
-                    self._print_progress(j - 1, np.ravel(self.logPi)[j - 1], L2=np.ravel(self.L2s)[j - 1],
-                                         prior=np.ravel(self.priors)[j - 1])
-            else:
-                if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
-                    print("Burning in...")
-            i += 1
-            self._step_counter = eng._step_counter
-            if checkpoint is not None and checkpoint_every and i % checkpoint_every == 0:
-                self.save_checkpoint(checkpoint, i, j, self.unpack(Xp), self.unpack(eng._pix(Pp)))
-        if checkpoint is not None:
-            self.save_checkpoint(checkpoint, i, j, self.unpack(Xp), self.unpack(eng._pix(Pp)))
-        self._track_flush()
-        self._stats_end()
-        self._final_state = (self.unpack(Xp), self.unpack(eng._pix(Pp)))
-        if graphed is not None:
-            graphed.release()
-        print("\nDONE")
-
     def iterate(self, X_curr, curr_preds, out=None):
         """One pass of the loop body (pxmcmc/mcmc.py:158-164) on device tensors
         [nchains, .]: gradg -> prox -> proposal -> new predictions.  `out = (X_buf, P_buf)`: where the new state and
@@ -878,16 +848,6 @@ class MYULA(PxMCMC):
         X_new = self._propose_dev(X_curr, proxf, gradg, out=out[0])
         return X_new, self._forward_dev(X_new, out=out[1])
 
-    def capture(self, X_curr, curr_preds, iterations=1):
-        """Record `iterations` passes of the loop body as ONE CUDA graph on private copies of the
-        state and return a `GraphedChain`: `.step()` replays it (a single launch instead of ~10-40
-        kernel launches: single-chain runs are launch-latency bound, SURVEY.md 7.2), `.state()` returns
-        the current (X, preds).  Needs `noise="device"` (the Philox step then lives in device memory
-        and is advanced inside the graph; the noise stream is the same as without the graph)."""
-        if self.noise != "device":
-            raise ValueError("capture() needs noise='device' (host RNG draws cannot be recorded)")
-        return GraphedChain(self, X_curr, curr_preds, iterations)
-
     def iterate_host(self, X_host, preds_host=None, X_out=None, preds_out=None, groups=None):
         """The same iteration through HOST buffers (pinned torch CPU tensors or numpy
         arrays [nchains, .]): copies the state in, runs the kernels, copies the new
@@ -903,7 +863,10 @@ class MYULA(PxMCMC):
         three-stage pipeline on three CUDA streams -- host->device copy of group g+1, kernels of
         group g, device->host copy of group g-1 -- so that both PCIe directions and the SMs work at
         the same time (the transfers, not the kernels, bound this path).  Results do not depend on
-        the grouping: chains are independent and chain c always draws Philox stream stream0 + c."""
+        the grouping: chains are independent and chain c always draws Philox stream stream0 + c.
+
+        Returns (X_out, preds_out), or X_out alone when predictions neither come in nor go out.  Outputs not given are
+        pinned tensors allocated here; with predictions in, no outputs and one chain group they are numpy arrays."""
         if self._summarise:
             raise NotImplementedError("summarise: iterate_host has no tracking grid (run() does); use a sampler "
                                       "without summarise=...")
@@ -911,95 +874,20 @@ class MYULA(PxMCMC):
             raise NotImplementedError("credible: iterate_host has no tracking grid (run() does); use a sampler "
                                       "without credible=...")
         dv = D.dev()
-        xh = X_host if D.is_dev(X_host) else torch.from_numpy(np.ascontiguousarray(X_host, dtype=np.complex128))
-        if preds_host is None:
-            return self._iterate_host_state(xh.unsqueeze(0) if xh.dim() == 1 else xh, X_out, preds_out, groups)
-        ph = preds_host if D.is_dev(preds_host) else torch.from_numpy(np.ascontiguousarray(preds_host, dtype=np.complex128))
-        if xh.dim() == 1:
-            xh, ph = xh.unsqueeze(0), ph.unsqueeze(0)
+        as_in = lambda a: a if D.is_dev(a) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.complex128))
+        as_out = lambda a: torch.from_numpy(a) if isinstance(a, np.ndarray) else a  # numpy outputs are filled in place
+        xh = as_in(X_host)
+        xh = xh.unsqueeze(0) if xh.dim() == 1 else xh
+        ph = None if preds_host is None else as_in(preds_host).reshape(xh.shape[0], -1)
         nch = xh.shape[0]
-        if groups is None:
-            groups = 8 if (nch >= 64 and nch % 8 == 0) else (4 if (nch >= 16 and nch % 4 == 0) else 1)
-        if isinstance(groups, int):
-            if nch % groups or self.noise != "device" and groups > 1:
-                groups = 1
-            sizes = [nch // groups] * groups
-        else:
-            sizes = [int(g) for g in groups]
-            if sum(sizes) != nch or min(sizes) < 1:
-                raise ValueError("group sizes must be positive and add up to the number of chains")
-            if self.noise != "device":
-                sizes = [nch]
-        groups = len(sizes)
-        if groups == 1:
-            Xn, Pn = self.iterate(xh.to(dv, non_blocking=True), ph.to(dv, non_blocking=True))
-            if X_out is not None:
-                X_out.copy_(Xn.reshape(X_out.shape), non_blocking=True)
-                preds_out.copy_(Pn.reshape(preds_out.shape), non_blocking=True)
-                torch.cuda.current_stream().synchronize()
-                return X_out, preds_out
-            return D.to_host(Xn), D.to_host(Pn)
+        sizes = self._group_sizes(nch, groups)
+        as_numpy = ph is not None and X_out is None and len(sizes) == 1
         if X_out is None:
-            X_out, preds_out = torch.empty_like(xh).pin_memory(), torch.empty_like(ph).pin_memory()
-        xo, po = X_out.reshape(xh.shape), preds_out.reshape(ph.shape)
-        st = getattr(self, "_pipe_streams", None)
-        if st is None:
-            st = self._pipe_streams = (torch.cuda.Stream(), torch.cuda.Stream())
-        s_in, s_out = st
-        s_cmp = torch.cuda.current_stream()
-        s_in.wait_stream(s_cmp)
-        starts = [sum(sizes[:g]) for g in range(groups)]
-        self._step_counter += 1
-        staged = []
-        for g in range(groups):  # all uploads are queued first: the copy engine never waits for the host
-            with torch.cuda.stream(s_in):
-                sl = slice(starts[g], starts[g] + sizes[g])
-                Xd, Pd = xh[sl].to(dv, non_blocking=True), ph[sl].to(dv, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(s_in)
-            staged.append((sl, Xd, Pd, ev))
-        try:
-            for g, (sl, Xd, Pd, ev) in enumerate(staged):
-                s_cmp.wait_event(ev)
-                Xd.record_stream(s_cmp)
-                Pd.record_stream(s_cmp)
-                self._group_offset = starts[g]
-                Xn, Pn = self.iterate(Xd, Pd)
-                done = torch.cuda.Event()
-                done.record(s_cmp)
-                s_out.wait_event(done)
-                with torch.cuda.stream(s_out):
-                    Xn.record_stream(s_out)
-                    Pn.record_stream(s_out)
-                    xo[sl].copy_(Xn, non_blocking=True)
-                    po[sl].copy_(Pn, non_blocking=True)
-        finally:
-            self._group_offset = None
-        s_out.synchronize()
-        return X_out, preds_out
-
-    def _iterate_host_state(self, xh, X_out, preds_out, groups):
-        """`iterate_host` without predictions on the way in (and, unless `preds_out` is given, on the way out): the same
-        three-stream pipeline over chain groups"""
-        dv = D.dev()
-        nch = xh.shape[0]
-        if groups is None:
-            groups = 8 if (nch >= 64 and nch % 8 == 0) else (4 if (nch >= 16 and nch % 4 == 0) else 1)
-        if isinstance(groups, int):
-            if nch % groups or self.noise != "device" and groups > 1:
-                groups = 1
-            sizes = [nch // groups] * groups
-        else:
-            sizes = [int(g) for g in groups]
-            if sum(sizes) != nch or min(sizes) < 1:
-                raise ValueError("group sizes must be positive and add up to the number of chains")
-            if self.noise != "device":
-                sizes = [nch]
-        if X_out is None:
-            X_out = torch.empty_like(xh).pin_memory()
-        as_t = lambda a: torch.from_numpy(a) if isinstance(a, np.ndarray) else a  # numpy outputs are filled in place
-        xo = as_t(X_out).reshape(xh.shape)
-        po = None if preds_out is None else as_t(preds_out).reshape(nch, -1)
+            X_out = torch.empty(xh.shape, dtype=xh.dtype, pin_memory=True)
+            if ph is not None:
+                preds_out = torch.empty(ph.shape, dtype=ph.dtype, pin_memory=True)
+        xo = as_out(X_out).reshape(xh.shape)
+        po = None if preds_out is None else as_out(preds_out).reshape(nch, -1)
         st = getattr(self, "_pipe_streams", None)
         if st is None:
             st = self._pipe_streams = (torch.cuda.Stream(), torch.cuda.Stream())
@@ -1007,23 +895,27 @@ class MYULA(PxMCMC):
         s_cmp = torch.cuda.current_stream()
         s_in.wait_stream(s_cmp)
         starts = [sum(sizes[:g]) for g in range(len(sizes))]
-        if self.noise == "device":
+        if self.noise == "device":  # one Philox step for the whole batch, every group at its chains' streams
             self._step_counter += 1
         staged = []
-        for g in range(len(sizes)):
+        for g in range(len(sizes)):  # all uploads are queued first: the copy engine never waits for the host
             with torch.cuda.stream(s_in):
                 sl = slice(starts[g], starts[g] + sizes[g])
                 Xd = xh[sl].to(dv, non_blocking=True)
+                Pd = None if ph is None else ph[sl].to(dv, non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record(s_in)
-            staged.append((sl, Xd, ev))
+            staged.append((sl, Xd, Pd, ev))
         try:
-            for g, (sl, Xd, ev) in enumerate(staged):
+            for g, (sl, Xd, Pd, ev) in enumerate(staged):
                 s_cmp.wait_event(ev)
                 Xd.record_stream(s_cmp)
-                if self.noise == "device":
-                    self._group_offset = starts[g]
-                Xn, Pn = self.iterate(Xd, self._initial_preds(Xd))
+                if Pd is None:
+                    Pd = self._initial_preds(Xd)
+                else:
+                    Pd.record_stream(s_cmp)
+                self._group_offset = starts[g]
+                Xn, Pn = self.iterate(Xd, Pd)
                 if po is not None:
                     Pn = self._pix(Pn)
                 done = torch.cuda.Event()
@@ -1038,7 +930,23 @@ class MYULA(PxMCMC):
         finally:
             self._group_offset = None
         s_out.synchronize()
-        return (X_out, preds_out) if preds_out is not None else X_out
+        if as_numpy:
+            return X_out.numpy(), preds_out.numpy()
+        return X_out if preds_out is None else (X_out, preds_out)
+
+    def _group_sizes(self, nch, groups):
+        """chain-group sizes of `iterate_host` from `groups` (None: 8 or 4 groups for wide batches, else 1; a count,
+        1 when it does not divide the batch; a list of sizes); one group with host noise (one numpy draw per call)"""
+        if groups is None:
+            groups = 8 if (nch >= 64 and nch % 8 == 0) else (4 if (nch >= 16 and nch % 4 == 0) else 1)
+        if isinstance(groups, int):
+            if nch % groups or self.noise != "device" and groups > 1:
+                groups = 1
+            return [nch // groups] * groups
+        sizes = [int(g) for g in groups]
+        if sum(sizes) != nch or min(sizes) < 1:
+            raise ValueError("group sizes must be positive and add up to the number of chains")
+        return sizes if self.noise == "device" else [nch]
 
     def chain_step(self, X, proxf, gradg):
         """One proposal from (X, prox(X), gradg) (pxmcmc/mcmc.py:185-201)."""
@@ -1046,44 +954,62 @@ class MYULA(PxMCMC):
         return out if D.is_dev(X) else D.to_host(out[0] if np.ndim(X) == 1 else out)
 
 
-class GraphedChain:
-    """A CUDA graph of MYULA iterations (see `MYULA.capture`)."""
+def _warm_up(body):
+    """run body() on a side stream and wait for it: tables, lazy uploads, kernel attributes and allocator pools are
+    ready before a CUDA graph capture, which must not create them"""
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        body()
+    torch.cuda.current_stream().wait_stream(side)
+    torch.cuda.synchronize()
 
-    def __init__(self, sampler, X, P, iterations=1):
+
+def _record_graph(body):
+    """body() recorded as one CUDA graph on a side stream (the capture executes nothing); the current stream waits
+    for the side stream"""
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph, stream=side):
+        body()
+    torch.cuda.current_stream().wait_stream(side)
+    return graph
+
+
+class GraphedChain:
+    """`iterations` passes of a sampler's `iterate` as one CUDA graph (see `PxMCMC.capture`).  The chain advances IN
+    PLACE: the update kernel (SKROCK: the last stage) writes X and the operator's last kernel writes P, so the graph
+    holds no copy-back and no ATen kernel.
+
+    Philox step: the graph reads and advances the device counter `dstep`, which this object keeps alive.
+    `sampler._dstep` points to it only while the graph is warmed up and recorded, so eager calls on the sampler draw
+    the host counter `sampler._step_counter`, and `step()` advances that counter with the graph."""
+
+    def __init__(self, sampler, X, P=None, iterations=1):
         self.sampler, self.iterations = sampler, int(iterations)
         self.X = sampler._state(X).clone()
-        if isinstance(P, RingPreds):
-            self.P = P.clone()
-        elif sampler._ring_mode():
-            self.P = sampler.forward.forward_ring(self.X)  # recomputed from the state in the form the iteration carries
-        else:
-            self.P = sampler._state(P).clone()
-        sampler._dstep = torch.full((1,), sampler._step_counter + 1, dtype=torch.int64, device=self.X.device)
-        # warm-up on a side stream (tables, kernel attributes, allocator pools), as CUDA graphs require
-        side = torch.cuda.Stream()
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
+        if P is not None:
+            P = P.clone() if isinstance(P, RingPreds) else sampler._state(P).clone()
+        self.P = sampler._initial_preds(self.X, P)  # (pixels are replaced by ring coefficients where those are carried)
+
+        def warm_up():  # `iterate` without `out` leaves X and P as they are
             x, p = self.X, self.P
             for _ in range(2):
                 x, p = sampler.iterate(x, p)
-        torch.cuda.current_stream().wait_stream(side)
-        torch.cuda.synchronize()
-        sampler._dstep.fill_(sampler._step_counter + 1)  # the warm-up did not happen as far as the chain is concerned
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            # the chain advances IN PLACE: the update kernel and the operator's last kernel write into X / P
-            # (no copy-back, no ATen kernel inside the graph)
-            import os
 
-            if os.environ.get("PXM_GRAPH_COPYBACK"):  # development A/B switch: the round-1 form (fresh buffers + copy-back)
-                x, p = self.X, self.P
-                for _ in range(self.iterations):
-                    x, p = sampler.iterate(x, p)
-                self.X.copy_(x)
-                self.P.copy_(p)
-            else:
-                for _ in range(self.iterations):
-                    sampler.iterate(self.X, self.P, out=(self.X, self.P))
+        def record():
+            for _ in range(self.iterations):
+                sampler.iterate(self.X, self.P, out=(self.X, self.P))
+
+        self.dstep = sampler._dstep = torch.full((1,), sampler._step_counter + 1, dtype=torch.int64,
+                                                 device=self.X.device)
+        try:
+            _warm_up(warm_up)
+            self.dstep.fill_(sampler._step_counter + 1)  # the warm-up did not happen as far as the chain is concerned
+            self.graph = _record_graph(record)
+        finally:
+            sampler._dstep = None
 
     def step(self):
         """advance the chain by `iterations` iterations (asynchronous, like any kernel launch)"""
@@ -1098,15 +1024,14 @@ class GraphedChain:
         return self.X, self.P
 
     def release(self):
-        self.sampler._dstep = None
+        """drop the graph and its step counter; X and P stay valid"""
+        self.graph = self.dstep = None
 
 
 class PxMALA(MYULA):
     """MYULA + Metropolis-Hastings correction, optional step-size tuning
     (pxmcmc/mcmc.py:204-289).  The accept decision uses numpy's global RNG after the
     Gaussian draw, as in the reference."""
-
-    use_graph = True  # device-resident loop: replay the iteration as one CUDA graph
 
     def __init__(self, forward, prox, mcmcparams=PxMCMCParams(), tune_delta=True, **kw):
         super().__init__(forward, prox, mcmcparams, **kw)
@@ -1201,19 +1126,10 @@ class PxMALA(MYULA):
         # run eagerly (they warm up tables, lazy uploads and allocator pools, and ARE iterations of the chain), then the
         # iteration is captured with its counters in the state blocks
         graph = None
-        i_start = i
-
-        def put(arr, c, j, val):
-            val = np.asarray(val)
-            if not np.iscomplexobj(arr):
-                val = val.real
-            if nch > 1:
-                arr[c, j] = val
-            else:
-                arr[j] = val
+        i_graph = i + 2 if self._graphed() else None
 
         def after(i):
-            on_grid = i >= self.nburn and (self.ngap == 0 or (i - self.nburn) % self.ngap == 0)
+            on_grid = self._on_grid(i)
             verbose = self.verbosity > 0 and (i + 1) % self.verbosity == 0
             if on_grid or verbose:
                 st = S.cpu().numpy()  # the only host synchronisation
@@ -1228,15 +1144,15 @@ class PxMALA(MYULA):
                     for c in take:
                         j = int(js[c])
                         if hasattr(self, "logPi"):
-                            put(self.logPi, c, j, complex(st[c, 4], st[c, 5]))
+                            self._put(self.logPi, j, complex(st[c, 4], st[c, 5]), c)
                         if hasattr(self, "L2s"):
-                            put(self.L2s, c, j, complex(st[c, 6], st[c, 7]))
+                            self._put(self.L2s, j, complex(st[c, 6], st[c, 7]), c)
                         if hasattr(self, "priors"):
-                            put(self.priors, c, j, st[c, 8])
+                            self._put(self.priors, j, st[c, 8], c)
                         if Ph is not None:
-                            put(self.preds, c, j, Ph[c])
+                            self._put(self.preds, j, Ph[c], c)
                         if Xh is not None:
-                            put(self.chain, c, j, Xh[c])
+                            self._put(self.chain, j, Xh[c], c)
                         js[c] += 1
                 if verbose:
                     done = sum(int(a.sum()) for a in acc_chunks) + int(acc[:, : (i % cap) + 1].sum().item())
@@ -1264,15 +1180,9 @@ class PxMALA(MYULA):
 
         while js.min() < self.nsamples:
             self._step_counter += 1
-            if graph is None and i >= i_start + 2 and self.use_graph:
+            if i == i_graph:
                 S[:, 13], S[:, 14] = float(i), float(self._step_counter)
-                side = torch.cuda.Stream()
-                side.wait_stream(torch.cuda.current_stream())
-                graph = torch.cuda.CUDAGraph()
-                with torch.cuda.stream(side):
-                    with torch.cuda.graph(graph, stream=side):
-                        body(-1, 0)
-                torch.cuda.current_stream().wait_stream(side)
+                graph = _record_graph(lambda: body(-1, 0))
             if graph is not None:
                 graph.replay()
             else:
@@ -1376,11 +1286,10 @@ class PxMALA(MYULA):
             if self.tune_delta:
                 self._tune_delta(i)
                 self.deltas_trace.append(self.delta)
-            if i >= self.nburn:
-                if (self.ngap == 0 or (i - self.nburn) % self.ngap == 0) and accept:
-                    self._tracking(j, X_curr, curr_preds, [logpiXc], [L2Xc], [priorXc])
-                    self._stats_push(X_curr, curr_preds, j)
-                    j += 1
+            if self._on_grid(i) and accept:
+                self._tracking(j, X_curr, curr_preds, [logpiXc], [L2Xc], [priorXc])
+                self._stats_push(X_curr, curr_preds, j)
+                j += 1
             if self.verbosity > 0 and (i + 1) % self.verbosity == 0:
                 self._print_progress(j - 1, np.real(logpiXc), L2=np.real(L2Xc), prior=priorXc,
                                      acceptanceRate=np.mean(self.acceptance_trace))
@@ -1397,40 +1306,6 @@ class PxMALA(MYULA):
         """pxmcmc/mcmc.py:277-279"""
         delta = self.delta * (1 + (self.acceptance_trace[i] - 0.5) / ((i + 1) ** 0.75))
         self.delta = min(max(delta, self.lmda * 1e-8), self.lmda / 2)
-
-
-class _GraphedSkrock:
-    def __init__(self, sampler, X):
-        self.sampler = sampler
-        self.X = sampler._state(X).clone()
-        counter = sampler._step_counter
-        for _ in range(2):  # warm-up (tables, lazy uploads, allocator pools) before the capture
-            x = sampler._chain_step_dev(self.X)
-            p = D.to_dev_c(sampler._forward_dev(x))
-        sampler._step_counter = counter  # the warm-up is not part of the chain: graphed and eager runs draw the same Philox steps
-        self.P = p.clone()
-        torch.cuda.synchronize()
-        # the graph reads (and advances) this counter on every replay: it must stay alive with the graph
-        self.dstep = sampler._dstep = torch.full((1,), sampler._step_counter + 1, dtype=torch.int64, device=self.X.device)
-        side = torch.cuda.Stream()
-        side.wait_stream(torch.cuda.current_stream())
-        self.graph = torch.cuda.CUDAGraph()
-        try:
-            with torch.cuda.stream(side):
-                with torch.cuda.graph(self.graph, stream=side):
-                    # in place: the last stage of the recursion writes X, the operator's last kernel writes P
-                    sampler._chain_step_dev(self.X, out=self.X)
-                    sampler._forward_dev(self.X, out=self.P)
-        finally:
-            sampler._dstep = None
-        torch.cuda.current_stream().wait_stream(side)
-
-    def step(self):
-        self.graph.replay()
-        self.sampler._step_counter += 1
-
-    def state(self):
-        return self.X, self.P
 
 
 class SKROCK(PxMCMC):
@@ -1482,45 +1357,20 @@ class SKROCK(PxMCMC):
             raise ValueError(f"checkpoint was written by a SKROCK sampler with scheme={scheme!r}, not {self._scheme!r}")
         return super()._load_ckpt(path)
 
-    def run(self, start_point=None, *, checkpoint=None, checkpoint_every=0, resume=None):
-        """the loop of pxmcmc/mcmc.py:308-336.  `checkpoint` / `checkpoint_every` / `resume` as in `MYULA.run`."""
-        i = 0
-        j = 0
-        self._stats_begin()
-        if resume is not None:
-            i, j, X_curr, curr_preds = self.load_checkpoint(resume)
-        else:
-            X_curr, curr_preds = self._initial_sample(start_point)
-        # a CUDA graph needs every operation of the step on the device: native operator and prior only
-        graphed = self.capture(X_curr) if (self.noise == "device" and self._native()
-                                           and getattr(self.forward, "_pxm_allreduce", None) is None) else None
-        while j < self.nsamples:
-            if graphed is not None:  # the whole step (s gradient evaluations + predictions) as one CUDA graph
-                graphed.step()
-                X_curr, curr_preds = graphed.state()
-            else:
-                X_curr = self._chain_step_dev(X_curr)
-                curr_preds = D.to_dev_c(self._forward_dev(X_curr))
-            if i >= self.nburn:
-                if self.ngap == 0 or (i - self.nburn) % self.ngap == 0:
-                    self._track_dev(j, X_curr, curr_preds)
-                    self._stats_push(X_curr, curr_preds, j)
-                    j += 1
-            if self.verbosity > 0 and (i + 1) % self.verbosity == 0 and j > 0:
-                self._track_flush()
-                self._print_progress(j - 1, np.ravel(self.logPi)[j - 1], L2=np.ravel(self.L2s)[j - 1],
-                                     prior=np.ravel(self.priors)[j - 1])
-            i += 1
-            if checkpoint is not None and checkpoint_every and i % checkpoint_every == 0:
-                self.save_checkpoint(checkpoint, i, j, X_curr, curr_preds)
-        if checkpoint is not None:
-            self.save_checkpoint(checkpoint, i, j, X_curr, curr_preds)
-        self._track_flush()
-        self._stats_end()
-        if graphed is not None:
-            X_curr, curr_preds = X_curr.clone(), curr_preds.clone()
-        self._final_state = (X_curr, curr_preds)
-        print("\nDONE")
+    def _initial_preds(self, Xd, P=None):
+        """pixels whatever the operator: the stage gradients are taken at other points than the state (`_gradg_at`),
+        so nothing consumes ring coefficients of the state"""
+        return D.to_dev_c(self._forward_dev(Xd)) if P is None else P
+
+    def iterate(self, X_curr, curr_preds, out=None):
+        """one step and the predictions of the new state on device tensors [nchains, .] (the step itself does not read
+        `curr_preds`).  `out = (X_buf, P_buf)` as in `MYULA.iterate`: the input buffers themselves are allowed, which
+        is how captured graphs advance in place."""
+        if out is None:
+            X_new = self._chain_step_dev(X_curr)
+            return X_new, D.to_dev_c(self._forward_dev(X_new))
+        X_new = self._chain_step_dev(X_curr, out=out[0])
+        return X_new, self._forward_dev(X_new, out=out[1])
 
     def _chain_step_dev(self, Xd, Z=None, out=None):
         """Z: real [nchains, n] normals, a (real, imaginary) pair when `complex` (pxmcmc/mcmc.py:344-347), or a
@@ -1546,13 +1396,6 @@ class SKROCK(PxMCMC):
         if dstep is not None:
             D.check(D.lib.pxm_counter_add(D.ptr(dstep), 1, D.stream_ptr()))
         return out
-
-    def capture(self, X_curr):
-        """One SKROCK step (s gradient evaluations, ~14 s launches) and its predictions as ONE CUDA graph; needs
-        noise="device".  Returns an object with .step() and .state() -> (X, preds)."""
-        if self.noise != "device":
-            raise ValueError("capture() needs noise='device' (host RNG draws cannot be recorded)")
-        return _GraphedSkrock(self, X_curr)
 
     def chain_step(self, X):
         """one SKROCK step (pxmcmc/mcmc.py:338-347)"""

@@ -511,6 +511,11 @@ def test_myula_graph_replay_matches_eager(px, iters_per_graph):
     Xg, Pg = chain.state()
     assert torch.equal(Xg, X) and torch.equal(Pg, eager._pix(P))  # bit-identical
     assert graphed._step_counter == eager._step_counter == 6
+    # an eager call after the capture draws the host counter, which the replays advanced
+    assert graphed._dstep is None
+    Xg, _ = graphed.iterate(*chain._state_raw())
+    X, P = eager.iterate(X, P)
+    assert torch.equal(Xg, X) and graphed._step_counter == eager._step_counter == 7
     with pytest.raises(ValueError):
         px.mcmc.MYULA(op, eager.prior, prm, noise="host").capture(X0, eager._pix(P0))
 
